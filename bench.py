@@ -2,11 +2,13 @@
 """bench.py -- SimMIM pre-training step throughput (samples/s) of the B200-native MaskedSST hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--precision bf16|fp32] [--impl reference] [--no-extra]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1]): one SimMIM masked-pretraining step = forward + backward + AdamW (+ the reference's
 grad clamp) of ViTSpatialSpectral(dim 96, depth 4+4, heads 8, mlp 64, dropout 0.1) on synthetic Houston2018-shaped
 cubes [B, 50, 8, 8] (bands 48-49 zero), tube masking ratio 0.7 / mask patch 4, blockwise decoder, lr .008 wd .05
-(configs/config.yaml, configs/pretrain_config.yaml of the reference).  Random-init weights, synthetic data.
+(configs/config.yaml, configs/pretrain_config.yaml of the reference).  Random-init weights, synthetic data; every step
+starts from the same initial weights (Workload.w0), so its inputs and outputs are the same from run to run.
 
 Prints ONE JSON line (rank 0).  `value` = whole-job samples/s with inputs (cubes + masks) resident in HBM;
 `e2e` = the same step through the public nn.Module API with HOST inputs: pinned cube -> H2D, masks drawn inside model(img),
@@ -47,7 +49,17 @@ def parse():
     ap.add_argument("--dropout", type=float, default=0.1)
     ap.add_argument("--workload", default="pretrain", choices=["pretrain", "finetune"],
                     help="pretrain = BASELINE configs[1] (default); finetune = CE classification step with Adam (configs[2])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, updated parameters, gradients) as "
+                         "DIR/<name>.npy.  The inputs (data, masks, dropout seeds, the weights every step starts from) are "
+                         "seeded and the same every run, so two runs or two builds agree to rounding (float-atomic gradient "
+                         "reductions: up to 6e-7 relative on a B200 at a 1000 W power limit)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs is written by --impl ours only")
+    return a
 
 
 def dist_env():
@@ -205,9 +217,20 @@ class Workload:
         else:
             self.dev_masks = [self.model.draw_masks(B, dev) for _ in range(pool)]
         self.sync = GradSync(self.opt.arena, overlap=overlap, boundaries=stage_boundaries(self.model)) if world > 1 else None
+        # Every step starts from these weights (the optimiser moments carry over).  The weight-gradient kernels reduce with
+        # float atomics, so a step's gradients vary in the last bits from run to run; training on would feed that back and
+        # amplify it (to ~20% of the parameters after 25 steps on a B200 at a 1000 W power limit).  From fixed weights each step's inputs are the same every run,
+        # what it computes agrees to rounding, and the kernels do the same work as in training.
+        self.w0 = self.opt.param_arena.clone()
+
+    def restore_weights(self):
+        self.opt.param_arena.copy_(self.w0)
+        if self.opt.bf16_arena is not None:
+            self.opt.bf16_arena.copy_(self.w0)
 
     def step_resident(self, i):
         from maskedsst_b200.dp import cross_entropy_dp
+        self.restore_weights()
         self.opt.zero_grad()
         k = i % self.pool
         if self.kind == "finetune":
@@ -224,6 +247,7 @@ class Workload:
         from maskedsst_b200.dp import cross_entropy_dp
         k = i % self.pool
         x = self.host_x[k].to(self.dev, non_blocking=True)       # H2D from pinned memory, inside the timed region
+        self.restore_weights()
         self.opt.zero_grad()
         if self.kind == "finetune":
             loss = cross_entropy_dp(self.model(x), self.host_y[k].to(self.dev, non_blocking=True), ignore_index=-1)
@@ -274,6 +298,23 @@ def time_resident(w, steps, warmup):
     launches = _lib.lib().msst_launch_count() - n0
     ms = max_over_ranks(ev0.elapsed_time(ev1), w.dev, w.world)
     return ms, launches, float(loss.item())
+
+
+def dump_outputs(out_dir, model, loss):
+    """What the timed step hands its caller, as of its last step: the loss, every updated parameter and every gradient, in
+    float32.  The bench models have under 2 M parameters, so the whole set (< 16 MB) fits the 64 MB budget unsampled."""
+    import numpy as np
+    arrays = {"loss": np.asarray(loss, dtype=np.float32)}
+    for name, p in model.named_parameters():
+        arrays["param." + name] = p.detach().float().cpu().numpy()
+        if p.grad is not None:
+            arrays["grad." + name] = p.grad.detach().float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the 64 MB budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def time_e2e(w, steps, backend="device"):
@@ -419,6 +460,8 @@ def run_ours(args):
     clocks.start()
     ms, launches, final_loss = time_resident(w, args.steps, 0)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:                          # before the e2e legs below train the model further
+        dump_outputs(args.dump_outputs, w.model, final_loss)
     # e2e leg: (a) masks drawn on the device (module option mask_backend="device"), (b) the reference-compatible host generator
     e2e_steps = max(3, min(args.steps, 10))
     e2e_res = {b: time_e2e(w, e2e_steps, b) for b in (("device", "host") if args.workload == "pretrain" else ("device",))}

@@ -34,9 +34,20 @@ def _digest():
     return h.hexdigest()
 
 
+def _up_to_date(dig):
+    stamp = os.path.join(OBJ, "digest.txt")
+    if not (os.path.exists(LIB) and os.path.exists(stamp)):
+        return False
+    with open(stamp) as f:
+        return f.read() == dig
+
+
 def build(force=False, verbose=False):
     """Serialised across processes (torchrun ranks may all find the library stale): an exclusive file lock around the whole
-    build, and the library is linked to a temporary name and renamed into place, so nobody ever dlopens a partial file."""
+    build, and the library is linked to a temporary name and renamed into place, so nobody ever dlopens a partial file.
+    An up-to-date library is returned before the lock is taken: loading it writes nothing, so a read-only tree works."""
+    if not force and _up_to_date(_digest()):
+        return LIB
     os.makedirs(OBJ, exist_ok=True)
     import fcntl
     with open(os.path.join(OBJ, "build.lock"), "w") as lock:
@@ -50,7 +61,7 @@ def build(force=False, verbose=False):
 def _build_locked(force, verbose):
     stamp = os.path.join(OBJ, "digest.txt")
     dig = _digest()
-    if not force and os.path.exists(LIB) and os.path.exists(stamp) and open(stamp).read() == dig:
+    if not force and _up_to_date(dig):
         return LIB
     if not os.path.exists(NVCC):
         if os.path.exists(LIB):
