@@ -73,8 +73,12 @@ typedef struct {
     const double* std;           /* device [raw_bands] float64 */
     int clip; float clip_lo, clip_hi;
     int win_y, win_x;            /* 0 / 1: one crop window per tile (above).  > 1: whole-tile sliding-window inference (notebook cell 13,
-                                    src/utils.py:477-605): sample n = window n % (win_y*win_x) of tile n / (win_y*win_x), its origin
-                                    (y0 + (w / win_x) * H, x0 + (w % win_x) * W) -- the windows are never copied out of the tile */
+                                    src/utils.py:477-605): the windows of all tiles are consecutive samples, never copied out of the tile */
+    int stride_y, stride_x;      /* window step in pixels, 1 <= stride <= window; 0 = the window size (non-overlapping) */
+    int win_first;               /* global index of the first window this launch reads (0: the first window of tile 0) */
+    /* Sample b is global window g = win_first + b: window w = g % (win_y*win_x) of tile g / (win_y*win_x), origin
+     *   oy = y0 + min((w / win_x) * stride_y, tile_h - y0 - H),   ox = x0 + min((w % win_x) * stride_x, tile_w - x0 - W)
+     * so a last window row / column that would cross the tile border is snapped flush to it. */
 } msst_raw_input;
 
 typedef struct {
@@ -236,6 +240,28 @@ MSST_API int msst_head_bwd(const msst_head_dims* d, const float* x, const float*
  * d_logits = softmax - onehot for valid pixels, 0 otherwise (UNSCALED: caller divides by the count). */
 MSST_API int msst_cross_entropy_fwd_bwd(const float* logits, const int64_t* labels, int B, int nc, int HW, int ignore_index,
                                float* loss_sum_count, float* d_logits, msst_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Whole-scene inference: blend overlapping window predictions into the scene (the usual fix for the seams of
+ * window-by-window classification).  Windows are laid out as in msst_raw_input with y0 = x0 = 0 and the scene as the tile:
+ * global window g is window g % (win_y*win_x) of scene g / (win_y*win_x), origins stepped by (stride_y, stride_x), the
+ * last row / column snapped to the border.  One call blends the chunk of windows [win_first, win_first + n):
+ *   logits [n, nc, win, win]   the chunk's head output (as msst_head_fwd writes it), read in place
+ *   weight [win, win] or NULL  per-window-pixel weight (NULL: 1)
+ *   acc  [B, nc, H, W] +=  weight * softmax_nc(logits)   summed over the chunk's windows covering the pixel
+ *   wsum [B, H, W]     +=  weight
+ * Deterministic: every scene pixel is owned by one thread that adds its windows in ascending g (acc = acc + c, no atomics),
+ * so the result is bitwise the same for any chunking as long as chunks are issued in ascending order.  Only the scene rows
+ * the chunk touches are visited.  1 <= stride <= win <= H, W;  win_y <= ceil((H - win) / stride_y) + 1 (ditto x); nc <= 256.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    int B, nc, H, W;             /* scenes, classes, scene rows / columns */
+    int win, stride_y, stride_x; /* square window side, window step */
+    int win_y, win_x;            /* windows per scene column / row */
+    int win_first, n;            /* this chunk: global windows [win_first, win_first + n) */
+} msst_scene_dims;
+MSST_API int msst_scene_blend(const msst_scene_dims* d, const float* logits, const float* weight, float* acc, float* wsum,
+                              msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * SimMIM decoder + masked L1 loss (vit_simmim_original.py:314-338, BlockwiseToPixels :9-40):

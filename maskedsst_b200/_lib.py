@@ -18,7 +18,8 @@ RAW_I16, RAW_U16, RAW_F32 = 0, 1, 2
 class RawInput(C.Structure):   # msst_raw_input
     _fields_ = [("tiles", vp), ("dtype", C.c_int), ("raw_bands", C.c_int), ("tile_h", C.c_int), ("tile_w", C.c_int),
                 ("y0", C.c_int), ("x0", C.c_int), ("mean", vp), ("std", vp), ("clip", C.c_int), ("clip_lo", C.c_float),
-                ("clip_hi", C.c_float), ("win_y", C.c_int), ("win_x", C.c_int)]
+                ("clip_hi", C.c_float), ("win_y", C.c_int), ("win_x", C.c_int), ("stride_y", C.c_int), ("stride_x", C.c_int),
+                ("win_first", C.c_int)]
 
 
 class EmbedDims(C.Structure):
@@ -49,6 +50,10 @@ class TfDims(C.Structure):
 
 class HeadDims(C.Structure):
     _fields_ = [("B", C.c_int), ("C", C.c_int), ("G", C.c_int), ("p1", C.c_int), ("D", C.c_int), ("nc", C.c_int)]
+
+
+class SceneDims(C.Structure):   # msst_scene_dims
+    _fields_ = [(n, C.c_int) for n in ("B", "nc", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n")]
 
 
 class DecodeDims(C.Structure):
@@ -93,6 +98,7 @@ SIGNATURES = {
     "msst_head_fwd": (C.c_int, [C.POINTER(HeadDims)] + [vp] * 6 + [vp]),
     "msst_head_bwd": (C.c_int, [C.POINTER(HeadDims)] + [vp] * 10 + [vp]),
     "msst_cross_entropy_fwd_bwd": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
+    "msst_scene_blend": (C.c_int, [C.POINTER(SceneDims), vp, vp, vp, vp, vp]),
     "msst_simmim_decode_l1_fwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 9 + [vp]),
     "msst_simmim_decode_l1_bwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 11 + [vp]),
     "msst_draw_masks": (C.c_int, [C.POINTER(MaskGenDims), vp, vp, vp]),

@@ -5,9 +5,17 @@ host synchronisation each time (inference_example.ipynb cell 13, src/utils.py:47
 windows of all tiles go through ONE forward: the patch-embedding kernel reads every window straight out of the tile through
 per-sample window offsets (csrc/pixel_source.cuh, `win_y` / `win_x` of msst_raw_input) -- no permute / copy of the input cube,
 raw int16 tiles with on-the-fly standardisation included -- and the argmax / accuracy stay on the device.
+
+Whole-scene inference (`predict_scene`) lifts the three limits of that path: any scene size (the last window row / column is
+snapped to the border), overlapping windows whose class probabilities are blended per pixel on the device (csrc/scene.cu, no seams
+every window), and chunks of windows so that a scene of any size fits.  `confusion_matrix` / `classification_metrics` score the
+resulting map as hyperspectral classification results are reported: overall accuracy, average (macro) accuracy and Cohen's kappa.
 """
+import ctypes as C
+
 import torch
 
+from . import _lib
 from .input import RawTiles
 
 
@@ -45,3 +53,119 @@ def tile_accuracy(logits, labels, ignore_index=-1):
     valid = labels != ignore_index
     n = valid.sum()
     return ((pred == labels) & valid).sum().float() / n.clamp_min(1), n
+
+
+def scene_windows(H, W, window, stride):
+    """(ny, nx): windows per scene column / row for a step of stride = (sy, sx) (or one int): ceil((H - window) / sy) + 1, so every
+    pixel is covered and the last window row / column, snapped to the border, ends flush with it."""
+    sy, sx = (stride, stride) if isinstance(stride, int) else stride
+    if not (1 <= sy <= window and 1 <= sx <= window):
+        raise ValueError(f"stride {(sy, sx)} must be in [1, window={window}]")
+    if H < window or W < window:
+        raise ValueError(f"scene {H}x{W} is smaller than the window {window}")
+    return -(-(H - window) // sy) + 1, -(-(W - window) // sx) + 1
+
+
+@torch.no_grad()
+def predict_scene(model, scene, *, stride=None, weight=None, batch_windows=4096):
+    """Classifies whole scenes with overlapping windows.
+
+    scene: standardised fp32 cube [B, C, H, W] (CUDA) or RawTiles over whole sensor scenes (crop (0, 0)); any H, W >= image_size.
+    stride: window step (int or (sy, sx)), 1 <= stride <= image_size, default image_size (no overlap).
+    weight: optional [image_size, image_size] per-window-pixel weight of a window's probabilities (e.g. a Gaussian that trusts window
+    centres more than borders); default uniform.
+    The windows run through the model in chunks of batch_windows (eval mode, no activations kept); each chunk's class probabilities
+    are accumulated into the scene on the device, deterministically and independently of batch_windows.
+    -> (probs [B, nc, H, W] fp32 = weighted mean of the covering windows' softmax, pred [B, H, W] int64 = probs.argmax(1))."""
+    w = model.image_size
+    stride = stride if stride is not None else w
+    if isinstance(scene, RawTiles):
+        if scene.crop != (0, 0):
+            raise ValueError(f"predict_scene: RawTiles must cover whole scenes (crop (0, 0)), got crop {scene.crop}")
+        tiles, means, stds, pad, clip = scene.tiles, scene.means, scene.stds, scene.pad_bands, scene.clip
+    else:
+        if scene.dim() != 4:
+            raise ValueError(f"predict_scene: scene must be [B, C, H, W], got {tuple(scene.shape)}")
+        tiles = scene if scene.dtype == torch.float32 else scene.float()
+        C_ = tiles.shape[1]
+        # identity statistics: (v - 0) / 1 in float64 rounds back to the same fp32 value
+        means, stds, pad, clip = torch.zeros(C_, dtype=torch.float64), torch.ones(C_, dtype=torch.float64), 0, None
+    B, _, H, W = tiles.shape
+    ny, nx = scene_windows(H, W, w, stride)
+    sy, sx = (stride, stride) if isinstance(stride, int) else stride
+    x = RawTiles(tiles, means, stds, image_size=w, pad_bands=pad, clip=clip, windows=(ny, nx), stride=(sy, sx))
+    dev = tiles.device
+    nc = model.num_classes
+    if weight is not None:
+        weight = torch.as_tensor(weight, dtype=torch.float32, device=dev).contiguous()
+        if weight.shape != (w, w):
+            raise ValueError(f"predict_scene: weight must be [{w}, {w}], got {tuple(weight.shape)}")
+    acc = torch.zeros(B, nc, H, W, device=dev, dtype=torch.float32)
+    wsum = torch.zeros(B, H, W, device=dev, dtype=torch.float32)
+    total, step = x.num_windows, max(1, int(batch_windows))
+    was_training = model.training
+    model.eval()
+    try:
+        for first in range(0, total, step):
+            n = min(step, total - first)
+            y = model(x.set_window_range(first, n))
+            if y.numel() != n * nc * w * w:   # e.g. the pixelwise head: one class vector per window, not a map of the window
+                raise ValueError(f"predict_scene: the model must classify every pixel of a window ([{n}, {nc}, {w}, {w}]), "
+                                 f"got {tuple(y.shape)}")
+            y = y.reshape(n, nc, w, w).float().contiguous()   # also restores a batch dim squeezed away for n == 1 (quirk C14)
+            blend_windows(y, acc, wsum, stride=(sy, sx), grid=(ny, nx), first=first, weight=weight)
+    finally:
+        model.train(was_training)
+    probs = acc / wsum[:, None]
+    return probs, probs.argmax(1)
+
+
+def blend_windows(logits, acc, wsum, *, stride, grid, first, weight=None):
+    """One chunk of msst_scene_blend: acc [B, nc, H, W] += weight * softmax(logits), wsum [B, H, W] += weight over the pixels of
+    global windows [first, first + n) (logits [n, nc, w, w] fp32, windows laid out as scene_windows / RawTiles(stride=...) lay them
+    out: grid = (ny, nx) per scene).  Chunks must be blended in ascending order; the sums are then bitwise independent of the
+    chunking."""
+    n, nc, w = logits.shape[0], logits.shape[1], logits.shape[-1]
+    B, _, H, W = acc.shape
+    for t, name in ((logits, "logits"), (acc, "acc"), (wsum, "wsum"), (weight, "weight")):
+        if t is not None and not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
+            raise ValueError(f"blend_windows: {name} must be a contiguous fp32 CUDA tensor")
+    if logits.shape != (n, nc, w, w) or acc.shape[1] != nc or wsum.shape != (B, H, W) or (weight is not None and weight.shape != (w, w)):
+        raise ValueError(f"blend_windows: shapes logits {tuple(logits.shape)}, acc {tuple(acc.shape)}, wsum {tuple(wsum.shape)} disagree")
+    dims = _lib.SceneDims(B, nc, H, W, w, stride[0], stride[1], grid[0], grid[1], first, n)
+    _lib.check(_lib.lib().msst_scene_blend(C.byref(dims), logits.data_ptr(), weight.data_ptr() if weight is not None else None,
+                                           acc.data_ptr(), wsum.data_ptr(), torch.cuda.current_stream(acc.device).cuda_stream))
+
+
+def confusion_matrix(pred, labels, num_classes, ignore_index=-1):
+    """[nc, nc] int64 counts, rows = true class, columns = predicted class.  A pixel counts when its label is not ignore_index and lies
+    in [0, num_classes) -- the validity rule of the fine-tuning loss (ce_kernel, csrc/head.cu).  Runs wherever the tensors are."""
+    labels = labels.reshape(-1).to(torch.int64)
+    pred = pred.reshape(-1).to(device=labels.device, dtype=torch.int64)
+    if pred.numel() != labels.numel():
+        raise ValueError(f"confusion_matrix: {pred.numel()} predictions for {labels.numel()} labels")
+    valid = (labels != ignore_index) & (labels >= 0) & (labels < num_classes)
+    lab, prd = labels[valid], pred[valid]
+    if bool(((prd < 0) | (prd >= num_classes)).any()):
+        raise ValueError(f"confusion_matrix: predictions outside [0, {num_classes})")
+    return torch.bincount(lab * num_classes + prd, minlength=num_classes * num_classes).reshape(num_classes, num_classes)
+
+
+def classification_metrics(conf):
+    """OA / AA / kappa of a confusion matrix (rows = true class), in float64:
+      oa    = trace / total                                      (overall accuracy)
+      per_class_acc[k] = conf[k, k] / conf[k, :].sum()           (recall; nan for a class absent from the labels)
+      aa    = mean of per_class_acc over the classes that occur in the labels (average accuracy; absent classes are left out
+              rather than counted as 0 or 1, so a scene that lacks a class is not penalised for it)
+      kappa = (oa - pe) / (1 - pe),  pe = sum_k rows_k * cols_k / total^2   (Cohen's kappa; nan when pe == 1)
+    -> dict(oa=float, aa=float, kappa=float, per_class_acc=[nc] float64 tensor on the CPU)."""
+    conf = torch.as_tensor(conf).detach().to("cpu", torch.float64)
+    total = conf.sum()
+    rows, cols, diag = conf.sum(1), conf.sum(0), conf.diagonal()
+    per_class = diag / rows                                   # 0 / 0 = nan for absent classes
+    present = rows > 0
+    oa = float(diag.sum() / total)
+    aa = float(per_class[present].mean()) if bool(present.any()) else float("nan")
+    pe = float((rows * cols).sum() / (total * total))
+    kappa = (oa - pe) / (1.0 - pe) if pe != 1.0 else float("nan")
+    return dict(oa=oa, aa=aa, kappa=kappa, per_class_acc=per_class)
