@@ -237,7 +237,9 @@ MSST_API int msst_head_bwd(const msst_head_dims* d, const float* x, const float*
                   msst_stream_t stream);
 /* nn.CrossEntropyLoss(ignore_index) over [B,nc,H,W] logits (finetune.py:136): loss_sum_count[0] = sum of
  * NLL over valid pixels, [1] = number of valid pixels (so data-parallel ranks can all-reduce both, §8(e));
- * d_logits = softmax - onehot for valid pixels, 0 otherwise (UNSCALED: caller divides by the count). */
+ * d_logits = softmax - onehot for valid pixels, 0 otherwise (UNSCALED: caller divides by the count).
+ * A pixel is valid when its label is in [0, nc) and != ignore_index.  A label outside [0, nc) is SKIPPED like ignore_index
+ * (no loss, not counted, zero gradient), where torch's cross_entropy raises an error. */
 MSST_API int msst_cross_entropy_fwd_bwd(const float* logits, const int64_t* labels, int B, int nc, int HW, int ignore_index,
                                float* loss_sum_count, float* d_logits, msst_stream_t stream);
 

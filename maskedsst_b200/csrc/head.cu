@@ -148,12 +148,14 @@ __global__ void ce_kernel(const float* __restrict__ logits, const int64_t* __res
         for (int c = 0; c < nc; ++c) mx = fmaxf(mx, p[(int64_t)c * HW]);
         float se = 0.f;
         for (int c = 0; c < nc; ++c) se += expf(p[(int64_t)c * HW] - mx);
-        const float lse = mx + logf(se);
-        if (valid) { nll = lse - p[lab * HW]; cnt = 1.f; }
+        // log-sum-exp is kept relative to the max: with large logits (|x| ~ 1e4, fp32 spacing ~1e-3) rounding mx + log(se) to
+        // fp32 would put an error of ~5e-4 into every probability that is not saturated
+        const float lse_rel = logf(se);
+        if (valid) { nll = (mx - p[lab * HW]) + lse_rel; cnt = 1.f; }
         if (d_logits) {
             float* dp = d_logits + (int64_t)b * nc * HW + px;
             for (int c = 0; c < nc; ++c)
-                dp[(int64_t)c * HW] = valid ? expf(p[(int64_t)c * HW] - lse) - (c == lab ? 1.f : 0.f) : 0.f;
+                dp[(int64_t)c * HW] = valid ? expf((p[(int64_t)c * HW] - mx) - lse_rel) - (c == lab ? 1.f : 0.f) : 0.f;
         }
     }
     nll = warp_sum(nll); cnt = warp_sum(cnt);

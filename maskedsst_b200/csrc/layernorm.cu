@@ -2,6 +2,7 @@
 // Reference: PreNorm, src/vit_spatial_spectral.py:22-29 (16 calls per forward).  HBM-bound:
 // fwd reads rows*D*4 B and writes rows*D*(4|2) B; one warp per row, D/32 values per lane in registers.
 #include "common.cuh"
+#include "kernels.h"
 
 namespace msst {
 
@@ -328,22 +329,20 @@ int layernorm_bwd(const float* x, const float* w, const float* stats, const floa
         MSST_LAUNCH_CHECK();
         return MSST_OK;
     }
-    MSST_REQUIRE(cast_out == nullptr, "layernorm_bwd: the fused bf16 cast needs D %% 4 == 0, D <= 128 and 16-byte aligned rows");
-    if (D > 256) {
-        ln_bwd_wide_kernel<<<ln_grid(rows), kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
-        MSST_LAUNCH_CHECK();
-        return MSST_OK;
-    }
+    // Otherwise (D > 128 in the bf16 transformer stack) the cast is a second pass over dx: cast_rows draws the same dropout mask
+    // (drop_factor4 of the element index / 4).  Its requirements are checked here, before anything is launched.
+    MSST_REQUIRE(cast_out == nullptr || (D % 4 == 0 && D <= 4096 && al16(dx) && (reinterpret_cast<uintptr_t>(cast_out) & 7) == 0),
+                 "layernorm_bwd: the bf16 cast of dx needs D %% 4 == 0, D <= 4096 and aligned rows");
     const int grid = ln_grid(rows);   // up to 8 CTAs/SM: the row loop is a dependent chain, memory-level parallelism comes from warps
-#define MSST_LN(NJ)                                                                                  \
-    if (nj <= NJ) {                                                                                  \
-        ln_bwd_kernel<NJ><<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D); \
-        MSST_LAUNCH_CHECK();                                                                         \
-        return MSST_OK;                                                                              \
-    }
-    MSST_LN(1) MSST_LN(2) MSST_LN(3) MSST_LN(4) MSST_LN(8)
-#undef MSST_LN
-    return MSST_ERR_ARG;
+    if (D > 256) ln_bwd_wide_kernel<<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
+    else if (nj <= 1) ln_bwd_kernel<1><<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
+    else if (nj <= 2) ln_bwd_kernel<2><<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
+    else if (nj <= 3) ln_bwd_kernel<3><<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
+    else if (nj <= 4) ln_bwd_kernel<4><<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
+    else ln_bwd_kernel<8><<<grid, kLnThreads, 0, st>>>(x, w, stats, dy, dx_add, dx, dw, db, rows, D);
+    MSST_LAUNCH_CHECK();
+    if (cast_out) return cast_rows_f32(dx, cast_out, cast_colsum, rows, D, cast_drop, st);
+    return MSST_OK;
 }
 
 }  // namespace msst

@@ -20,7 +20,7 @@ GTOL = 1e-4
 def make_encoder(spec, dropout=0.0):
     return M.ViTSpatialSpectral(
         image_size=spec.image_size, spatial_patch_size=spec.spatial_patch_size, spectral_patch_size=spec.spectral_patch_size,
-        num_classes=spec.num_classes, dim=spec.dim, depth=spec.depth, heads=spec.heads, mlp_dim=spec.mlp_dim,
+        num_classes=spec.num_classes, dim=spec.dim, depth=spec.depth, heads=spec.heads, dim_head=spec.dim_head, mlp_dim=spec.mlp_dim,
         dropout=dropout, emb_dropout=dropout, channels=spec.channels, spectral_pos_embed=spec.spectral_pos_embed,
         blockwise_patch_embed=spec.blockwise_patch_embed, spectral_pos=spec.pos(), spectral_only=spec.spectral_only)
 
