@@ -264,6 +264,27 @@ typedef struct {
 } msst_scene_dims;
 MSST_API int msst_scene_blend(const msst_scene_dims* d, const float* logits, const float* weight, float* acc, float* wsum,
                               msst_stream_t stream);
+/* Whole-scene embedding maps: the same windows, chunks, weight and ownership contract as msst_scene_blend, but each covering window
+ * contributes its encoder feature at the pixel instead of class probabilities.  One call blends the chunk [win_first, win_first + n):
+ *   tokens [n, C*S, D]         the chunk's forward_features output (fp32, t = c*S + s, S = G*G, G = win / p1), read in place
+ *   weight [win, win] or NULL  per-window-pixel weight (NULL: 1)
+ *   f(y, x) = (1/C) sum_c tokens[g - win_first, c*S + s, :],  s = ((y - oy) / p1) * G + (x - ox) / p1   ((oy, ox): origin of window g)
+ *              -- the spectral mean the default head normalises (vit_spatial_spectral.py:550-553), repeated over the p1 x p1 pixels
+ *              of each spatial patch
+ *   acc  [B, D, H, W] +=  weight * f                   summed over the chunk's windows covering the pixel, ascending g
+ *   wsum [B, H, W]    +=  weight
+ * Bitwise independent of the chunking (chunks in ascending order); only the scene rows the chunk touches are visited.
+ * 1 <= stride <= win <= H, W;  win_y <= ceil((H - win) / stride_y) + 1 (ditto x);  D <= 256;  C, p1 >= 1;  win % p1 == 0.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    int B, D, H, W;              /* scenes, feature width, scene rows / columns */
+    int win, stride_y, stride_x; /* square window side, window step */
+    int win_y, win_x;            /* windows per scene column / row */
+    int win_first, n;            /* this chunk: global windows [win_first, win_first + n) */
+    int C, p1;                   /* spectral blocks, spatial patch side */
+} msst_scene_embed_dims;
+MSST_API int msst_scene_embed(const msst_scene_embed_dims* d, const float* tokens, const float* weight, float* acc, float* wsum,
+                              msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * SimMIM decoder + masked L1 loss (vit_simmim_original.py:314-338, BlockwiseToPixels :9-40):

@@ -56,6 +56,10 @@ class SceneDims(C.Structure):   # msst_scene_dims
     _fields_ = [(n, C.c_int) for n in ("B", "nc", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n")]
 
 
+class SceneEmbedDims(C.Structure):   # msst_scene_embed_dims
+    _fields_ = [(n, C.c_int) for n in ("B", "D", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n", "C", "p1")]
+
+
 class DecodeDims(C.Structure):
     _fields_ = [("B", C.c_int), ("C", C.c_int), ("G", C.c_int), ("p0", C.c_int), ("p1", C.c_int), ("D", C.c_int),
                 ("nm", C.c_int), ("n_weight_blocks", C.c_int), ("raw", C.POINTER(RawInput))]
@@ -99,6 +103,7 @@ SIGNATURES = {
     "msst_head_bwd": (C.c_int, [C.POINTER(HeadDims)] + [vp] * 10 + [vp]),
     "msst_cross_entropy_fwd_bwd": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
     "msst_scene_blend": (C.c_int, [C.POINTER(SceneDims), vp, vp, vp, vp, vp]),
+    "msst_scene_embed": (C.c_int, [C.POINTER(SceneEmbedDims), vp, vp, vp, vp, vp]),
     "msst_simmim_decode_l1_fwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 9 + [vp]),
     "msst_simmim_decode_l1_bwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 11 + [vp]),
     "msst_draw_masks": (C.c_int, [C.POINTER(MaskGenDims), vp, vp, vp]),

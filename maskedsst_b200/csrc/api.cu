@@ -16,5 +16,5 @@ void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 }  // namespace msst
 
 extern "C" const char* msst_last_error(void) { return msst::g_err; }
-extern "C" int msst_version(void) { return 101; }
+extern "C" int msst_version(void) { return 102; }
 extern "C" long long msst_launch_count(void) { return msst::g_launches.load(); }

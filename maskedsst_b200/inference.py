@@ -11,12 +11,15 @@ snapped to the border), overlapping windows whose class probabilities are blende
 every window), and chunks of windows so that a scene of any size fits.  `confusion_matrix` / `classification_metrics` score the
 resulting map as hyperspectral classification results are reported: overall accuracy, average (macro) accuracy and Cohen's kappa.
 """
-import ctypes as C
+import ctypes
+import math
 
 import torch
 
 from . import _lib
 from .input import RawTiles
+from .vit_simmim_original import SimMIMSpatialSpectral
+from .vit_spatial_spectral import ViTSpatialSpectral
 
 
 @torch.no_grad()
@@ -66,6 +69,32 @@ def scene_windows(H, W, window, stride):
     return -(-(H - window) // sy) + 1, -(-(W - window) // sx) + 1
 
 
+def _scene_input(who, scene, w, stride, weight):
+    """The window view of a scene shared by predict_scene / embed_scene -> (RawTiles over all windows, (sy, sx), (ny, nx), weight on
+    the scene's device or None)."""
+    stride = stride if stride is not None else w
+    if isinstance(scene, RawTiles):
+        if scene.crop != (0, 0):
+            raise ValueError(f"{who}: RawTiles must cover whole scenes (crop (0, 0)), got crop {scene.crop}")
+        tiles, means, stds, pad, clip = scene.tiles, scene.means, scene.stds, scene.pad_bands, scene.clip
+    else:
+        if scene.dim() != 4:
+            raise ValueError(f"{who}: scene must be [B, C, H, W], got {tuple(scene.shape)}")
+        tiles = scene if scene.dtype == torch.float32 else scene.float()
+        C_ = tiles.shape[1]
+        # identity statistics: (v - 0) / 1 in float64 rounds back to the same fp32 value
+        means, stds, pad, clip = torch.zeros(C_, dtype=torch.float64), torch.ones(C_, dtype=torch.float64), 0, None
+    _, _, H, W = tiles.shape
+    ny, nx = scene_windows(H, W, w, stride)
+    sy, sx = (stride, stride) if isinstance(stride, int) else stride
+    x = RawTiles(tiles, means, stds, image_size=w, pad_bands=pad, clip=clip, windows=(ny, nx), stride=(sy, sx))
+    if weight is not None:
+        weight = torch.as_tensor(weight, dtype=torch.float32, device=tiles.device).contiguous()
+        if weight.shape != (w, w):
+            raise ValueError(f"{who}: weight must be [{w}, {w}], got {tuple(weight.shape)}")
+    return x, (sy, sx), (ny, nx), weight
+
+
 @torch.no_grad()
 def predict_scene(model, scene, *, stride=None, weight=None, batch_windows=4096):
     """Classifies whole scenes with overlapping windows.
@@ -78,28 +107,10 @@ def predict_scene(model, scene, *, stride=None, weight=None, batch_windows=4096)
     are accumulated into the scene on the device, deterministically and independently of batch_windows.
     -> (probs [B, nc, H, W] fp32 = weighted mean of the covering windows' softmax, pred [B, H, W] int64 = probs.argmax(1))."""
     w = model.image_size
-    stride = stride if stride is not None else w
-    if isinstance(scene, RawTiles):
-        if scene.crop != (0, 0):
-            raise ValueError(f"predict_scene: RawTiles must cover whole scenes (crop (0, 0)), got crop {scene.crop}")
-        tiles, means, stds, pad, clip = scene.tiles, scene.means, scene.stds, scene.pad_bands, scene.clip
-    else:
-        if scene.dim() != 4:
-            raise ValueError(f"predict_scene: scene must be [B, C, H, W], got {tuple(scene.shape)}")
-        tiles = scene if scene.dtype == torch.float32 else scene.float()
-        C_ = tiles.shape[1]
-        # identity statistics: (v - 0) / 1 in float64 rounds back to the same fp32 value
-        means, stds, pad, clip = torch.zeros(C_, dtype=torch.float64), torch.ones(C_, dtype=torch.float64), 0, None
-    B, _, H, W = tiles.shape
-    ny, nx = scene_windows(H, W, w, stride)
-    sy, sx = (stride, stride) if isinstance(stride, int) else stride
-    x = RawTiles(tiles, means, stds, image_size=w, pad_bands=pad, clip=clip, windows=(ny, nx), stride=(sy, sx))
-    dev = tiles.device
+    x, (sy, sx), (ny, nx), weight = _scene_input("predict_scene", scene, w, stride, weight)
+    B, _, H, W = x.tiles.shape
+    dev = x.tiles.device
     nc = model.num_classes
-    if weight is not None:
-        weight = torch.as_tensor(weight, dtype=torch.float32, device=dev).contiguous()
-        if weight.shape != (w, w):
-            raise ValueError(f"predict_scene: weight must be [{w}, {w}], got {tuple(weight.shape)}")
     acc = torch.zeros(B, nc, H, W, device=dev, dtype=torch.float32)
     wsum = torch.zeros(B, H, W, device=dev, dtype=torch.float32)
     total, step = x.num_windows, max(1, int(batch_windows))
@@ -133,7 +144,64 @@ def blend_windows(logits, acc, wsum, *, stride, grid, first, weight=None):
     if logits.shape != (n, nc, w, w) or acc.shape[1] != nc or wsum.shape != (B, H, W) or (weight is not None and weight.shape != (w, w)):
         raise ValueError(f"blend_windows: shapes logits {tuple(logits.shape)}, acc {tuple(acc.shape)}, wsum {tuple(wsum.shape)} disagree")
     dims = _lib.SceneDims(B, nc, H, W, w, stride[0], stride[1], grid[0], grid[1], first, n)
-    _lib.check(_lib.lib().msst_scene_blend(C.byref(dims), logits.data_ptr(), weight.data_ptr() if weight is not None else None,
+    _lib.check(_lib.lib().msst_scene_blend(ctypes.byref(dims), logits.data_ptr(), weight.data_ptr() if weight is not None else None,
+                                           acc.data_ptr(), wsum.data_ptr(), torch.cuda.current_stream(acc.device).cuda_stream))
+
+
+@torch.no_grad()
+def embed_scene(model, scene, *, stride=None, weight=None, batch_windows=4096):
+    """Per-pixel encoder features of whole scenes from overlapping windows: the map a k-NN / linear probe, a clustering or another
+    model starts from after pretraining.
+
+    model: ViTSpatialSpectral with any head (the head is not run; spectral_only too), or SimMIMSpatialSpectral, whose encoder is used
+    (so a pretraining checkpoint embeds directly).  fp32 or bf16 precision; the features are fp32 either way.
+    scene, stride, weight, batch_windows: as in predict_scene (weight weighs a window's features instead of its probabilities).
+    A window's feature at a pixel is the spectral mean of its tokens at the pixel's spatial patch, the input of the default head's
+    LayerNorm; the covering windows' features are blended on the device, deterministically and independently of batch_windows.
+    -> features [B, dim, H, W] fp32 = weighted mean of the covering windows' features."""
+    enc = model.encoder if isinstance(model, SimMIMSpatialSpectral) else model
+    if not isinstance(enc, ViTSpatialSpectral):   # ViTSpatialSpectral_V1.forward_features returns a tuple of token sets
+        raise ValueError(f"embed_scene: needs a ViTSpatialSpectral encoder, got {type(enc).__name__}")
+    w = enc.image_size
+    x, (sy, sx), (ny, nx), weight = _scene_input("embed_scene", scene, w, stride, weight)
+    B, _, H, W = x.tiles.shape
+    D, nblk, p1 = enc.dim, enc.num_spectral_patches, enc.patch_height
+    acc = torch.zeros(B, D, H, W, device=x.tiles.device, dtype=torch.float32)
+    wsum = torch.zeros(B, H, W, device=x.tiles.device, dtype=torch.float32)
+    total, step = x.num_windows, max(1, int(batch_windows))
+    was_training = enc.training
+    enc.eval()
+    try:
+        for first in range(0, total, step):
+            n = min(step, total - first)
+            tokens = enc.forward_features(x.set_window_range(first, n))   # [n, C*S, D] fp32 (the residual stream)
+            embed_windows(tokens, acc, wsum, C=nblk, p1=p1, stride=(sy, sx), grid=(ny, nx), first=first, weight=weight)
+    finally:
+        enc.train(was_training)
+    return acc / wsum[:, None]
+
+
+def embed_windows(tokens, acc, wsum, *, C, p1, stride, grid, first, weight=None):
+    """One chunk of msst_scene_embed: acc [B, D, H, W] += weight * f, wsum [B, H, W] += weight over the pixels of global windows
+    [first, first + n), where f is the window's spectral-mean feature at the pixel's spatial patch, (1/C) sum_c tokens[c*S + s]
+    (tokens [n, C*S, D] fp32 = forward_features of the chunk, S = G*G, window side G*p1; windows laid out as in blend_windows).
+    Chunks must be embedded in ascending order; the sums are then bitwise independent of the chunking."""
+    for t, name in ((tokens, "tokens"), (acc, "acc"), (wsum, "wsum"), (weight, "weight")):
+        if t is not None and not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
+            raise ValueError(f"embed_windows: {name} must be a contiguous fp32 CUDA tensor")
+    if tokens.dim() != 3 or acc.dim() != 4 or C < 1 or p1 < 1:
+        raise ValueError(f"embed_windows: tokens must be [n, C*S, D] and acc [B, D, H, W], got {tuple(tokens.shape)}, {tuple(acc.shape)}")
+    n, T, D = tokens.shape
+    B, _, H, W = acc.shape
+    S = T // C
+    G = math.isqrt(S)
+    w = G * p1
+    if (T != C * S or G * G != S or acc.shape[1] != D or wsum.shape != (B, H, W)
+            or (weight is not None and weight.shape != (w, w))):
+        raise ValueError(f"embed_windows: shapes tokens {tuple(tokens.shape)} (C={C}, p1={p1}), acc {tuple(acc.shape)}, "
+                         f"wsum {tuple(wsum.shape)} disagree")
+    dims = _lib.SceneEmbedDims(B, D, H, W, w, stride[0], stride[1], grid[0], grid[1], first, n, C, p1)
+    _lib.check(_lib.lib().msst_scene_embed(ctypes.byref(dims), tokens.data_ptr(), weight.data_ptr() if weight is not None else None,
                                            acc.data_ptr(), wsum.data_ptr(), torch.cuda.current_stream(acc.device).cuda_stream))
 
 
