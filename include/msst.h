@@ -14,7 +14,10 @@
  *   - token order t = c*S + s (spectral block major), patch vector order (p0 p1 p2), qkv rows q|k|v each
  *     head-major (h d)  -- reference vit_spatial_spectral.py:198,218,68-69 (SURVEY.md C18)
  *   - dropout masks are never stored: (seed, site, element index) -> counter hash (lowbias32, 16-bit lanes); p = 0 disables;
- *     `seed_dev` (optional device uint64) is added to the seed so a captured CUDA graph draws fresh masks per replay
+ *     `seed_dev` (optional device uint64) is added to the seed so a captured CUDA graph draws fresh masks per replay.
+ *     An element is kept iff its 16-bit lane >= floor(p * 2^32) >> 16, so p is resolved to 2^-16: a p below 2^-16 drops
+ *     nothing but still scales by 1/(1-p).  p = 1 drops everything (factor 0, as nn.Dropout(1.0)).  A p outside [0, 1],
+ *     NaN included, is MSST_ERR_ARG before any launch.
  */
 #ifndef MSST_H_
 #define MSST_H_

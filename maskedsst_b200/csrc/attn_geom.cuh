@@ -42,6 +42,7 @@ inline int make_attn_geom(const msst_attn_dims* d, AttnGeom& g, bool any_dh) {
     MSST_REQUIRE(any_dh ? (d->dh == 32 || d->dh == 64 || d->dh == 128) : d->dh == 64, "attention: dim_head=%d unsupported (%s)", d->dh, any_dh ? "32, 64, 128" : "bf16 mode: 64");
     MSST_REQUIRE(d->n_seq % d->inner == 0, "attention: n_seq must be a multiple of inner");
     MSST_REQUIRE(d->H <= 65535, "attention: too many heads");
+    MSST_REQUIRE(drop_p_ok(d->drop_p), "attention: drop_p=%g outside [0, 1]", (double)d->drop_p);
     g.n_seq = d->n_seq; g.N = d->N; g.inner = d->inner; g.H = d->H; g.dh = d->dh;
     g.scale = 1.0f / sqrtf((float)d->dh);
     g.gpb = 0;

@@ -118,9 +118,11 @@ struct Drop {
     const uint64_t* seed_dev;   // optional device-resident seed offset (lets a captured CUDA graph draw fresh masks per replay)
     uint32_t site;
     uint32_t thresh;   // 0 => dropout disabled
-    float scale;       // 1/(1-p)
+    float scale;       // 1/(1-p); 0 for p = 1 (a lane of 0xFFFF still passes the compare, and must yield 0, not inf)
     __host__ __device__ bool on() const { return thresh != 0u; }
 };
+// p must lie in [0, 1] (nn.Dropout's range; NaN fails): every entry point that takes a dropout probability checks it first
+inline bool drop_p_ok(float p) { return p >= 0.f && p <= 1.f; }
 inline Drop make_drop(float p, uint64_t seed, uint32_t site, const uint64_t* seed_dev = nullptr) {
     Drop d; d.seed = seed; d.site = site; d.seed_dev = seed_dev;
     if (p <= 0.f) { d.thresh = 0u; d.scale = 1.f; }
@@ -128,7 +130,7 @@ inline Drop make_drop(float p, uint64_t seed, uint32_t site, const uint64_t* see
         double t = (double)p * 4294967296.0;
         d.thresh = t >= 4294967295.0 ? 4294967295u : (uint32_t)t;
         if (d.thresh == 0u) d.thresh = 1u;
-        d.scale = 1.f / (1.f - p);
+        d.scale = p >= 1.f ? 0.f : 1.f / (1.f - p);
     }
     return d;
 }

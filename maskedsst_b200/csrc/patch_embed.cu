@@ -317,6 +317,7 @@ static int make_geom(const msst_embed_dims* d, const float* img, EmbedGeom& g) {
     MSST_REQUIRE(d && d->B > 0 && d->C > 0 && d->G > 0 && d->p0 > 0 && d->p1 > 0, "patch_embed: bad dims");
     MSST_REQUIRE(d->D % 32 == 0 && d->D >= 32 && d->D <= 256, "patch_embed: D=%d must be a multiple of 32 in [32,256]", d->D);
     MSST_REQUIRE(d->n_weight_blocks == 1 || d->n_weight_blocks == d->C, "patch_embed: n_weight_blocks must be 1 or C");
+    MSST_REQUIRE(drop_p_ok(d->drop_p), "patch_embed: drop_p=%g outside [0, 1]", (double)d->drop_p);
     g.B = d->B; g.C = d->C; g.G = d->G; g.p0 = d->p0; g.p1 = d->p1; g.D = d->D;
     g.P = d->p0 * d->p1 * d->p1; g.S = d->G * d->G; g.T = g.C * g.S;
     g.Wimg = d->G * d->p1; g.HW = g.Wimg * g.Wimg; g.nb = 1;

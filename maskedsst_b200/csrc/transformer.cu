@@ -94,6 +94,7 @@ static int check_dims(const msst_tf_dims* d) {
     MSST_REQUIRE(d->D > 0 && d->D <= 256 && d->M > 0 && d->H > 0, "transformer: bad model dims");
     MSST_REQUIRE(d->D % 4 == 0 && d->M % 4 == 0, "transformer: D and M must be multiples of 4");
     MSST_REQUIRE(d->prec == MSST_PREC_FP32 || d->prec == MSST_PREC_BF16, "transformer: unknown precision mode %d", d->prec);
+    MSST_REQUIRE(drop_p_ok(d->drop_p), "transformer: drop_p=%g outside [0, 1]", (double)d->drop_p);
     if (d->prec == MSST_PREC_BF16) {
         MSST_REQUIRE(d->dh == 64, "transformer (bf16): dim_head must be 64");
         MSST_REQUIRE(d->D % 8 == 0 && d->M % 8 == 0 && d->L <= 8, "transformer (bf16): D, M must be multiples of 8 and L <= 8");
@@ -408,6 +409,7 @@ extern "C" int msst_transformer_bwd(const msst_tf_dims* d, const msst_layer_para
 extern "C" int msst_linear_fwd(const msst_linear_dims* d, const void* x, const void* W, const float* bias, const float* residual,
                                void* y, void* pre_act, msst_stream_t stream) {
     MSST_REQUIRE(d, "linear_fwd: null dims");
+    MSST_REQUIRE(drop_p_ok(d->drop_p), "linear_fwd: drop_p=%g outside [0, 1]", (double)d->drop_p);
     const Drop drop = make_drop(d->drop_p, d->seed, d->site, d->seed_dev);
     if (d->prec == MSST_PREC_BF16) {
         GemmBf16Args a{(const __nv_bfloat16*)x, (const __nv_bfloat16*)W, d->M, d->N, d->K, bias, residual, y, d->y_fp32,
@@ -420,6 +422,7 @@ extern "C" int msst_linear_fwd(const msst_linear_dims* d, const void* x, const v
 extern "C" int msst_linear_bwd_data(const msst_linear_dims* d, const void* dy, const void* W, const void* pre_act,
                                     const float* dx_add, void* dx, msst_stream_t stream) {
     MSST_REQUIRE(d, "linear_bwd_data: null dims");
+    MSST_REQUIRE(drop_p_ok(d->drop_p), "linear_bwd_data: drop_p=%g outside [0, 1]", (double)d->drop_p);
     const Drop drop = make_drop(d->drop_p, d->seed, d->site, d->seed_dev);
     if (d->prec == MSST_PREC_BF16) {   // dx[M,K] = dy[M,N] . (W^T)[K,N]^T
         GemmBf16Args a{(const __nv_bfloat16*)dy, (const __nv_bfloat16*)W, d->M, d->K, d->N, nullptr, dx_add, dx, d->y_fp32,
@@ -481,6 +484,7 @@ extern "C" int msst_mlp_block_fwd(const void* h2, const float* xmid, const void*
                                   float drop_p, uint64_t seed, uint32_t site_hidden, uint32_t site_out, const uint64_t* seed_dev, msst_stream_t stream) {
     MSST_REQUIRE(h2 && xmid && w1 && w2 && b1 && b2 && u && g && y, "mlp_block_fwd: null pointer");
     MSST_REQUIRE(!h1 || (ln_w && ln_b && ln_stats), "mlp_block_fwd: h1 needs ln_w, ln_b and ln_stats");
+    MSST_REQUIRE(drop_p_ok(drop_p), "mlp_block_fwd: drop_p=%g outside [0, 1]", (double)drop_p);
     return mlp_block_fwd((const bf16*)h2, xmid, (const bf16*)w1, (const bf16*)w2, b1, b2, (bf16*)u, (bf16*)g, y, ln_w, ln_b, (bf16*)h1, ln_stats, R, D, M,
                          make_drop(drop_p, seed, site_hidden, seed_dev), make_drop(drop_p, seed, site_out, seed_dev), (cudaStream_t)stream);
 }
@@ -488,10 +492,12 @@ extern "C" int msst_mlp_block_bwd(const void* dyb, const void* u, const void* g,
                                   float* d_w2, float* d_b1, float* d_h, int64_t R, int D, int M, float drop_p, uint64_t seed, uint32_t site_hidden,
                                   const uint64_t* seed_dev, msst_stream_t stream) {
     MSST_REQUIRE(dyb && u && g && h2 && w2_t && w1_t && d_w1 && d_w2 && d_b1 && d_h, "mlp_block_bwd: null pointer");
+    MSST_REQUIRE(drop_p_ok(drop_p), "mlp_block_bwd: drop_p=%g outside [0, 1]", (double)drop_p);
     return mlp_block_bwd((const bf16*)dyb, (const bf16*)u, (const bf16*)g, (const bf16*)h2, (const bf16*)w2_t, (const bf16*)w1_t, d_w1, d_w2, d_b1, d_h,
                          R, D, M, make_drop(drop_p, seed, site_hidden, seed_dev), (cudaStream_t)stream);
 }
 extern "C" int msst_dropout_apply(const float* x, float* y, int64_t n, float p, uint64_t seed, uint32_t site,
                                   const uint64_t* seed_dev, msst_stream_t stream) {
+    MSST_REQUIRE(drop_p_ok(p), "dropout_apply: p=%g outside [0, 1]", (double)p);
     return dropout_apply_f32(x, y, n, make_drop(p, seed, site, seed_dev), (cudaStream_t)stream);
 }

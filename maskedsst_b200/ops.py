@@ -35,6 +35,12 @@ def _seed_dev():
     return None if _device_seed is None else _device_seed.data_ptr()
 
 
+def _check_drop_p(p):
+    """nn.Dropout's range: p in [0, 1] (p = 1 zeroes the branch); NaN or anything outside is an error, not a silent mask."""
+    if not 0.0 <= float(p) <= 1.0:
+        raise ValueError(f"maskedsst_b200: dropout probability must be in [0, 1], got {p}")
+
+
 def _stream():
     return torch.cuda.current_stream().cuda_stream
 
@@ -149,6 +155,7 @@ class PatchEmbedFn(torch.autograd.Function):
 
 def patch_embed(img, pre_w, pre_b, W, bias, post_w, post_b, pos, mask_token=None, mask=None, *, geom, drop_p=0.0,
                 seed=0, want_ln=False):
+    _check_drop_p(drop_p)
     out, pln = PatchEmbedFn.apply(img, pre_w, pre_b, W, bias, post_w, post_b, pos, mask_token, mask, geom, drop_p, seed, want_ln)
     return (out, pln) if want_ln else out
 
@@ -205,6 +212,7 @@ class TransformerStackFn(torch.autograd.Function):
 def transformer_stack(x, layer_params, *, n_seq, N, inner, heads, dim_head, mlp_dim, drop_p=0.0, seed=0, site_base=SITE_LAYER_BASE,
                       prec=PREC_FP32):
     """layer_params: list (per layer) of the 11 tensors in _LAYER_FIELDS order."""
+    _check_drop_p(drop_p)
     flat = [t for lp in layer_params for t in lp]
     # Function.forward runs with grad mode off, so decide here whether activations must be kept for backward
     need_grad = torch.is_grad_enabled() and (x.requires_grad or any(t.requires_grad for t in flat))
@@ -443,4 +451,5 @@ class AttentionFn(torch.autograd.Function):
 
 def attention(qkv, *, n_seq, N, inner=1, heads=8, dim_head=64, drop_p=0.0, seed=0, site=0):
     """qkv [n_seq*N, 3*heads*dim_head] -> [n_seq*N, heads*dim_head]."""
+    _check_drop_p(drop_p)
     return AttentionFn.apply(qkv, (n_seq, N, inner, heads, dim_head, drop_p, seed, site))

@@ -278,45 +278,56 @@ def gelu_erf(x):
     return 0.5 * x * (1.0 + torch.erf(x / math.sqrt(2.0)))
 
 
-def attention(x, sd, base: str, heads: int, dim_head: int, drop: float = 0.0):
-    """Attention.forward (vit_spatial_spectral.py:67-78). x [n,N,D].  drop > 0 = training-mode dropout on the
-    probabilities (:74) and the output projection (:62), only used by the CPU-baseline timing leg."""
+SITE_EMB, SITE_LAYER_BASE = 1, 16   # dropout site ids: emb-dropout; layer l of a stack uses base + 8 l + (0 probs, 1 attn out,
+                                   # 2 MLP hidden, 3 MLP out); the spectral stack after a spatial one starts at 16 + 8 depth
+
+
+def _dropout(t, drop, site, layout):
+    """drop: a float p = training-mode torch dropout (the CPU-baseline timing leg); or a callable drop(t, site, layout) that
+    returns t * mask, so a test can apply the exact masks of a kernel run (layout: "spatial" / "spectral" stack, "emb")."""
+    return drop(t, site, layout) if callable(drop) else F.dropout(t, drop)
+
+
+def attention(x, sd, base: str, heads: int, dim_head: int, drop=0.0, site: int = SITE_LAYER_BASE, layout=None):
+    """Attention.forward (vit_spatial_spectral.py:67-78). x [n,N,D].  drop (see _dropout): dropout on the
+    probabilities (:74, site) and the output projection (:62, site + 1)."""
     n, N, D = x.shape
     qkv = x @ sd[base + "to_qkv.weight"].T
     q, k, v = qkv.split(heads * dim_head, dim=-1)
     sh = lambda t: t.reshape(n, N, heads, dim_head).permute(0, 2, 1, 3)
     q, k, v = sh(q), sh(k), sh(v)
     dots = (q @ k.transpose(-1, -2)) * dim_head ** -0.5
-    p = F.dropout(torch.softmax(dots, dim=-1), drop)
+    p = _dropout(torch.softmax(dots, dim=-1), drop, site, layout)
     o = (p @ v).permute(0, 2, 1, 3).reshape(n, N, heads * dim_head)
-    return F.dropout(o @ sd[base + "to_out.0.weight"].T + sd[base + "to_out.0.bias"], drop)
+    return _dropout(o @ sd[base + "to_out.0.weight"].T + sd[base + "to_out.0.bias"], drop, site + 1, layout)
 
 
-def transformer(x, sd, base: str, spec: Spec, drop: float = 0.0):
+def transformer(x, sd, base: str, spec: Spec, drop=0.0, layout=None, site_base: int = SITE_LAYER_BASE):
     """Transformer.forward (vit_spatial_spectral.py:100-104): pre-norm attn + pre-norm MLP, no final norm."""
     for l in range(spec.depth):
         b = base + f"layers.{l}."
+        site = site_base + 8 * l
         h = _ln(x, sd[b + "0.norm.weight"], sd[b + "0.norm.bias"])
-        x = attention(h, sd, b + "0.fn.", spec.heads, spec.dim_head, drop) + x
+        x = attention(h, sd, b + "0.fn.", spec.heads, spec.dim_head, drop, site, layout) + x
         h = _ln(x, sd[b + "1.norm.weight"], sd[b + "1.norm.bias"])
-        u = F.dropout(gelu_erf(h @ sd[b + "1.fn.net.0.weight"].T + sd[b + "1.fn.net.0.bias"]), drop)
-        x = F.dropout(u @ sd[b + "1.fn.net.3.weight"].T + sd[b + "1.fn.net.3.bias"], drop) + x
+        u = _dropout(gelu_erf(h @ sd[b + "1.fn.net.0.weight"].T + sd[b + "1.fn.net.0.bias"]), drop, site + 2, layout)
+        x = _dropout(u @ sd[b + "1.fn.net.3.weight"].T + sd[b + "1.fn.net.3.bias"], drop, site + 3, layout) + x
     return x
 
 
-def transformer_forward(tokens, sd, spec: Spec, pre: str = "", drop: float = 0.0):
+def transformer_forward(tokens, sd, spec: Spec, pre: str = "", drop=0.0):
     """spatial_spectral_transformer (vit_spatial_spectral.py:393-431). tokens [B,T,D], t = c*S + s."""
     B = tokens.shape[0]
     C, S, D = spec.C, spec.S, spec.dim
     base = pre + "spatial_spectral_transformer."
     x = tokens
     if not spec.spectral_only:
-        x = transformer(x.reshape(B * C, S, D), sd, base + "1.", spec, drop)
+        x = transformer(x.reshape(B * C, S, D), sd, base + "1.", spec, drop, "spatial")
         x = x.reshape(B, C, S, D).permute(0, 2, 1, 3).reshape(B * S, C, D)
-        x = transformer(x, sd, base + "3.", spec, drop)
+        x = transformer(x, sd, base + "3.", spec, drop, "spectral", SITE_LAYER_BASE + 8 * spec.depth)
     else:
         x = x.reshape(B, C, S, D).permute(0, 2, 1, 3).reshape(B * S, C, D)
-        x = transformer(x, sd, base + "1.", spec, drop)
+        x = transformer(x, sd, base + "1.", spec, drop, "spectral")
     return x.reshape(B, S, C, D).permute(0, 2, 1, 3).reshape(B, spec.T, D)
 
 
@@ -344,7 +355,7 @@ def encoder_forward(img, sd, spec: Spec, pre: str = ""):
 
 
 def simmim_forward(img, sd, spec: Spec, bool_mask: torch.Tensor, idx: torch.Tensor,
-                   blockwise_decoder: bool = True, return_parts: bool = False, drop: float = 0.0,
+                   blockwise_decoder: bool = True, return_parts: bool = False, drop=0.0,
                    intermediate_losses: bool = False):
     """SimMIMSpatialSpectral.forward (vit_simmim_original.py:203-340) with the mask pair supplied
     from outside (the pair may be mutually inconsistent, SURVEY.md C3).  Dropout off; the SimMIM

@@ -12,6 +12,7 @@ import torch.nn.functional as F
 from maskedsst_b200 import _lib, ops
 from maskedsst_b200.input import RawTiles
 from oracle import maskedsst_oracle as O
+from tests import dropout_ref
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -91,11 +92,8 @@ def _run_embed(B, C_, G, p0, p1, D, nwb, mask_mode, with_ln, drop_p=0.0, seed=0,
     _lib.check(lib.msst_patch_embed_fwd(C.byref(dims), _p(img), *[_p(t) for t in prm[:7]], _p(mask_u8),
                                         _p(prm[7]) if mask is not None else None, _p(tokens), _p(pln), _st()))
     fac = None
-    if drop_p > 0:   # the embedding's dropout site is 1: the mask msst_dropout_apply draws at the same (seed, site)
-        ones = torch.ones(B * T * D, device=DEV)
-        fac = torch.empty_like(ones)
-        _lib.check(lib.msst_dropout_apply(_p(ones), _p(fac), B * T * D, drop_p, seed, 1, None, _st()))
-        fac = fac.view(B, T, D).double()
+    if drop_p > 0:   # the embedding's dropout site is 1, element row * D + f of the tokens: the host model of the mask
+        fac = torch.from_numpy(dropout_ref.elem_mask(drop_p, seed, 1, B * T * D)).view(B, T, D).double().to(DEV)
     ref = [t.double().requires_grad_(True) for t in prm]
     want, want_ln = _embed_ref(img.double(), ref, mask, C_, G, p0, p1, fac)
     assert _err(tokens, want) < 1e-5
