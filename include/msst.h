@@ -290,6 +290,32 @@ MSST_API int msst_scene_embed(const msst_scene_embed_dims* d, const float* token
                               msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * k-nearest-neighbour probing of embeddings (e.g. msst_scene_embed maps): cosine similarity, k best references per query, class vote.
+ *   msst_knn_prepare   x [n, dim] fp32 rows -> out [n, 3*dim] bf16: y = x / max(||x||, 1e-12) (F.normalize) split into three bf16
+ *                      parts y = hi + mid + lo, stored [hi | mid | lo].  Run once on the references and once per query chunk.
+ *   msst_knn_topk      scores [n_query, k] fp32 (descending) and index [n_query, k] int64 of the k references with the largest cosine
+ *                      similarity to each query, from prepared ref [n_ref, 3*dim] and query [n_query, 3*dim].  A score is
+ *                      sum_{i+j<=2} part_i(q) . part_j(r) with fp32 accumulation: |score - exact cosine| <= 2.4e-7 + the fp32
+ *                      accumulation error (DESIGN.md §3).  Order (score descending, reference index ascending): an equal score goes to the
+ *                      lower index.  Bitwise independent of how the queries are chunked.  No atomics.
+ *   msst_knn_vote      probs [n_query, nc] fp32 and pred [n_query] int64 from (scores, index) and ref_labels [n_ref] int64:
+ *                      w_j = exp((s_j - s_0) / temperature), probs[c] = sum_{j: label(index_j) == c} w_j / sum_j w_j (the DINO k-NN
+ *                      vote; subtracting the top score s_0 keeps exp in range), pred = argmax, lowest class on ties.
+ *                      temperature = +inf is the uniform vote.  A label outside [0, nc) casts no vote but its weight stays in the sum.
+ * Limits (MSST_ERR_ARG before any launch, outputs untouched): dim a multiple of 32 in [32, 256]; 1 <= k <= 64; k <= n_ref < 2^31;
+ * 1 <= nc <= 256; temperature > 0; no NULL pointer.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    int64_t n_ref, n_query;      /* reference rows, query rows of this call */
+    int dim, k;                  /* feature width, neighbours per query */
+} msst_knn_dims;
+MSST_API int msst_knn_prepare(const float* x, int64_t n, int dim, void* out, msst_stream_t stream);
+MSST_API int msst_knn_topk(const msst_knn_dims* d, const void* ref, const void* query, float* scores, int64_t* index,
+                           msst_stream_t stream);
+MSST_API int msst_knn_vote(int64_t n_query, int k, int64_t n_ref, const float* scores, const int64_t* index, const int64_t* ref_labels,
+                           int nc, float temperature, float* probs, int64_t* pred, msst_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * SimMIM decoder + masked L1 loss (vit_simmim_original.py:314-338, BlockwiseToPixels :9-40):
  *   pred[b,n,:] = W[blk] enc[b, idx[b,n], :] + bias[blk],  blk = idx / S (0 when n_weight_blocks == 1)
  *   target      = raw pixels of patch idx gathered from img (or target_tokens [B,T,P] if not NULL)

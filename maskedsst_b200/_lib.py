@@ -60,6 +60,10 @@ class SceneEmbedDims(C.Structure):   # msst_scene_embed_dims
     _fields_ = [(n, C.c_int) for n in ("B", "D", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n", "C", "p1")]
 
 
+class KnnDims(C.Structure):   # msst_knn_dims
+    _fields_ = [("n_ref", C.c_int64), ("n_query", C.c_int64), ("dim", C.c_int), ("k", C.c_int)]
+
+
 class DecodeDims(C.Structure):
     _fields_ = [("B", C.c_int), ("C", C.c_int), ("G", C.c_int), ("p0", C.c_int), ("p1", C.c_int), ("D", C.c_int),
                 ("nm", C.c_int), ("n_weight_blocks", C.c_int), ("raw", C.POINTER(RawInput))]
@@ -104,6 +108,9 @@ SIGNATURES = {
     "msst_cross_entropy_fwd_bwd": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
     "msst_scene_blend": (C.c_int, [C.POINTER(SceneDims), vp, vp, vp, vp, vp]),
     "msst_scene_embed": (C.c_int, [C.POINTER(SceneEmbedDims), vp, vp, vp, vp, vp]),
+    "msst_knn_prepare": (C.c_int, [vp, C.c_int64, C.c_int, vp, vp]),
+    "msst_knn_topk": (C.c_int, [C.POINTER(KnnDims), vp, vp, vp, vp, vp]),
+    "msst_knn_vote": (C.c_int, [C.c_int64, C.c_int, C.c_int64, vp, vp, vp, C.c_int, C.c_float, vp, vp, vp]),
     "msst_simmim_decode_l1_fwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 9 + [vp]),
     "msst_simmim_decode_l1_bwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 11 + [vp]),
     "msst_draw_masks": (C.c_int, [C.POINTER(MaskGenDims), vp, vp, vp]),

@@ -10,6 +10,10 @@ Whole-scene inference (`predict_scene`) lifts the three limits of that path: any
 snapped to the border), overlapping windows whose class probabilities are blended per pixel on the device (csrc/scene.cu, no seams
 every window), and chunks of windows so that a scene of any size fits.  `confusion_matrix` / `classification_metrics` score the
 resulting map as hyperspectral classification results are reported: overall accuracy, average (macro) accuracy and Cohen's kappa.
+
+`embed_scene` returns per-pixel encoder features of whole scenes.  `knn_neighbors` / `knn_classify` / `knn_scene` probe them with
+k-nearest neighbours by cosine similarity (csrc/knn.cu).  The references stream through the tensor cores past each query tile, and
+every query keeps its running top k on chip, so the [queries, references] score matrix is never stored.
 """
 import ctypes
 import math
@@ -237,3 +241,135 @@ def classification_metrics(conf):
     pe = float((rows * cols).sum() / (total * total))
     kappa = (oa - pe) / (1.0 - pe) if pe != 1.0 else float("nan")
     return dict(oa=oa, aa=aa, kappa=kappa, per_class_acc=per_class)
+
+
+KNN_MAX_K, KNN_MAX_DIM, KNN_MAX_CLASSES = 64, 256, 256
+
+
+def _knn_features(who, name, x):
+    if not isinstance(x, torch.Tensor) or x.dim() != 2 or x.dtype != torch.float32 or not x.is_cuda:
+        raise ValueError(f"{who}: {name} must be a 2-D fp32 CUDA tensor [rows, dim], got "
+                         f"{tuple(x.shape) if isinstance(x, torch.Tensor) else type(x).__name__}"
+                         f"{f' {x.dtype} on {x.device}' if isinstance(x, torch.Tensor) else ''}")
+    D = x.shape[1]
+    if D % 32 or not 32 <= D <= KNN_MAX_DIM:
+        raise ValueError(f"{who}: feature width {D} must be a multiple of 32 in [32, {KNN_MAX_DIM}]")
+    return x.contiguous()
+
+
+def _knn_check(who, ref, query, k, batch_queries):
+    ref, query = _knn_features(who, "ref", ref), _knn_features(who, "query", query)
+    if ref.shape[1] != query.shape[1] or ref.device != query.device:
+        raise ValueError(f"{who}: ref {tuple(ref.shape)} on {ref.device} and query {tuple(query.shape)} on {query.device} disagree")
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= KNN_MAX_K:
+        raise ValueError(f"{who}: k={k!r} must be an int in [1, {KNN_MAX_K}]")
+    if not k <= ref.shape[0] < 2 ** 31:
+        raise ValueError(f"{who}: {ref.shape[0]} reference rows; need k={k} <= rows < 2^31")
+    if isinstance(batch_queries, bool) or not isinstance(batch_queries, int) or batch_queries < 1:
+        raise ValueError(f"{who}: batch_queries={batch_queries!r} must be a positive int")
+    return ref, query
+
+
+def _knn_prepare(x):
+    """msst_knn_prepare: rows [n, D] fp32 -> normalised, split operand rows [n, 3 * D] bf16."""
+    out = torch.empty(x.shape[0], 3 * x.shape[1], device=x.device, dtype=torch.bfloat16)
+    _lib.check(_lib.lib().msst_knn_prepare(x.data_ptr(), x.shape[0], x.shape[1], out.data_ptr(),
+                                           torch.cuda.current_stream(x.device).cuda_stream))
+    return out
+
+
+def _knn_chunks(ref, query, k, batch_queries):
+    """Yields (first, last, scores [n, k], index [n, k]) for the query chunks [first, last) in order."""
+    N, D = ref.shape
+    rp = _knn_prepare(ref)
+    stream = torch.cuda.current_stream(ref.device).cuda_stream
+    for first in range(0, query.shape[0], batch_queries):
+        last = min(first + batch_queries, query.shape[0])
+        qp = _knn_prepare(query[first:last])
+        scores = torch.empty(last - first, k, device=ref.device, dtype=torch.float32)
+        index = torch.empty(last - first, k, device=ref.device, dtype=torch.int64)
+        dims = _lib.KnnDims(N, last - first, D, k)
+        _lib.check(_lib.lib().msst_knn_topk(ctypes.byref(dims), rp.data_ptr(), qp.data_ptr(), scores.data_ptr(), index.data_ptr(), stream))
+        yield first, last, scores, index
+
+
+@torch.no_grad()
+def knn_neighbors(ref, query, k, *, batch_queries=262144):
+    """The k nearest references of every query by cosine similarity, found on the device without the [Q, N] score matrix.
+
+    ref [N, D], query [Q, D]: fp32 CUDA tensors, D a multiple of 32 in [32, 256], 1 <= k <= 64, k <= N < 2^31.  Rows are normalised as
+    F.normalize does (eps 1e-12), so a zero row scores 0 against everything.  Scores are fp32-accurate (three-part bf16 split on the
+    tensor cores, DESIGN.md §3).  Queries run in chunks of batch_queries; the result is bitwise the same for any chunk size.
+    -> (scores [Q, k] fp32, descending; index [Q, k] int64), ordered by (score descending, reference index ascending)."""
+    ref, query = _knn_check("knn_neighbors", ref, query, k, batch_queries)
+    scores = torch.empty(query.shape[0], k, device=ref.device, dtype=torch.float32)
+    index = torch.empty(query.shape[0], k, device=ref.device, dtype=torch.int64)
+    for first, last, s, i in _knn_chunks(ref, query, k, batch_queries):
+        scores[first:last], index[first:last] = s, i
+    return scores, index
+
+
+def _knn_vote_args(who, ref, ref_labels, num_classes, temperature):
+    if isinstance(num_classes, bool) or not isinstance(num_classes, int) or not 1 <= num_classes <= KNN_MAX_CLASSES:
+        raise ValueError(f"{who}: num_classes={num_classes!r} must be an int in [1, {KNN_MAX_CLASSES}]")
+    t = float(temperature)
+    if not t > 0:   # NaN fails too
+        raise ValueError(f"{who}: temperature={temperature!r} must be > 0 (float('inf') for a uniform vote)")
+    if (not isinstance(ref_labels, torch.Tensor) or ref_labels.shape != (ref.shape[0],) or ref_labels.device != ref.device
+            or ref_labels.dtype.is_floating_point or ref_labels.dtype.is_complex or ref_labels.dtype == torch.bool):
+        raise ValueError(f"{who}: ref_labels must be an integer tensor [{ref.shape[0]}] on {ref.device}, got "
+                         f"{tuple(ref_labels.shape) if isinstance(ref_labels, torch.Tensor) else type(ref_labels).__name__}")
+    ref_labels = ref_labels.to(torch.int64).contiguous()
+    if bool(((ref_labels < 0) | (ref_labels >= num_classes)).any()):
+        raise ValueError(f"{who}: reference labels outside [0, {num_classes})")
+    return ref_labels, t
+
+
+@torch.no_grad()
+def knn_classify(ref, ref_labels, query, *, num_classes, k=20, temperature=0.07, batch_queries=262144):
+    """k-NN classification of queries by labelled references (the usual probe of a self-supervised encoder).
+
+    ref, query, k, batch_queries: as in knn_neighbors.  ref_labels [N] integers in [0, num_classes), num_classes <= 256.
+    Each query's k nearest references vote with weight w_j = exp((s_j - s_0) / temperature) (s: cosine similarities, s_0 the largest;
+    the DINO k-NN protocol), normalised to sum 1; temperature=float('inf') gives the uniform vote.
+    -> (probs [Q, num_classes] fp32, pred [Q] int64 = argmax, lowest class on ties)."""
+    ref, query = _knn_check("knn_classify", ref, query, k, batch_queries)
+    ref_labels, t = _knn_vote_args("knn_classify", ref, ref_labels, num_classes, temperature)
+    probs = torch.empty(query.shape[0], num_classes, device=ref.device, dtype=torch.float32)
+    pred = torch.empty(query.shape[0], device=ref.device, dtype=torch.int64)
+    stream = torch.cuda.current_stream(ref.device).cuda_stream
+    for first, last, s, i in _knn_chunks(ref, query, k, batch_queries):
+        _lib.check(_lib.lib().msst_knn_vote(last - first, k, ref.shape[0], s.data_ptr(), i.data_ptr(), ref_labels.data_ptr(), num_classes,
+                                            t, probs[first:last].data_ptr(), pred[first:last].data_ptr(), stream))
+    return probs, pred
+
+
+@torch.no_grad()
+def knn_scene(model, scene, train_labels, *, num_classes, k=20, temperature=0.07, stride=None, weight=None, batch_windows=4096,
+              ignore_index=-1, batch_queries=262144):
+    """k-NN probe of an encoder on whole scenes: embed_scene features, the labelled pixels as references, every pixel as a query.
+
+    model, scene, stride, weight, batch_windows: as in embed_scene (a SimMIMSpatialSpectral checkpoint works directly).
+    train_labels [B, H, W] integers on the scene's device: a pixel is a reference when its label is != ignore_index and in
+    [0, num_classes) (the rule of confusion_matrix).  k, temperature, batch_queries: as in knn_classify.
+    Score the result against held-out labels with confusion_matrix / classification_metrics.
+    -> (probs [B, num_classes, H, W] fp32, pred [B, H, W] int64)."""
+    tiles = scene.tiles if isinstance(scene, RawTiles) else scene
+    if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
+        raise ValueError("knn_scene: scene must be a [B, C, H, W] tensor or RawTiles")
+    B, _, H, W = tiles.shape
+    if (not isinstance(train_labels, torch.Tensor) or train_labels.shape != (B, H, W) or train_labels.dtype.is_floating_point
+            or train_labels.dtype == torch.bool or train_labels.device != tiles.device):
+        raise ValueError(f"knn_scene: train_labels must be an integer tensor [{B}, {H}, {W}] on {tiles.device}")
+    if not tiles.is_cuda:
+        raise ValueError("knn_scene: the scene must be on a CUDA device")
+    if isinstance(num_classes, bool) or not isinstance(num_classes, int) or not 1 <= num_classes <= KNN_MAX_CLASSES:
+        raise ValueError(f"knn_scene: num_classes={num_classes!r} must be an int in [1, {KNN_MAX_CLASSES}]")
+    labels = train_labels.reshape(-1).to(torch.int64)
+    valid = (labels != ignore_index) & (labels >= 0) & (labels < num_classes)
+    feats = embed_scene(model, scene, stride=stride, weight=weight, batch_windows=batch_windows)   # [B, D, H, W]
+    D = feats.shape[1]
+    flat = feats.permute(0, 2, 3, 1).reshape(B * H * W, D)   # the one copy: pixels as rows
+    probs, pred = knn_classify(flat[valid], labels[valid], flat, num_classes=num_classes, k=k, temperature=temperature,
+                               batch_queries=batch_queries)
+    return probs.reshape(B, H, W, num_classes).permute(0, 3, 1, 2).contiguous(), pred.reshape(B, H, W)
