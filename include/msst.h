@@ -316,6 +316,45 @@ MSST_API int msst_knn_vote(int64_t n_query, int k, int64_t n_ref, const float* s
                            int nc, float temperature, float* probs, int64_t* pred, msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Linear probing of embeddings: softmax regression on frozen fp32 feature rows, H heads (learning rate / weight decay pairs)
+ * trained in the same launches.
+ *   z = LN(x):   mean and biased variance over dim, eps 1e-5, no affine (F.layer_norm(x, (dim,)), the default head's LayerNorm
+ *                with weight 1 and bias 0); one device function normalises a row in training and in prediction.
+ *   params [heads][nc*dim + nc]: head h is W_h [nc, dim] row-major followed by b_h [nc]; logits = W_h z + b_h.  The Adam moments
+ *                m, v use the same layout.
+ *   msst_linprobe_workspace  bytes of the workspace of msst_linprobe_grad / msst_linprobe_update for d->batch rows:
+ *                ceil(batch / 128) * heads * (nc*dim + nc + 1) * 4; -1 (and the error message) on bad dims.
+ *   msst_linprobe_grad       rows i = 0 .. batch-1 of the minibatch are x[index[i]] with label labels[index[i]].  Per 128-row slice
+ *                of the minibatch and head it writes to the workspace sum_i (softmax(W_h z_i + b_h) - onehot(y_i)) (x) [z_i | 1]
+ *                (the slice's dW_h and db_h sums) and sum_i CE_i.  A row whose index is outside [0, n) or whose label is outside
+ *                [0, nc) contributes nothing (it still counts in the batch size).
+ *   msst_linprobe_update     sums the slices' partials in ascending slice order, divides by batch and applies torch.optim.AdamW to
+ *                every head in one launch: betas (0.9, 0.999), eps 1e-8, decoupled weight decay wd[h] on W_h and b_h, learning
+ *                rate lr[h], 1-based step `step`, no clamp.  loss_sum [heads] = the step's CE sums (ascending slice order).
+ *   msst_linprobe_predict    probs [n_query, nc] = softmax(W z + b), pred [n_query] int64 = argmax of probs, lowest class on ties,
+ *                for the single head `params` [nc*dim + nc].
+ * Deterministic: every sum runs in a fixed order (no atomics), a (slice, head) pair is one CTA and a parameter one thread, so the
+ * results are bitwise independent of the SM count, of how many heads are trained together, and of how queries are chunked.
+ * Limits (MSST_ERR_ARG before any launch, outputs untouched): dim a multiple of 32 in [32, 256]; 1 <= nc <= 256; 1 <= heads <= 16;
+ * 1 <= n < 2^31; 1 <= batch; step >= 1; every lr[h], wd[h] finite and >= 0; 1 <= n_query < 2^31; no NULL pointer.
+ * ------------------------------------------------------------------------------------------- */
+#define MSST_LINPROBE_MAX_HEADS 16
+typedef struct {
+    int64_t n;                   /* rows of x (and labels) */
+    int dim, nc, heads;          /* feature width, classes, heads */
+    int batch;                   /* rows of this minibatch (entries of index) */
+    int step;                    /* 1-based AdamW step (msst_linprobe_update) */
+    float lr[MSST_LINPROBE_MAX_HEADS], wd[MSST_LINPROBE_MAX_HEADS];   /* per head; entries >= heads are ignored */
+} msst_linprobe_dims;
+MSST_API int64_t msst_linprobe_workspace(const msst_linprobe_dims* d);
+MSST_API int msst_linprobe_grad(const msst_linprobe_dims* d, const float* x, const int64_t* labels, const int64_t* index,
+                                const float* params, float* workspace, msst_stream_t stream);
+MSST_API int msst_linprobe_update(const msst_linprobe_dims* d, const float* workspace, float* params, float* m, float* v,
+                                  float* loss_sum, msst_stream_t stream);
+MSST_API int msst_linprobe_predict(int64_t n_query, int dim, int nc, const float* x, const float* params, float* probs, int64_t* pred,
+                                   msst_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * SimMIM decoder + masked L1 loss (vit_simmim_original.py:314-338, BlockwiseToPixels :9-40):
  *   pred[b,n,:] = W[blk] enc[b, idx[b,n], :] + bias[blk],  blk = idx / S (0 when n_weight_blocks == 1)
  *   target      = raw pixels of patch idx gathered from img (or target_tokens [B,T,P] if not NULL)

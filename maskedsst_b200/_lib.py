@@ -64,6 +64,11 @@ class KnnDims(C.Structure):   # msst_knn_dims
     _fields_ = [("n_ref", C.c_int64), ("n_query", C.c_int64), ("dim", C.c_int), ("k", C.c_int)]
 
 
+class LinprobeDims(C.Structure):   # msst_linprobe_dims
+    _fields_ = [("n", C.c_int64), ("dim", C.c_int), ("nc", C.c_int), ("heads", C.c_int), ("batch", C.c_int), ("step", C.c_int),
+                ("lr", C.c_float * 16), ("wd", C.c_float * 16)]
+
+
 class DecodeDims(C.Structure):
     _fields_ = [("B", C.c_int), ("C", C.c_int), ("G", C.c_int), ("p0", C.c_int), ("p1", C.c_int), ("D", C.c_int),
                 ("nm", C.c_int), ("n_weight_blocks", C.c_int), ("raw", C.POINTER(RawInput))]
@@ -111,6 +116,10 @@ SIGNATURES = {
     "msst_knn_prepare": (C.c_int, [vp, C.c_int64, C.c_int, vp, vp]),
     "msst_knn_topk": (C.c_int, [C.POINTER(KnnDims), vp, vp, vp, vp, vp]),
     "msst_knn_vote": (C.c_int, [C.c_int64, C.c_int, C.c_int64, vp, vp, vp, C.c_int, C.c_float, vp, vp, vp]),
+    "msst_linprobe_workspace": (C.c_int64, [C.POINTER(LinprobeDims)]),
+    "msst_linprobe_grad": (C.c_int, [C.POINTER(LinprobeDims), vp, vp, vp, vp, vp, vp]),
+    "msst_linprobe_update": (C.c_int, [C.POINTER(LinprobeDims), vp, vp, vp, vp, vp, vp]),
+    "msst_linprobe_predict": (C.c_int, [C.c_int64, C.c_int, C.c_int, vp, vp, vp, vp, vp]),
     "msst_simmim_decode_l1_fwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 9 + [vp]),
     "msst_simmim_decode_l1_bwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 11 + [vp]),
     "msst_draw_masks": (C.c_int, [C.POINTER(MaskGenDims), vp, vp, vp]),

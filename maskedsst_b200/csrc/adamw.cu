@@ -2,21 +2,9 @@
 // (pretrain.py:71-73, SURVEY C9) and the data-parallel 1/world scale folded in, optionally emitting the bf16 copy
 // of the updated weights that the tcgen05 GEMMs consume.  Update rules: torch.optim.AdamW / Adam as configured by
 // src/utils.py:36-44 and finetune.py:133-135.  HBM-bound: 28 B/param (read g,p,m,v; write p,m,v) [+2 B bf16].
-#include "common.cuh"
+#include "adam.cuh"
 
 namespace msst {
-
-struct AdamK { float lr, b1, b2, eps, wd, clamp, gscale, inv_bc1, inv_sqrt_bc2; int decoupled; const int* step_dev; };
-
-__device__ __forceinline__ void adam_one(const AdamK& a, float& p, float g, float& m, float& v) {
-    g *= a.gscale;
-    if (a.clamp > 0.f) g = fminf(fmaxf(g, -a.clamp), a.clamp);
-    if (a.decoupled) p *= (1.f - a.lr * a.wd); else g = fmaf(a.wd, p, g);
-    m = a.b1 * m + (1.f - a.b1) * g;
-    v = a.b2 * v + (1.f - a.b2) * g * g;
-    const float denom = sqrtf(v) * a.inv_sqrt_bc2 + a.eps;
-    p -= (a.lr * a.inv_bc1) * (m / denom);
-}
 
 __global__ void __launch_bounds__(256) adam_kernel(AdamK a, float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                    float* __restrict__ v, __nv_bfloat16* __restrict__ bf, int64_t n, int vec) {
@@ -65,6 +53,7 @@ extern "C" int msst_adam_step(const msst_adam_args* a, float* p, const float* g,
     AdamK k;
     k.lr = a->lr; k.b1 = a->beta1; k.b2 = a->beta2; k.eps = a->eps; k.wd = a->weight_decay; k.clamp = a->clamp;
     k.gscale = a->grad_scale; k.decoupled = a->decoupled;
+    k.omb1 = 1.f - k.b1; k.omb2 = 1.f - k.b2;
     const int st = a->step >= 1 ? a->step : 1;
     k.inv_bc1 = (float)(1.0 / (1.0 - pow((double)a->beta1, (double)st)));
     k.inv_sqrt_bc2 = (float)(1.0 / sqrt(1.0 - pow((double)a->beta2, (double)st)));

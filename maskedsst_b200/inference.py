@@ -14,6 +14,12 @@ resulting map as hyperspectral classification results are reported: overall accu
 `embed_scene` returns per-pixel encoder features of whole scenes.  `knn_neighbors` / `knn_classify` / `knn_scene` probe them with
 k-nearest neighbours by cosine similarity (csrc/knn.cu).  The references stream through the tensor cores past each query tile, and
 every query keeps its running top k on chip, so the [queries, references] score matrix is never stored.
+
+`linear_probe_fit` / `LinearProbe` / `linear_probe_scene` are the other standard probe: softmax regression on LayerNorm'ed frozen
+features, trained with AdamW for several (lr, weight_decay) heads at once (csrc/linprobe.cu: per minibatch one gradient launch, which
+writes fixed 128-row slice partials for every head, and one launch that sums them in order and applies AdamW to every head).  Fits are
+bitwise reproducible and each head is bitwise the head fitted alone.  `LinearProbe.load_into` writes a probe into the default head of
+a ViTSpatialSpectral, whose LayerNorm and per-patch Linear then compute exactly the probe's function of the embed_scene features.
 """
 import ctypes
 import math
@@ -354,22 +360,248 @@ def knn_scene(model, scene, train_labels, *, num_classes, k=20, temperature=0.07
     [0, num_classes) (the rule of confusion_matrix).  k, temperature, batch_queries: as in knn_classify.
     Score the result against held-out labels with confusion_matrix / classification_metrics.
     -> (probs [B, num_classes, H, W] fp32, pred [B, H, W] int64)."""
+    labels, valid = _scene_labels("knn_scene", scene, train_labels, num_classes, ignore_index)
+    feats = embed_scene(model, scene, stride=stride, weight=weight, batch_windows=batch_windows)   # [B, D, H, W]
+    flat = _pixel_rows(feats)
+    probs, pred = knn_classify(flat[valid], labels[valid], flat, num_classes=num_classes, k=k, temperature=temperature,
+                               batch_queries=batch_queries)
+    return _pixel_map(probs, feats), pred.reshape(feats.shape[0], *feats.shape[2:])
+
+
+def _scene_labels(who, scene, train_labels, num_classes, ignore_index, name="train_labels"):
+    """Checks a whole-scene probe's scene and per-pixel labels -> (labels [B*H*W] int64, valid [B*H*W] bool).  A pixel is valid when
+    its label is != ignore_index and in [0, num_classes): the rule of confusion_matrix."""
     tiles = scene.tiles if isinstance(scene, RawTiles) else scene
     if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
-        raise ValueError("knn_scene: scene must be a [B, C, H, W] tensor or RawTiles")
+        raise ValueError(f"{who}: scene must be a [B, C, H, W] tensor or RawTiles")
     B, _, H, W = tiles.shape
     if (not isinstance(train_labels, torch.Tensor) or train_labels.shape != (B, H, W) or train_labels.dtype.is_floating_point
             or train_labels.dtype == torch.bool or train_labels.device != tiles.device):
-        raise ValueError(f"knn_scene: train_labels must be an integer tensor [{B}, {H}, {W}] on {tiles.device}")
+        raise ValueError(f"{who}: {name} must be an integer tensor [{B}, {H}, {W}] on {tiles.device}")
     if not tiles.is_cuda:
-        raise ValueError("knn_scene: the scene must be on a CUDA device")
+        raise ValueError(f"{who}: the scene must be on a CUDA device")
     if isinstance(num_classes, bool) or not isinstance(num_classes, int) or not 1 <= num_classes <= KNN_MAX_CLASSES:
-        raise ValueError(f"knn_scene: num_classes={num_classes!r} must be an int in [1, {KNN_MAX_CLASSES}]")
+        raise ValueError(f"{who}: num_classes={num_classes!r} must be an int in [1, {KNN_MAX_CLASSES}]")
     labels = train_labels.reshape(-1).to(torch.int64)
-    valid = (labels != ignore_index) & (labels >= 0) & (labels < num_classes)
+    return labels, (labels != ignore_index) & (labels >= 0) & (labels < num_classes)
+
+
+def _pixel_rows(feats):
+    """[B, D, H, W] -> [B*H*W, D]: the one copy that makes pixels rows."""
+    return feats.permute(0, 2, 3, 1).reshape(-1, feats.shape[1])
+
+
+def _pixel_map(rows, feats):
+    """[B*H*W, nc] per-pixel rows -> [B, nc, H, W] over the scenes of feats [B, D, H, W]."""
+    B, _, H, W = feats.shape
+    return rows.reshape(B, H, W, rows.shape[1]).permute(0, 3, 1, 2).contiguous()
+
+
+LINPROBE_MAX_HEADS = 16
+
+
+def _linprobe_heads(who, heads):
+    try:
+        pairs = [(float(lr), float(wd)) for lr, wd in heads]
+    except (TypeError, ValueError):
+        raise ValueError(f"{who}: heads must be a sequence of (lr, weight_decay) pairs, got {heads!r}") from None
+    if not 1 <= len(pairs) <= LINPROBE_MAX_HEADS:
+        raise ValueError(f"{who}: {len(pairs)} heads; need 1 to {LINPROBE_MAX_HEADS}")
+    for lr, wd in pairs:
+        if not (0 <= lr < math.inf and 0 <= wd < math.inf):   # NaN fails too
+            raise ValueError(f"{who}: lr={lr!r} and weight_decay={wd!r} must be finite and >= 0")
+    return pairs
+
+
+def _int_arg(who, name, v, lo):
+    if isinstance(v, bool) or not isinstance(v, int) or v < lo:
+        raise ValueError(f"{who}: {name}={v!r} must be an int >= {lo}")
+
+
+def _labelled_rows(who, x, y, num_classes, name):
+    x = _knn_features(who, name, x)
+    if not x.shape[0] < 2 ** 31 or x.shape[0] < 1:
+        raise ValueError(f"{who}: {name} has {x.shape[0]} rows; need 1 <= rows < 2^31")
+    if (not isinstance(y, torch.Tensor) or y.shape != (x.shape[0],) or y.device != x.device or y.dtype.is_floating_point
+            or y.dtype.is_complex or y.dtype == torch.bool):
+        raise ValueError(f"{who}: labels of {name} must be an integer tensor [{x.shape[0]}] on {x.device}, got "
+                         f"{tuple(y.shape) if isinstance(y, torch.Tensor) else type(y).__name__}")
+    y = y.to(torch.int64).contiguous()
+    if bool(((y < 0) | (y >= num_classes)).any()):
+        raise ValueError(f"{who}: labels of {name} outside [0, {num_classes})")
+    return x, y
+
+
+def _linprobe_dims(n, dim, nc, heads, batch=1, step=1):
+    d = _lib.LinprobeDims(n, dim, nc, len(heads), batch, step)
+    for h, (lr, wd) in enumerate(heads):
+        d.lr[h], d.wd[h] = lr, wd
+    return d
+
+
+def _linprobe_grad(dims, x, labels, index, params, workspace):
+    """One msst_linprobe_grad launch: the minibatch x[index] -> per-slice partials in workspace (dims.batch = index.numel())."""
+    _lib.check(_lib.lib().msst_linprobe_grad(ctypes.byref(dims), x.data_ptr(), labels.data_ptr(), index.data_ptr(), params.data_ptr(),
+                                             workspace.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream))
+
+
+def _linprobe_update(dims, workspace, params, m, v, loss_sum):
+    """One msst_linprobe_update launch: AdamW step dims.step of every head; loss_sum [H] = the step's CE sums."""
+    _lib.check(_lib.lib().msst_linprobe_update(ctypes.byref(dims), workspace.data_ptr(), params.data_ptr(), m.data_ptr(), v.data_ptr(),
+                                               loss_sum.data_ptr(), torch.cuda.current_stream(params.device).cuda_stream))
+
+
+class LinearProbe:
+    """A fitted linear probe: per head h, W[h] [nc, dim] and b[h] [nc] on LN(x) (F.layer_norm(x, (dim,)), no affine).
+
+    params [H, nc*dim + nc] fp32 (CUDA): head h is W_h row-major followed by b_h (the msst_linprobe layout); W / b are views.
+    heads: the (lr, weight_decay) pairs; train_loss [epochs, H] float64: mean training CE per epoch; val_acc [H] float64 or None: OA of
+    each head on the validation rows; best: the head predict / load_into use by default (argmax of val_acc, lowest index on ties)."""
+
+    def __init__(self, params, num_classes, dim, heads, train_loss=None, val_acc=None, best=0):
+        self.params, self.num_classes, self.dim, self.heads = params, num_classes, dim, list(heads)
+        self.train_loss, self.val_acc, self.best = train_loss, val_acc, best
+
+    @property
+    def W(self):
+        return self.params[:, :self.num_classes * self.dim].view(-1, self.num_classes, self.dim)
+
+    @property
+    def b(self):
+        return self.params[:, self.num_classes * self.dim:]
+
+    def _head(self, who, head):
+        head = self.best if head is None else head
+        if isinstance(head, bool) or not isinstance(head, int) or not 0 <= head < self.params.shape[0]:
+            raise ValueError(f"{who}: head={head!r} must be an int in [0, {self.params.shape[0]})")
+        return head
+
+    @torch.no_grad()
+    def predict(self, x, *, head=None, batch_queries=262144):
+        """x [Q, dim] fp32 CUDA -> (probs [Q, nc] fp32 = softmax(W z + b), pred [Q] int64 = argmax, lowest class on ties) of one head
+        (default: best).  Queries run in chunks of batch_queries; the result is bitwise the same for any chunk size."""
+        head = self._head("LinearProbe.predict", head)
+        x = _knn_features("LinearProbe.predict", "x", x)
+        if x.shape[1] != self.dim or x.device != self.params.device:
+            raise ValueError(f"LinearProbe.predict: x {tuple(x.shape)} on {x.device} does not match dim {self.dim} on {self.params.device}")
+        if isinstance(batch_queries, bool) or not isinstance(batch_queries, int) or batch_queries < 1:
+            raise ValueError(f"LinearProbe.predict: batch_queries={batch_queries!r} must be a positive int")
+        nc, Q = self.num_classes, x.shape[0]
+        probs = torch.empty(Q, nc, device=x.device, dtype=torch.float32)
+        pred = torch.empty(Q, device=x.device, dtype=torch.int64)
+        p = self.params[head].contiguous()
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        for first in range(0, Q, batch_queries):
+            last = min(first + batch_queries, Q)
+            _lib.check(_lib.lib().msst_linprobe_predict(last - first, self.dim, nc, x[first:last].data_ptr(), p.data_ptr(),
+                                                        probs[first:last].data_ptr(), pred[first:last].data_ptr(), stream))
+        return probs, pred
+
+    @torch.no_grad()
+    def load_into(self, model, head=None):
+        """Writes head `head` (default: best) into the default head of a ViTSpatialSpectral: LayerNorm weight 1 and bias 0 (so the
+        head normalises as the probe does), the Linear's rows (pi*p1 + pj)*nc + c = W[c] and bias b[c] for every sub-pixel (pi, pj)
+        of a spatial patch (HeadRearrange order).  The model then classifies windows as the probe classifies their embed_scene
+        features.  Writes in place (copy_), so optimiser state built over the model's parameters stays valid."""
+        head = self._head("LinearProbe.load_into", head)
+        if not isinstance(model, ViTSpatialSpectral):
+            raise ValueError(f"LinearProbe.load_into: needs a ViTSpatialSpectral, got {type(model).__name__}")
+        if model.pixelwise or model.spectral_mlp_head:
+            raise ValueError("LinearProbe.load_into: only the default head (LayerNorm + Linear per spatial patch) can take a probe; "
+                             "this model has a pixelwise or spectral-MLP head")
+        if model.dim != self.dim or model.num_classes != self.num_classes:
+            raise ValueError(f"LinearProbe.load_into: model dim {model.dim} / num_classes {model.num_classes} do not match the probe's "
+                             f"{self.dim} / {self.num_classes}")
+        ln, lin = model.mlp_head[0], model.mlp_head[1]
+        reps = model.patch_height * model.patch_width
+        ln.weight.fill_(1.0)
+        ln.bias.zero_()
+        lin.weight.copy_(self.W[head].repeat(reps, 1))
+        lin.bias.copy_(self.b[head].repeat(reps))
+
+
+@torch.no_grad()
+def linear_probe_fit(ref, ref_labels, *, num_classes, heads=((1e-3, 0.0),), epochs=100, batch_size=4096, seed=0, val=None):
+    """Fits linear probes (softmax regression) on frozen features: the usual second probe of a self-supervised encoder next to k-NN,
+    and the first step of linear-probe-then-fine-tune (LinearProbe.load_into).
+
+    ref [N, dim] fp32 CUDA (dim a multiple of 32 in [32, 256], N < 2^31), ref_labels [N] integers in [0, num_classes), num_classes <= 256.
+    Rows are normalised as F.layer_norm(x, (dim,)) does (no affine).  heads: 1 to 16 (lr, weight_decay) pairs, trained together in
+    the same launches; W and b start at 0.  Per epoch: perm = torch.randperm(N, generator=g, device=ref.device) with one
+    g = torch.Generator(ref.device).manual_seed(seed) for the whole fit, minibatches = consecutive slices of batch_size rows of perm
+    (the last may be shorter), the minibatch mean of cross-entropy, torch.optim.AdamW (betas (0.9, 0.999), eps 1e-8, decoupled decay on
+    W and b, one 1-based step counter over the fit).  Bitwise reproducible, and each head is bitwise the head fitted alone.
+    val: optional (x_val [M, dim], y_val [M]): val_acc[h] = OA of head h on it, best = argmax (lowest index on ties).  Without val
+    only one head is allowed (there is nothing to choose with).
+    -> LinearProbe with train_loss [epochs, H] float64: per epoch the sum of its steps' CE sums, added in step order, over N."""
+    who = "linear_probe_fit"
+    if isinstance(num_classes, bool) or not isinstance(num_classes, int) or not 1 <= num_classes <= KNN_MAX_CLASSES:
+        raise ValueError(f"{who}: num_classes={num_classes!r} must be an int in [1, {KNN_MAX_CLASSES}]")
+    ref, ref_labels = _labelled_rows(who, ref, ref_labels, num_classes, "ref")
+    heads = _linprobe_heads(who, heads)
+    _int_arg(who, "epochs", epochs, 1)
+    _int_arg(who, "batch_size", batch_size, 1)
+    _int_arg(who, "seed", seed, 0)
+    if val is not None:
+        if not isinstance(val, (tuple, list)) or len(val) != 2:
+            raise ValueError(f"{who}: val must be a pair (x_val, y_val)")
+        xv, yv = _labelled_rows(who, val[0], val[1], num_classes, "val")
+        if xv.shape[1] != ref.shape[1] or xv.device != ref.device:
+            raise ValueError(f"{who}: val rows {tuple(xv.shape)} on {xv.device} do not match ref {tuple(ref.shape)} on {ref.device}")
+    elif len(heads) > 1:
+        raise ValueError(f"{who}: {len(heads)} heads need val=(x_val, y_val) to choose the best one")
+    N, D = ref.shape
+    H, nc, dev = len(heads), num_classes, ref.device
+    batch = min(batch_size, N)
+    params = torch.zeros(H, nc * D + nc, device=dev, dtype=torch.float32)
+    m, v = torch.zeros_like(params), torch.zeros_like(params)
+    dims = _linprobe_dims(N, D, nc, heads, batch=batch)
+    workspace = torch.empty(_lib.lib().msst_linprobe_workspace(ctypes.byref(dims)) // 4, device=dev, dtype=torch.float32)
+    steps_per_epoch = -(-N // batch)
+    loss = torch.empty(epochs * steps_per_epoch, H, device=dev, dtype=torch.float32)
+    g = torch.Generator(device=dev).manual_seed(seed)
+    step = 0
+    for _ in range(epochs):
+        perm = torch.randperm(N, generator=g, device=dev)
+        for first in range(0, N, batch):
+            idx = perm[first:first + batch]
+            step += 1
+            dims.batch, dims.step = idx.numel(), step
+            _linprobe_grad(dims, ref, ref_labels, idx, params, workspace)
+            _linprobe_update(dims, workspace, params, m, v, loss[step - 1])
+    sums = loss.cpu().double().numpy().reshape(epochs, steps_per_epoch, H).cumsum(axis=1)[:, -1]   # cumsum: in step order
+    probe = LinearProbe(params, nc, D, heads, train_loss=torch.from_numpy(sums / N))
+    if val is not None:
+        acc = [float((probe.predict(xv, head=h)[1] == yv).double().mean()) for h in range(H)]
+        probe.val_acc = torch.tensor(acc, dtype=torch.float64)
+        probe.best = int(torch.argmax(probe.val_acc))
+    return probe
+
+
+@torch.no_grad()
+def linear_probe_scene(model, scene, train_labels, *, num_classes, val_labels=None, heads=((1e-3, 0.0),), epochs=100, batch_size=4096,
+                       seed=0, stride=None, weight=None, batch_windows=4096, ignore_index=-1, batch_queries=262144):
+    """Linear probe of an encoder on whole scenes: embed_scene features, fitted on the labelled pixels of train_labels (validated on
+    those of val_labels), then every pixel predicted.
+
+    model, scene, stride, weight, batch_windows: as in embed_scene (a SimMIMSpatialSpectral checkpoint works directly).
+    train_labels / val_labels [B, H, W] integers on the scene's device: a pixel is used when its label is != ignore_index and in
+    [0, num_classes) (the rule of confusion_matrix).  heads, epochs, batch_size, seed: as in linear_probe_fit (several heads need
+    val_labels).  Score the result against held-out labels with confusion_matrix / classification_metrics.
+    -> (probs [B, num_classes, H, W] fp32, pred [B, H, W] int64 of the best head, the LinearProbe)."""
+    who = "linear_probe_scene"
+    labels, valid = _scene_labels(who, scene, train_labels, num_classes, ignore_index)
+    if val_labels is not None:
+        vlabels, vvalid = _scene_labels(who, scene, val_labels, num_classes, ignore_index, name="val_labels")
+    _linprobe_heads(who, heads)
+    if val_labels is None and len(heads) > 1:
+        raise ValueError(f"{who}: {len(heads)} heads need val_labels to choose the best one")
+    if not bool(valid.any()) or (val_labels is not None and not bool(vvalid.any())):
+        raise ValueError(f"{who}: train_labels and val_labels need at least one labelled pixel each")
     feats = embed_scene(model, scene, stride=stride, weight=weight, batch_windows=batch_windows)   # [B, D, H, W]
-    D = feats.shape[1]
-    flat = feats.permute(0, 2, 3, 1).reshape(B * H * W, D)   # the one copy: pixels as rows
-    probs, pred = knn_classify(flat[valid], labels[valid], flat, num_classes=num_classes, k=k, temperature=temperature,
-                               batch_queries=batch_queries)
-    return probs.reshape(B, H, W, num_classes).permute(0, 3, 1, 2).contiguous(), pred.reshape(B, H, W)
+    flat = _pixel_rows(feats)
+    val = (flat[vvalid], vlabels[vvalid]) if val_labels is not None else None
+    probe = linear_probe_fit(flat[valid], labels[valid], num_classes=num_classes, heads=heads, epochs=epochs, batch_size=batch_size,
+                             seed=seed, val=val)
+    probs, pred = probe.predict(flat, batch_queries=batch_queries)
+    return _pixel_map(probs, feats), pred.reshape(feats.shape[0], *feats.shape[2:]), probe
