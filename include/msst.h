@@ -355,6 +355,58 @@ MSST_API int msst_linprobe_predict(int64_t n_query, int dim, int nc, const float
                                    msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * k-means clustering of embeddings (Lloyd's algorithm with k-means++ seeding), R restarts run together in the same launches.
+ *   rows:        x [n, dim] fp32.  normalize = 1 uses every row as F.normalize(x, dim=1, eps=1e-12), y = x / max(||x||, 1e-12) in fp32
+ *                (one device function, so every kernel sees the same bits); the normalised row is never stored.  normalize = 0 uses x.
+ *   centroids    [R, K, dim] fp32; restart r owns centroids[r].
+ *   distance     d(y, c) = sum_d (y_d - c_d)^2 in fp32, the direct difference form (not |y|^2 - 2 y.c + |c|^2, which cancels
+ *                catastrophically for rows far from the origin).
+ *   slices       rows [4096 s, 4096 s + 4096): a fixed length, independent of the grid and the SM count.  S = ceil(n / 4096).
+ *   msst_kmeans_workspace  bytes of the workspace of msst_kmeans_seed / _assign / _update: 8*R*S + 4*R*S*K*dim + 4*R*S*K + 4*R*S;
+ *                -1 (and the error message) on bad dims.
+ *   msst_kmeans_assign     labels [R, n] int64 = argmin_k d(y_i, c_rk), the LOWEST k on ties; dist [R, n] fp32 = that minimum (dist may
+ *                be NULL).  With a workspace it also writes, per (slice, restart): the per-cluster sums of the assigned rows (fp64 in
+ *                ascending row order, stored rounded to fp32), the per-cluster counts, the slice's inertia (fp64 sum of the minima in
+ *                ascending row order) and the number of rows whose label differs from the one in `labels` on entry (-1 before the
+ *                first pass).  workspace = NULL is prediction: labels and distances only, `labels` is not read.
+ *   msst_kmeans_update     thread = (restart, cluster, feature): c = (fp32)(sum_s sums_s / sum_s counts_s), the slices added in
+ *                ascending order in fp64.  An EMPTY cluster keeps its previous centroid bit for bit (no relocation).  Per restart:
+ *                inertia [R] fp64 = sum of the slices' inertias (ascending slice order) of the assignment that produced the sums,
+ *                changed [R] int32 = rows whose label changed, empty [R] int32 = clusters with no row.  centroids are updated in place.
+ *   msst_kmeans_seed       round j of k-means++ for every restart, u [R, K] fp64 uniforms in [0, 1) from the host:
+ *                j = 0:  row i = min(floor(u[r][0] * n), n - 1)
+ *                j > 0:  mindist [R, n] fp32 holds the distance of each row to the nearest of centroids 0 .. j-1 of its restart and
+ *                        the workspace the fp64 per-slice sums of it (ascending row order); P_s = sum of the sums of slices < s and
+ *                        T = P_S (ascending slice order), t = u[r][j] * T.  The round takes the first row i, in ascending order, with
+ *                        P_s + L_i > t (strictly), L_i = the fp64 running sum of mindist over rows 4096 s .. i of its slice s.  When
+ *                        T == 0 (fewer distinct rows than K) it falls back to the j = 0 rule with u[r][j].
+ *                The chosen row (normalised when normalize = 1) becomes centroid j, index [R, K] int64 records it.  Unless j = K-1,
+ *                a second launch then folds d(y_i, c_j) into mindist (j = 0: sets it) and refreshes the slice sums.  Rounds must
+ *                run in order 0 .. K-1 on the same mindist / workspace.
+ * Deterministic: no float atomics; a (slice, restart) pair is one CTA, every sum runs in a fixed order.  A restart's results depend
+ * only on x, its own u row (or its given centroids) and the dims, so fits are bitwise reproducible, a restart run among others equals
+ * the same restart run alone, and labels / dist of prediction are bitwise independent of how the rows are chunked.
+ * Limits (MSST_ERR_ARG before any launch, outputs untouched): dim a multiple of 32 in [32, 256]; 1 <= K <= 256 and
+ * K * dim <= MSST_KMEANS_MAX_KD (the per-cluster fp64 sums and the centroids live in shared memory: K = 128 at dim = 96, K = 64
+ * at dim = 256); 1 <= R <= 16; n < 2^31 with K <= n for seeding and for assignment with a workspace, n >= 1 for prediction;
+ * 0 <= round < K; no NULL pointer where one is required.
+ * ------------------------------------------------------------------------------------------- */
+#define MSST_KMEANS_MAX_RESTARTS 16
+#define MSST_KMEANS_MAX_KD 16384
+typedef struct {
+    int64_t n;                   /* rows of x */
+    int dim, k, restarts;        /* feature width, clusters, restarts R */
+    int normalize;               /* 1: rows are F.normalize'd when staged */
+} msst_kmeans_dims;
+MSST_API int64_t msst_kmeans_workspace(const msst_kmeans_dims* d);
+MSST_API int msst_kmeans_seed(const msst_kmeans_dims* d, int round, const float* x, const double* u, float* centroids, int64_t* index,
+                              float* mindist, void* workspace, msst_stream_t stream);
+MSST_API int msst_kmeans_assign(const msst_kmeans_dims* d, const float* x, const float* centroids, int64_t* labels, float* dist,
+                                void* workspace, msst_stream_t stream);
+MSST_API int msst_kmeans_update(const msst_kmeans_dims* d, const void* workspace, float* centroids, double* inertia, int32_t* changed,
+                                int32_t* empty, msst_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * SimMIM decoder + masked L1 loss (vit_simmim_original.py:314-338, BlockwiseToPixels :9-40):
  *   pred[b,n,:] = W[blk] enc[b, idx[b,n], :] + bias[blk],  blk = idx / S (0 when n_weight_blocks == 1)
  *   target      = raw pixels of patch idx gathered from img (or target_tokens [B,T,P] if not NULL)

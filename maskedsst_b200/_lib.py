@@ -69,6 +69,10 @@ class LinprobeDims(C.Structure):   # msst_linprobe_dims
                 ("lr", C.c_float * 16), ("wd", C.c_float * 16)]
 
 
+class KmeansDims(C.Structure):   # msst_kmeans_dims
+    _fields_ = [("n", C.c_int64), ("dim", C.c_int), ("k", C.c_int), ("restarts", C.c_int), ("normalize", C.c_int)]
+
+
 class DecodeDims(C.Structure):
     _fields_ = [("B", C.c_int), ("C", C.c_int), ("G", C.c_int), ("p0", C.c_int), ("p1", C.c_int), ("D", C.c_int),
                 ("nm", C.c_int), ("n_weight_blocks", C.c_int), ("raw", C.POINTER(RawInput))]
@@ -120,6 +124,10 @@ SIGNATURES = {
     "msst_linprobe_grad": (C.c_int, [C.POINTER(LinprobeDims), vp, vp, vp, vp, vp, vp]),
     "msst_linprobe_update": (C.c_int, [C.POINTER(LinprobeDims), vp, vp, vp, vp, vp, vp]),
     "msst_linprobe_predict": (C.c_int, [C.c_int64, C.c_int, C.c_int, vp, vp, vp, vp, vp]),
+    "msst_kmeans_workspace": (C.c_int64, [C.POINTER(KmeansDims)]),
+    "msst_kmeans_seed": (C.c_int, [C.POINTER(KmeansDims), C.c_int, vp, vp, vp, vp, vp, vp, vp]),
+    "msst_kmeans_assign": (C.c_int, [C.POINTER(KmeansDims), vp, vp, vp, vp, vp, vp]),
+    "msst_kmeans_update": (C.c_int, [C.POINTER(KmeansDims), vp, vp, vp, vp, vp, vp]),
     "msst_simmim_decode_l1_fwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 9 + [vp]),
     "msst_simmim_decode_l1_bwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 11 + [vp]),
     "msst_draw_masks": (C.c_int, [C.POINTER(MaskGenDims), vp, vp, vp]),

@@ -20,10 +20,16 @@ features, trained with AdamW for several (lr, weight_decay) heads at once (csrc/
 writes fixed 128-row slice partials for every head, and one launch that sums them in order and applies AdamW to every head).  Fits are
 bitwise reproducible and each head is bitwise the head fitted alone.  `LinearProbe.load_into` writes a probe into the default head of
 a ViTSpatialSpectral, whose LayerNorm and per-patch Linear then compute exactly the probe's function of the embed_scene features.
+
+`kmeans_fit` / `KMeans` / `cluster_scene` cluster the features without labels (csrc/kmeans.cu: Lloyd's algorithm, per iteration one
+assignment launch that writes fixed 4096-row slice partials for every restart and one launch that sums them in order; k-means++ seeding
+in at most two launches per centroid).  `clustering_metrics` scores a clustering against ground truth: NMI, ARI and the accuracy of the
+best one-to-one (Hungarian) and of the majority cluster -> class maps.
 """
 import ctypes
 import math
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -605,3 +611,288 @@ def linear_probe_scene(model, scene, train_labels, *, num_classes, val_labels=No
                              seed=seed, val=val)
     probs, pred = probe.predict(flat, batch_queries=batch_queries)
     return _pixel_map(probs, feats), pred.reshape(feats.shape[0], *feats.shape[2:]), probe
+
+
+KMEANS_MAX_K, KMEANS_MAX_RESTARTS, KMEANS_MAX_KD = 256, 16, 16384
+
+
+def _kmeans_args(who, num_clusters, dim, n, restarts, iters, seed, normalize):
+    """The checks of kmeans_fit that need no tensor: the feature width dim, K, R, iterations, seed, normalize and the row count n."""
+    if isinstance(num_clusters, bool) or not isinstance(num_clusters, int) or not 1 <= num_clusters <= KMEANS_MAX_K:
+        raise ValueError(f"{who}: num_clusters={num_clusters!r} must be an int in [1, {KMEANS_MAX_K}]")
+    if dim % 32 or not 32 <= dim <= KNN_MAX_DIM:
+        raise ValueError(f"{who}: feature width {dim} must be a multiple of 32 in [32, {KNN_MAX_DIM}]")
+    if num_clusters * dim > KMEANS_MAX_KD:
+        raise ValueError(f"{who}: num_clusters * dim = {num_clusters} * {dim} exceeds {KMEANS_MAX_KD} (the per-cluster sums live in "
+                         f"shared memory)")
+    if isinstance(restarts, bool) or not isinstance(restarts, int) or not 1 <= restarts <= KMEANS_MAX_RESTARTS:
+        raise ValueError(f"{who}: restarts={restarts!r} must be an int in [1, {KMEANS_MAX_RESTARTS}]")
+    _int_arg(who, "iters", iters, 1)
+    _int_arg(who, "seed", seed, 0)
+    if not isinstance(normalize, bool):
+        raise ValueError(f"{who}: normalize={normalize!r} must be a bool")
+    if not num_clusters <= n < 2 ** 31:
+        raise ValueError(f"{who}: {n} rows; need num_clusters={num_clusters} <= rows < 2^31")
+
+
+def _kmeans_dims(n, dim, k, restarts, normalize):
+    return _lib.KmeansDims(n, dim, k, restarts, 1 if normalize else 0)
+
+
+def _stream(t):
+    return torch.cuda.current_stream(t.device).cuda_stream
+
+
+def _kmeans_seed(dims, rnd, x, u, centroids, index, mindist, workspace):
+    """One msst_kmeans_seed round (k-means++ choice `rnd` of every restart, then the mindist refresh unless it is the last)."""
+    _lib.check(_lib.lib().msst_kmeans_seed(ctypes.byref(dims), rnd, x.data_ptr(), u.data_ptr(), centroids.data_ptr(), index.data_ptr(),
+                                           mindist.data_ptr(), workspace.data_ptr(), _stream(x)))
+
+
+def _kmeans_assign(dims, x, centroids, labels, dist=None, workspace=None):
+    """One msst_kmeans_assign launch: labels [R, n] (and dist [R, n]); with a workspace also the slice partials of the update."""
+    _lib.check(_lib.lib().msst_kmeans_assign(ctypes.byref(dims), x.data_ptr(), centroids.data_ptr(), labels.data_ptr(),
+                                             dist.data_ptr() if dist is not None else None,
+                                             workspace.data_ptr() if workspace is not None else None, _stream(x)))
+
+
+def _kmeans_update(dims, workspace, centroids, inertia, changed, empty):
+    """One msst_kmeans_update launch: new centroids in place, inertia [R] fp64, changed [R] / empty [R] int32."""
+    _lib.check(_lib.lib().msst_kmeans_update(ctypes.byref(dims), workspace.data_ptr(), centroids.data_ptr(), inertia.data_ptr(),
+                                             changed.data_ptr(), empty.data_ptr(), _stream(centroids)))
+
+
+def _kmeans_uniforms(seed, restarts, k, device):
+    """u [R, K] float64: restart r draws torch.rand(K) from torch.Generator(device).manual_seed(seed + r)."""
+    return torch.stack([torch.rand(k, generator=torch.Generator(device=device).manual_seed(seed + r), device=device, dtype=torch.float64)
+                        for r in range(restarts)])
+
+
+class KMeans:
+    """A k-means fit of R restarts.
+
+    centroids [R, K, dim] fp32 (CUDA), in the space the rows were clustered in (normalised rows when normalize);
+    inertia [R] float64: sum over the rows of the squared distance to their centroid, for the last assignment of the restart (the
+    one that produced its centroids; for a converged restart that is its final centroids' own inertia);
+    iterations [R] int64: assign + update passes run until the restart's labels stopped changing (iters when they never did);
+    converged [R] bool; best: the restart of lowest inertia, lowest index on ties; seed_index [R, K] int64: the rows k-means++ chose
+    (None for a fit from init)."""
+
+    def __init__(self, centroids, inertia, iterations, converged, normalize, seed_index=None):
+        self.centroids, self.inertia, self.iterations, self.converged = centroids, inertia, iterations, converged
+        self.normalize, self.seed_index = normalize, seed_index
+        self.best = int(torch.argmin(inertia))   # the first of equal minima
+
+    @property
+    def num_clusters(self):
+        return self.centroids.shape[1]
+
+    @torch.no_grad()
+    def predict(self, x, *, restart=None, batch_queries=262144):
+        """x [Q, dim] fp32 CUDA -> (labels [Q] int64 = the nearest centroid of restart `restart` (default: best), lowest index on ties;
+        dist [Q] fp32 = the squared distance to it), rows normalised as in the fit.  Queries run in chunks of batch_queries; the result is
+        bitwise the same for any chunk size."""
+        who = "KMeans.predict"
+        restart = self.best if restart is None else restart
+        R, K, D = self.centroids.shape
+        if isinstance(restart, bool) or not isinstance(restart, int) or not 0 <= restart < R:
+            raise ValueError(f"{who}: restart={restart!r} must be an int in [0, {R})")
+        x = _knn_features(who, "x", x)
+        if x.shape[1] != D or x.device != self.centroids.device:
+            raise ValueError(f"{who}: x {tuple(x.shape)} on {x.device} does not match dim {D} on {self.centroids.device}")
+        if isinstance(batch_queries, bool) or not isinstance(batch_queries, int) or batch_queries < 1:
+            raise ValueError(f"{who}: batch_queries={batch_queries!r} must be a positive int")
+        Q = x.shape[0]
+        if not Q < 2 ** 31:
+            raise ValueError(f"{who}: {Q} rows; need rows < 2^31")
+        labels = torch.empty(Q, device=x.device, dtype=torch.int64)
+        dist = torch.empty(Q, device=x.device, dtype=torch.float32)
+        c = self.centroids[restart].contiguous()
+        for first in range(0, Q, batch_queries):
+            last = min(first + batch_queries, Q)
+            dims = _kmeans_dims(last - first, D, K, 1, self.normalize)
+            _kmeans_assign(dims, x[first:last], c, labels[first:last], dist[first:last])
+        return labels, dist
+
+
+@torch.no_grad()
+def kmeans_fit(x, num_clusters, *, restarts=1, iters=100, seed=0, normalize=True, init=None):
+    """k-means (Lloyd's algorithm) on the device: the unsupervised probe of an encoder and the usual clustering of a scene.
+
+    x [n, dim] fp32 CUDA, dim a multiple of 32 in [32, 256], num_clusters <= n < 2^31; 1 <= num_clusters <= 256 with
+    num_clusters * dim <= 16384; 1 <= restarts <= 16.  normalize: cluster F.normalize(x, dim=1) (cosine geometry, the usual choice for
+    self-supervised features); the rows are normalised on the fly and never stored.  Distances are squared Euclidean in fp32 in the
+    direct difference form, a centroid is the mean of its rows (fp64 sums, not renormalised), an empty cluster keeps its centroid.
+    Seeding: k-means++, restart r drawing its K uniforms from torch.Generator(x.device).manual_seed(seed + r), so restart r of a fit
+    equals a one-restart fit with seed + r.  init: optional [restarts, num_clusters, dim] fp32 CUDA starting centroids (no seeding).
+    Each iteration is one assignment and one update launch for all restarts; the fit stops when no restart changed a label, or after
+    iters.  Bitwise reproducible; a restart does not depend on the others.
+    -> KMeans."""
+    who = "kmeans_fit"
+    x = _knn_features(who, "x", x)
+    n, D = x.shape
+    _kmeans_args(who, num_clusters, D, n, restarts, iters, seed, normalize)
+    R, K, dev = restarts, num_clusters, x.device
+    if init is not None:
+        if (not isinstance(init, torch.Tensor) or init.shape != (R, K, D) or init.dtype != torch.float32 or not init.is_cuda
+                or init.device != dev):
+            raise ValueError(f"{who}: init must be an fp32 tensor [{R}, {K}, {D}] on {dev}, got "
+                             f"{tuple(init.shape) if isinstance(init, torch.Tensor) else type(init).__name__}"
+                             f"{f' {init.dtype} on {init.device}' if isinstance(init, torch.Tensor) else ''}")
+    dims = _kmeans_dims(n, D, K, R, normalize)
+    workspace = torch.empty(_lib.lib().msst_kmeans_workspace(ctypes.byref(dims)), device=dev, dtype=torch.uint8)
+    seed_index = None
+    if init is not None:
+        centroids = init.clone().contiguous()
+    else:
+        centroids = torch.empty(R, K, D, device=dev, dtype=torch.float32)
+        seed_index = torch.empty(R, K, device=dev, dtype=torch.int64)
+        u = _kmeans_uniforms(seed, R, K, dev)
+        mindist = torch.empty(R, n, device=dev, dtype=torch.float32)
+        for j in range(K):
+            _kmeans_seed(dims, j, x, u, centroids, seed_index, mindist, workspace)
+        del mindist
+    labels = torch.full((R, n), -1, device=dev, dtype=torch.int64)
+    inertia = torch.empty(R, device=dev, dtype=torch.float64)
+    changed = torch.empty(R, device=dev, dtype=torch.int32)
+    empty = torch.empty(R, device=dev, dtype=torch.int32)
+    iterations = torch.full((R,), iters, dtype=torch.int64)
+    converged = torch.zeros(R, dtype=torch.bool)
+    for it in range(1, iters + 1):
+        _kmeans_assign(dims, x, centroids, labels, workspace=workspace)
+        _kmeans_update(dims, workspace, centroids, inertia, changed, empty)
+        done = changed.cpu() == 0                      # the one read-back per iteration
+        iterations[done & ~converged] = it
+        converged |= done
+        if bool(converged.all()):
+            break
+    return KMeans(centroids, inertia.cpu(), iterations, converged, normalize,
+                  seed_index=seed_index.cpu() if seed_index is not None else None)
+
+
+@torch.no_grad()
+def cluster_scene(model, scene, *, num_clusters, restarts=1, iters=100, seed=0, normalize=True, stride=None, weight=None,
+                  batch_windows=4096, batch_queries=262144):
+    """k-means of an encoder's features on whole scenes: embed_scene, every pixel a row, kmeans_fit on all pixels, every pixel assigned
+    to the nearest centroid of the best restart (the unsupervised segmentation of the scene).
+
+    model, scene, stride, weight, batch_windows: as in embed_scene (a SimMIMSpatialSpectral checkpoint works directly).
+    num_clusters, restarts, iters, seed, normalize: as in kmeans_fit; batch_queries: as in KMeans.predict.
+    Score the result against ground truth with clustering_metrics.
+    -> (clusters [B, H, W] int64, the KMeans)."""
+    who = "cluster_scene"
+    tiles = scene.tiles if isinstance(scene, RawTiles) else scene
+    if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
+        raise ValueError(f"{who}: scene must be a [B, C, H, W] tensor or RawTiles")
+    if not tiles.is_cuda:
+        raise ValueError(f"{who}: the scene must be on a CUDA device")
+    enc = model.encoder if isinstance(model, SimMIMSpatialSpectral) else model
+    if not isinstance(enc, ViTSpatialSpectral):
+        raise ValueError(f"{who}: needs a ViTSpatialSpectral encoder, got {type(enc).__name__}")
+    B, _, H, W = tiles.shape
+    _kmeans_args(who, num_clusters, enc.dim, B * H * W, restarts, iters, seed, normalize)
+    if isinstance(batch_queries, bool) or not isinstance(batch_queries, int) or batch_queries < 1:
+        raise ValueError(f"{who}: batch_queries={batch_queries!r} must be a positive int")
+    feats = embed_scene(model, scene, stride=stride, weight=weight, batch_windows=batch_windows)   # [B, D, H, W]
+    flat = _pixel_rows(feats)
+    km = kmeans_fit(flat, num_clusters, restarts=restarts, iters=iters, seed=seed, normalize=normalize)
+    clusters, _ = km.predict(flat, batch_queries=batch_queries)
+    return clusters.reshape(B, H, W), km
+
+
+def _min_cost_assignment(cost):
+    """Rows of cost [n, m] (int64, n <= m) to distinct columns at the least total cost (the Hungarian method with potentials,
+    O(n^2 m), one vectorised pass over the columns per step) -> col [n] int64."""
+    n, m = cost.shape
+    big = np.iinfo(np.int64).max // 4
+    u, v = np.zeros(n + 1, np.int64), np.zeros(m + 1, np.int64)
+    p, way = np.zeros(m + 1, np.int64), np.zeros(m + 1, np.int64)   # p[j]: 1-based row on column j (0: none); column 0 is the root
+    for i in range(1, n + 1):
+        p[0], j0 = i, 0
+        minv = np.full(m + 1, big, np.int64)
+        used = np.zeros(m + 1, bool)
+        while True:
+            used[j0] = True
+            i0 = p[j0]
+            free = ~used[1:]
+            cur = cost[i0 - 1] - u[i0] - v[1:]
+            better = free & (cur < minv[1:])
+            minv[1:][better] = cur[better]
+            way[1:][better] = j0
+            cand = np.where(free, minv[1:], big)
+            j1 = int(np.argmin(cand)) + 1
+            delta = cand[j1 - 1]
+            u[p[used]] += delta
+            v[used] -= delta
+            minv[~used] -= delta
+            j0 = j1
+            if p[j0] == 0:
+                break
+        while j0:
+            j1 = way[j0]
+            p[j0] = p[j1]
+            j0 = j1
+    col = np.full(n, -1, np.int64)
+    rows = p[1:] > 0
+    col[p[1:][rows] - 1] = np.nonzero(rows)[0]
+    return col
+
+
+def clustering_metrics(clusters, labels, *, num_clusters, num_classes, ignore_index=-1):
+    """Scores a clustering against ground-truth classes on the host, in float64.  A pixel counts when its label is != ignore_index and in
+    [0, num_classes) (the rule of confusion_matrix); its cluster must then lie in [0, num_clusters).  num_clusters, num_classes <= 256.
+      contingency [nc, K] int64        pixels of class c in cluster k
+      nmi            mutual information / ((H(classes) + H(clusters)) / 2), natural log; 1.0 when both sides have one occupied label
+      ari            adjusted Rand index (Hubert and Arabie); 1.0 in the degenerate cases (both sides one label, or all singletons)
+      hungarian_map [K] int64, oa_hungarian   the one-to-one cluster -> class matching with the most matched pixels (-1 for the
+                     clusters left unmatched when K > nc) and the share of pixels it gets right
+      majority_map [K] int64, oa_majority     each cluster to its most frequent class (lowest class on ties; class 0 for an empty
+                     cluster) and the share of pixels that gets right
+    With a map, map[clusters] is a class prediction for confusion_matrix / classification_metrics (AA, kappa); pixels of a cluster
+    that hungarian_map leaves at -1 are outside the classes there, so score K > nc with majority_map.
+    -> dict of the above (maps and contingency as CPU tensors, the scores as floats)."""
+    who = "clustering_metrics"
+    for name, v in (("num_clusters", num_clusters), ("num_classes", num_classes)):
+        if isinstance(v, bool) or not isinstance(v, int) or not 1 <= v <= KMEANS_MAX_K:
+            raise ValueError(f"{who}: {name}={v!r} must be an int in [1, {KMEANS_MAX_K}]")
+    K, nc = num_clusters, num_classes
+    cl, lab = torch.as_tensor(clusters), torch.as_tensor(labels)
+    for name, t in (("clusters", cl), ("labels", lab)):
+        if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+            raise ValueError(f"{who}: {name} must be an integer tensor, got {t.dtype}")
+    if cl.numel() != lab.numel():
+        raise ValueError(f"{who}: {cl.numel()} clusters for {lab.numel()} labels")
+    cl = cl.reshape(-1).to("cpu", torch.int64).numpy()
+    lab = lab.reshape(-1).to("cpu", torch.int64).numpy()
+    valid = (lab != ignore_index) & (lab >= 0) & (lab < nc)
+    cl, lab = cl[valid], lab[valid]
+    if cl.size == 0:
+        raise ValueError(f"{who}: no labelled pixel")
+    if bool(((cl < 0) | (cl >= K)).any()):
+        raise ValueError(f"{who}: clusters outside [0, {K})")
+    cont = np.bincount(lab * K + cl, minlength=nc * K).reshape(nc, K)
+    N = float(cl.size)
+    a, b = cont.sum(1).astype(np.float64), cont.sum(0).astype(np.float64)
+    if np.count_nonzero(a) == 1 and np.count_nonzero(b) == 1:
+        nmi = 1.0
+    else:
+        nz = cont > 0
+        nij = cont[nz].astype(np.float64)
+        outer = np.outer(a, b)[nz]
+        mi = float(np.sum(nij / N * (np.log(nij) + math.log(N) - np.log(outer))))
+        ent = lambda s: float(-np.sum(s[s > 0] / N * np.log(s[s > 0] / N)))
+        nmi = mi / ((ent(a) + ent(b)) / 2)
+    comb = lambda v: v * (v - 1) / 2
+    index, sa, sb, pairs = float(comb(cont.astype(np.float64)).sum()), float(comb(a).sum()), float(comb(b).sum()), comb(N)
+    expected = sa * sb / pairs if pairs > 0 else 0.0
+    top = (sa + sb) / 2
+    ari = 1.0 if top == expected else (index - expected) / (top - expected)
+    hmap = np.full(K, -1, np.int64)
+    if K <= nc:
+        hmap[:] = _min_cost_assignment(-cont.T.astype(np.int64))
+    else:
+        hmap[_min_cost_assignment(-cont.astype(np.int64))] = np.arange(nc)
+    matched = int(sum(cont[hmap[k], k] for k in range(K) if hmap[k] >= 0))
+    mmap = cont.argmax(0).astype(np.int64)
+    return dict(contingency=torch.from_numpy(cont.astype(np.int64)), nmi=nmi, ari=ari, oa_hungarian=matched / N,
+                hungarian_map=torch.from_numpy(hmap), oa_majority=float(cont.max(0).sum()) / N, majority_map=torch.from_numpy(mmap))
