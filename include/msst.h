@@ -288,6 +288,32 @@ typedef struct {
 } msst_scene_embed_dims;
 MSST_API int msst_scene_embed(const msst_scene_embed_dims* d, const float* tokens, const float* weight, float* acc, float* wsum,
                               msst_stream_t stream);
+/* Whole-scene masked reconstruction (SimMIM decoding): the same windows, chunks, weight and ownership contract as msst_scene_blend,
+ * but each covering window contributes the decoder's prediction of the scene entries a scene mask hides.  One call blends the chunk
+ * [win_first, win_first + n):
+ *   tokens [n, C*S, D]         the chunk's encoder output with the masked tokens replaced by the mask token (fp32, t = c*S + s,
+ *                              S = G*G, G = win / p1), read in place
+ *   mask   [B, C, H, W] uint8  scene mask: nonzero = the p0 bands of spectral block c at pixel (y, x) are hidden
+ *   W [n_wb, P, D], bias [n_wb, P]   the decoder: to_pixels (n_wb = 1) or BlockwiseToPixels (n_wb = C, block c uses row block c);
+ *                              P = p0 * p1 * p1, output p = j * p1^2 + i1 * p1 + i2 is band c*p0 + j at (i1, i2) inside the patch
+ *   weight [win, win] or NULL  per-window-pixel weight (NULL: 1)
+ *   for every masked entry (b, band = c*p0 + j, y, x), over the chunk's windows covering (y, x) (origin (oy, ox), py = y - oy, px = x - ox):
+ *     acc [B, C*p0, H, W] +=  weight(py, px) * (W[blk] . tokens[g - win_first, c*S + s, :] + bias[blk])[p],
+ *                             s = (py / p1) * G + px / p1,  p = j * p1^2 + (py % p1) * p1 + px % p1,  blk = n_wb == 1 ? 0 : c
+ *   wsum [B, H, W]      +=  weight(py, px)   once per covering window (entries of visible blocks are left as they are)
+ * Bitwise independent of the chunking (chunks in ascending order); only the scene rows the chunk touches are visited.
+ * 1 <= stride <= win <= H, W;  win_y <= ceil((H - win) / stride_y) + 1 (ditto x);  D a multiple of 32 in [32, 256];  P <= 16;
+ * n_wb in {1, C};  win % p1 == 0;  C * p0 <= 1760 (shared memory).  MSST_ERR_ARG before any launch otherwise, outputs untouched.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    int B, D, H, W;              /* scenes, feature width, scene rows / columns */
+    int win, stride_y, stride_x; /* square window side, window step */
+    int win_y, win_x;            /* windows per scene column / row */
+    int win_first, n;            /* this chunk: global windows [win_first, win_first + n) */
+    int C, p0, p1, n_wb;         /* spectral blocks, spectral / spatial patch side, decoder weight blocks (1 or C) */
+} msst_scene_reconstruct_dims;
+MSST_API int msst_scene_reconstruct(const msst_scene_reconstruct_dims* d, const float* tokens, const uint8_t* mask, const float* W,
+                                    const float* bias, const float* weight, float* acc, float* wsum, msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * k-nearest-neighbour probing of embeddings (e.g. msst_scene_embed maps): cosine similarity, k best references per query, class vote.

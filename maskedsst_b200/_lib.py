@@ -60,6 +60,11 @@ class SceneEmbedDims(C.Structure):   # msst_scene_embed_dims
     _fields_ = [(n, C.c_int) for n in ("B", "D", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n", "C", "p1")]
 
 
+class SceneReconstructDims(C.Structure):   # msst_scene_reconstruct_dims
+    _fields_ = [(n, C.c_int) for n in ("B", "D", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n", "C", "p0",
+                                       "p1", "n_wb")]
+
+
 class KnnDims(C.Structure):   # msst_knn_dims
     _fields_ = [("n_ref", C.c_int64), ("n_query", C.c_int64), ("dim", C.c_int), ("k", C.c_int)]
 
@@ -117,6 +122,7 @@ SIGNATURES = {
     "msst_cross_entropy_fwd_bwd": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
     "msst_scene_blend": (C.c_int, [C.POINTER(SceneDims), vp, vp, vp, vp, vp]),
     "msst_scene_embed": (C.c_int, [C.POINTER(SceneEmbedDims), vp, vp, vp, vp, vp]),
+    "msst_scene_reconstruct": (C.c_int, [C.POINTER(SceneReconstructDims)] + [vp] * 7 + [vp]),
     "msst_knn_prepare": (C.c_int, [vp, C.c_int64, C.c_int, vp, vp]),
     "msst_knn_topk": (C.c_int, [C.POINTER(KnnDims), vp, vp, vp, vp, vp]),
     "msst_knn_vote": (C.c_int, [C.c_int64, C.c_int, C.c_int64, vp, vp, vp, C.c_int, C.c_float, vp, vp, vp]),

@@ -5,7 +5,7 @@
 // One thread owns one scene pixel and adds its covering windows in ascending global window index, one at a time (acc = acc + c): no
 // atomics, so the sums are bitwise independent of how the windows were cut into chunks.  Which windows cover the pixel follows from
 // the origin rule of the pixel reader (window_origin, pixel_source.cuh); the windows are never enumerated.  msst_scene_embed blends
-// per-pixel encoder features the same way (below).
+// per-pixel encoder features and msst_scene_reconstruct the SimMIM decoder's predictions of masked values the same way (below).
 #include "common.cuh"
 #include "pixel_source.cuh"
 
@@ -147,6 +147,80 @@ __global__ void __launch_bounds__(kEmbedThreads) scene_embed_kernel(SceneGeom g,
     }
 }
 
+// Masked reconstruction (msst_scene_reconstruct): the same ownership and window order again, but each covering window contributes, for
+// every spectral block c that the scene mask hides at the pixel, the SimMIM decoder output of its token (c, s) at the pixel's place in
+// the patch: v[j] = W[blk, p] . token + bias[blk, p],  p = j * p1^2 + (py % p1) * p1 + px % p1  (band c * p0 + j; target_pixel's
+// layout in simmim.cu).  A block owns kEmbedPix consecutive scene pixels with their running band sums in shared memory,
+// [C * p0][kEmbedPix + 1], loaded and stored with lanes over pixels; one warp per pixel decodes with lanes over features (each token row
+// is read as whole lines, each decoder row from L1) and the warp's butterfly sum leaves every dot product in every lane.  Entries whose
+// block is visible are loaded and stored back unchanged.
+template <int NJ>
+__global__ void __launch_bounds__(kEmbedThreads) scene_reconstruct_kernel(SceneGeom g, int C, int p0, int p1, int n_wb,
+                                                                          const float* __restrict__ tokens,
+                                                                          const uint8_t* __restrict__ mask,
+                                                                          const float* __restrict__ Wd, const float* __restrict__ bd,
+                                                                          const float* __restrict__ weight, float* __restrict__ acc,
+                                                                          float* __restrict__ wsum) {
+    constexpr int LD = kEmbedPix + 1;
+    extern __shared__ float sacc[];
+    const int nb = g.nc;                 // C * p0 bands
+    float* sws = sacc + nb * LD;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    constexpr int kWarps = kEmbedThreads / 32;
+    constexpr int D = NJ * 32;
+    const int64_t HW = (int64_t)g.H * g.W;
+    const int64_t q0 = (int64_t)blockIdx.x * kEmbedPix;
+    const bool mine = q0 + lane < g.npix;
+    const int64_t pl = g.pix0 + q0 + lane;
+    float* ap = acc + (pl / HW) * nb * HW + pl % HW;
+    if (mine) {
+        for (int c = warp; c < nb; c += kWarps) sacc[c * LD + lane] = ap[c * HW];
+        if (warp == 0) sws[lane] = wsum[pl];
+    }
+    __syncthreads();
+    const int G = g.win / p1, S = G * G, pp = p1 * p1, P = p0 * pp;
+    for (int k = warp; k < kEmbedPix && q0 + k < g.npix; k += kWarps) {
+        const int64_t p = g.pix0 + q0 + k;
+        const int b = (int)(p / HW);
+        const int64_t yx = p % HW;
+        const int y = (int)(yx / g.W), x = (int)(yx % g.W);
+        const uint8_t* mp = mask + (int64_t)b * C * HW + yx;
+        float ws = sws[k];
+        for_each_covering_window(g, b, y, x, [&](int64_t gw, int py, int px) {
+            const float wt = weight ? __ldg(weight + py * g.win + px) : 1.f;
+            const int s = (py / p1) * G + px / p1, sub = (py % p1) * p1 + px % p1;
+            const float* tw = tokens + (gw - g.g0) * C * S * D;
+            for (int c = 0; c < C; ++c) {
+                if (!__ldg(mp + c * HW)) continue;
+                const float* tp = tw + ((int64_t)c * S + s) * D;
+                float e[NJ];
+#pragma unroll
+                for (int j = 0; j < NJ; ++j) e[j] = __ldg(tp + lane + 32 * j);
+                const int blk = n_wb == 1 ? 0 : c;
+                for (int j0 = 0; j0 < p0; ++j0) {
+                    const int o = blk * P + j0 * pp + sub;
+                    const float* w = Wd + (int64_t)o * D;
+                    float a = 0.f;
+#pragma unroll
+                    for (int j = 0; j < NJ; ++j) a = fmaf(e[j], __ldg(w + lane + 32 * j), a);
+                    a = warp_sum(a);
+                    if (lane == (j0 & 31)) {
+                        float* r = sacc + (c * p0 + j0) * LD + k;
+                        *r = __fadd_rn(*r, __fmul_rn(wt, __fadd_rn(a, __ldg(bd + o))));
+                    }
+                }
+            }
+            ws = __fadd_rn(ws, wt);
+        });
+        if (lane == 0) sws[k] = ws;
+    }
+    __syncthreads();
+    if (mine) {
+        for (int c = warp; c < nb; c += kWarps) ap[c * HW] = sacc[c * LD + lane];
+        if (warp == 0) wsum[pl] = sws[lane];
+    }
+}
+
 static int64_t windows_along(int extent, int win, int step) { return (extent - win + step - 1) / step + 1; }
 
 // Checks the window geometry both entry points share (msst_scene_dims and msst_scene_embed_dims name it alike) and fills g: the
@@ -202,6 +276,38 @@ extern "C" int msst_scene_embed(const msst_scene_embed_dims* d, const float* tok
     const size_t smem = sizeof(float) * ((size_t)g.nc * (kEmbedPix + 1) + kEmbedPix);   // <= 33.9 KB at D = 256
     scene_embed_kernel<<<(unsigned)ceil_div(g.npix, kEmbedPix), kEmbedThreads, smem, (cudaStream_t)stream>>>(g, d->C, d->p1, tokens,
                                                                                                           weight, acc, wsum);
+    MSST_LAUNCH_CHECK();
+    return MSST_OK;
+}
+
+extern "C" int msst_scene_reconstruct(const msst_scene_reconstruct_dims* d, const float* tokens, const uint8_t* mask, const float* W,
+                                      const float* bias, const float* weight, float* acc, float* wsum, msst_stream_t stream) {
+    MSST_REQUIRE(d && d->B > 0 && d->D > 0 && d->win > 0 && d->C > 0 && d->p0 > 0 && d->p1 > 0 && d->n_wb > 0,
+                 "scene_reconstruct: bad dims");
+    MSST_REQUIRE(d->D % 32 == 0 && d->D <= kEmbedMaxDim, "scene_reconstruct: D=%d must be a multiple of 32 in [32, %d]", d->D,
+                 kEmbedMaxDim);
+    MSST_REQUIRE((int64_t)d->p0 * d->p1 * d->p1 <= 16, "scene_reconstruct: pixels per patch p0*p1^2 = %lld > 16 unsupported",
+                 (long long)d->p0 * d->p1 * d->p1);
+    MSST_REQUIRE(d->n_wb == 1 || d->n_wb == d->C, "scene_reconstruct: n_wb=%d must be 1 or C=%d", d->n_wb, d->C);
+    MSST_REQUIRE(d->win % d->p1 == 0, "scene_reconstruct: window %d is not a multiple of the spatial patch side p1=%d", d->win, d->p1);
+    const int64_t nb = (int64_t)d->C * d->p0;
+    const size_t smem = sizeof(float) * ((size_t)nb * (kEmbedPix + 1) + kEmbedPix);
+    MSST_REQUIRE(smem <= 227 * 1024, "scene_reconstruct: C*p0=%lld bands need %zu B of shared memory > 227 KB", (long long)nb, smem);
+    SceneGeom g;
+    const int rc = scene_geom("scene_reconstruct", d, (int)nb, g);
+    if (rc != MSST_OK) return rc;
+    MSST_REQUIRE(tokens && mask && W && bias && acc && wsum, "scene_reconstruct: tokens / mask / W / bias / acc / wsum must be set");
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned grid = (unsigned)ceil_div(g.npix, kEmbedPix);
+#define MSST_R(NJ)                                                                                                                  \
+    case NJ:                                                                                                                        \
+        if (smem > 48 * 1024) MSST_CUDA(cudaFuncSetAttribute(scene_reconstruct_kernel<NJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                                             (int)smem));                                                           \
+        scene_reconstruct_kernel<NJ><<<grid, kEmbedThreads, smem, st>>>(g, d->C, d->p0, d->p1, d->n_wb, tokens, mask, W, bias, weight, \
+                                                                        acc, wsum);                                                 \
+        break;
+    switch (d->D / 32) { MSST_R(1) MSST_R(2) MSST_R(3) MSST_R(4) MSST_R(5) MSST_R(6) MSST_R(7) MSST_R(8) }
+#undef MSST_R
     MSST_LAUNCH_CHECK();
     return MSST_OK;
 }

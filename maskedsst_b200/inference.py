@@ -25,6 +25,13 @@ a ViTSpatialSpectral, whose LayerNorm and per-patch Linear then compute exactly 
 assignment launch that writes fixed 4096-row slice partials for every restart and one launch that sums them in order; k-means++ seeding
 in at most two launches per centroid).  `clustering_metrics` scores a clustering against ground truth: NMI, ARI and the accuracy of the
 best one-to-one (Hungarian) and of the majority cluster -> class maps.
+
+`reconstruct_scene` runs the SimMIM objective itself on whole scenes: a scene mask [B, C, H, W] hides spectral blocks at pixels (a
+`scene_mask` drawn with the model's masking settings, or a map of dead stripes / saturated pixels), every window masks the tokens whose
+patch touches a hidden entry, and csrc/scene.cu decodes the masked tokens with the trained to_pixels and blends each hidden entry's
+predictions over the covering windows with the same ownership contract as the blends above.  The result is the inpainted scene in
+the model's units; `reconstruction_metrics` gives the held-out masked L1 / RMSE per band and overall, and |recon - scene| is a
+per-pixel reconstruction-error map.
 """
 import ctypes
 import math
@@ -219,6 +226,221 @@ def embed_windows(tokens, acc, wsum, *, C, p1, stride, grid, first, weight=None)
     dims = _lib.SceneEmbedDims(B, D, H, W, w, stride[0], stride[1], grid[0], grid[1], first, n, C, p1)
     _lib.check(_lib.lib().msst_scene_embed(ctypes.byref(dims), tokens.data_ptr(), weight.data_ptr() if weight is not None else None,
                                            acc.data_ptr(), wsum.data_ptr(), torch.cuda.current_stream(acc.device).cuda_stream))
+
+
+def _recon_encoder(who, model):
+    """The encoder of a SimMIM model whose decoder output maps back to scene pixels, else ValueError."""
+    if not isinstance(model, SimMIMSpatialSpectral):
+        raise ValueError(f"{who}: needs a SimMIMSpatialSpectral model (its decoder reconstructs the masked values), got "
+                         f"{type(model).__name__}")
+    enc = model.encoder
+    if model.v1 or not isinstance(enc, ViTSpatialSpectral):
+        raise ValueError(f"{who}: needs a ViTSpatialSpectral encoder, got {type(enc).__name__}")
+    if not enc.blockwise_patch_embed:
+        raise ValueError(f"{who}: needs the blockwise patch embedding (blockwise_patch_embed=True): with PatchEmbed the decoder predicts "
+                         f"LayerNorm'ed patches, which do not map back to pixel values")
+    return enc
+
+
+def _model_units(scene, pad):
+    """The scene as the model sees it, fp32 [B, bands, H, W]: the cube itself, or RawTiles standardised (pad: with the pad bands)."""
+    if isinstance(scene, RawTiles):
+        return scene.standardize(scene.tiles, pad=pad)
+    return scene if scene.dtype == torch.float32 else scene.float()
+
+
+def _patch_any(mask, p1):
+    """[B, C, H, W] bool -> [B, C, H - p1 + 1, W - p1 + 1]: whether any pixel of the p1 x p1 square with top-left corner (y, x) is set."""
+    if p1 == 1:
+        return mask
+    h, w = mask.shape[2] - p1 + 1, mask.shape[3] - p1 + 1
+    out = mask[:, :, :h, :w].clone()
+    for i in range(p1):
+        for j in range(p1):
+            out |= mask[:, :, i:i + h, j:j + w]
+    return out
+
+
+def _window_mask(pany, p1, window, stride, grid, first, n):
+    """Token mask [n, C*S] (t = c*S + s) of global windows [first, first + n), laid out as in blend_windows, from _patch_any(scene mask,
+    p1): token (c, s) of a window is masked when any pixel of its spatial patch s has block c set."""
+    B, C, h, w = pany.shape
+    H, W = h + p1 - 1, w + p1 - 1
+    (sy, sx), (ny, nx) = stride, grid
+    dev = pany.device
+    g = torch.arange(first, first + n, device=dev)
+    b, k = g // (ny * nx), g % (ny * nx)
+    oy = torch.clamp_max((k // nx) * sy, H - window)                    # the origin rule of window_origin (csrc/pixel_source.cuh)
+    ox = torch.clamp_max((k % nx) * sx, W - window)
+    r = torch.arange(window // p1, device=dev) * p1
+    c = torch.arange(C, device=dev)
+    m = pany[b[:, None, None, None], c[None, :, None, None], (oy[:, None] + r)[:, None, :, None], (ox[:, None] + r)[:, None, None, :]]
+    return m.reshape(n, -1)
+
+
+def _check_scene_mask(who, mask, B, C, H, W, device):
+    if (not isinstance(mask, torch.Tensor) or mask.dtype != torch.bool or tuple(mask.shape) != (B, C, H, W)
+            or mask.device != device):
+        got = (f"{mask.dtype} {tuple(mask.shape)} on {mask.device}" if isinstance(mask, torch.Tensor) else type(mask).__name__)
+        raise ValueError(f"{who}: mask must be a bool tensor [{B}, {C}, {H}, {W}] (one entry per spectral block) on {device}, got {got}")
+
+
+@torch.no_grad()
+def reconstruct_scene(model, scene, mask, *, stride=None, weight=None, batch_windows=4096):
+    """Masked reconstruction of whole scenes by a SimMIM checkpoint: inpainting of hidden values, held-out reconstruction error
+    (reconstruction_metrics) and per-pixel error maps.
+
+    model: SimMIMSpatialSpectral over a ViTSpatialSpectral with the blockwise patch embedding, either decoder (to_pixels or
+    BlockwiseToPixels), spectral_only too; fp32 or bf16 precision.
+    scene, stride, weight, batch_windows: as in predict_scene (weight weighs a window's predictions).
+    mask [B, C, H, W] bool on the scene's device, C = encoder.num_spectral_patches: entry (b, c, y, x) hides the p0 bands
+    c*p0 ... c*p0 + p0 - 1 at pixel (y, x) (scene_mask draws one; a map of dead stripes or saturated pixels works the same way).
+    In every window, token (c, s) is masked when any pixel of spatial patch s has block c hidden, so a hidden entry is masked in every
+    window that covers it and its own value never reaches the encoder.  The windows run in chunks through the patch embedding (with
+    the mask token) and the encoder in eval mode; msst_scene_reconstruct decodes the masked tokens and blends each hidden entry's
+    predictions over the covering windows on the device, deterministically and independently of batch_windows.
+    -> recon [B, C*p0, H, W] fp32 in the model's units: hidden entries hold the weighted mean prediction, visible entries the input
+    (the standardised cube, pad bands included for RawTiles)."""
+    who = "reconstruct_scene"
+    enc = _recon_encoder(who, model)
+    tiles = scene.tiles if isinstance(scene, RawTiles) else scene
+    if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
+        raise ValueError(f"{who}: scene must be a [B, C, H, W] tensor or RawTiles")
+    if not tiles.is_cuda:
+        raise ValueError(f"{who}: the scene must be on a CUDA device")
+    C, p0, p1 = enc.num_spectral_patches, enc.patch_depth, enc.patch_height
+    B, nb, H, W = tiles.shape
+    nb += scene.pad_bands if isinstance(scene, RawTiles) else 0
+    if nb != C * p0:
+        raise ValueError(f"{who}: the scene has {nb} bands, the model {C * p0}")
+    _check_scene_mask(who, mask, B, C, H, W, tiles.device)
+    w = enc.image_size
+    x, (sy, sx), (ny, nx), weight = _scene_input(who, scene, w, stride, weight)
+    if model.to_pixels_per_spectral_block:
+        Wd, bd = model.to_pixels.kernel_params()
+    else:
+        Wd, bd = model.to_pixels.weight[None], model.to_pixels.bias[None]
+    Wd, bd = Wd.detach().float().contiguous(), bd.detach().float().contiguous()
+    mask = mask.contiguous()
+    pany = _patch_any(mask, p1)
+    acc = torch.zeros(B, C * p0, H, W, device=tiles.device, dtype=torch.float32)
+    wsum = torch.zeros(B, H, W, device=tiles.device, dtype=torch.float32)
+    total, step = x.num_windows, max(1, int(batch_windows))
+    was_training = model.training
+    model.eval()
+    try:
+        pos = enc._pos_rows()
+        for first in range(0, total, step):
+            n = min(step, total - first)
+            wmask = _window_mask(pany, p1, w, (sy, sx), (ny, nx), first, n)
+            tokens = enc.to_patch_embedding._embed_img(x.set_window_range(first, n), pos=pos, mask_token=model.mask_token, mask=wmask)
+            tokens = enc.transformer_forward(tokens)                        # [n, C*S, D] fp32
+            reconstruct_windows(tokens, mask.view(torch.uint8), Wd, bd, acc, wsum, C=C, p0=p0, p1=p1, stride=(sy, sx), grid=(ny, nx),
+                                first=first, weight=weight)
+    finally:
+        model.train(was_training)
+    acc.div_(wsum[:, None])
+    return torch.where(mask.repeat_interleave(p0, 1), acc, _model_units(scene, pad=True))
+
+
+def reconstruct_windows(tokens, mask, W, bias, acc, wsum, *, C, p0, p1, stride, grid, first, weight=None):
+    """One chunk of msst_scene_reconstruct: for every entry (b, c*p0 + j, y, x) that the scene mask [B, C, H, W] (uint8 or bool) hides,
+    acc [B, C*p0, H, W] += weight * (W[blk] . token + bias[blk])[j*p1^2 + (py % p1)*p1 + px % p1] over the global windows
+    [first, first + n) that cover (y, x), token = tokens[window, c*S + (py // p1)*G + px // p1] ((py, px): the pixel in the window;
+    blk = c for a per-block decoder W [C, P, D], bias [C, P], else 0 for W [1, P, D], bias [1, P]; P = p0*p1^2), and wsum [B, H, W]
+    += weight once per covering window.  tokens [n, C*S, D] fp32 is the encoder output of the chunk's masked windows; windows laid out
+    as in blend_windows.  Chunks must be added in ascending order; the sums are then bitwise independent of the chunking."""
+    who = "reconstruct_windows"
+    for t, name in ((tokens, "tokens"), (W, "W"), (bias, "bias"), (acc, "acc"), (wsum, "wsum"), (weight, "weight")):
+        if (t is not None or name != "weight") and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32
+                                                         and t.is_contiguous()):
+            raise ValueError(f"{who}: {name} must be a contiguous fp32 CUDA tensor")
+    if not (isinstance(mask, torch.Tensor) and mask.is_cuda and mask.dtype in (torch.uint8, torch.bool) and mask.is_contiguous()):
+        raise ValueError(f"{who}: mask must be a contiguous uint8 or bool CUDA tensor")
+    if any(t is not None and t.device != acc.device for t in (tokens, mask, W, bias, wsum, weight)):
+        raise ValueError(f"{who}: all tensors must be on {acc.device}")
+    if tokens.dim() != 3 or acc.dim() != 4 or W.dim() != 3 or bias.dim() != 2 or min(C, p0, p1) < 1:
+        raise ValueError(f"{who}: tokens must be [n, C*S, D], acc [B, C*p0, H, W], W [n_wb, P, D] and bias [n_wb, P], got "
+                         f"{tuple(tokens.shape)}, {tuple(acc.shape)}, {tuple(W.shape)}, {tuple(bias.shape)}")
+    n, T, D = tokens.shape
+    B, nb, H, Wd = acc.shape
+    S = T // C
+    G = math.isqrt(S)
+    w, P = G * p1, p0 * p1 * p1
+    if (T != C * S or G * G != S or nb != C * p0 or tuple(mask.shape) != (B, C, H, Wd) or tuple(wsum.shape) != (B, H, Wd)
+            or W.shape[0] not in (1, C) or tuple(W.shape[1:]) != (P, D) or tuple(bias.shape) != (W.shape[0], P)
+            or (weight is not None and tuple(weight.shape) != (w, w))):
+        raise ValueError(f"{who}: shapes tokens {tuple(tokens.shape)} (C={C}, p0={p0}, p1={p1}), mask {tuple(mask.shape)}, "
+                         f"W {tuple(W.shape)}, bias {tuple(bias.shape)}, acc {tuple(acc.shape)}, wsum {tuple(wsum.shape)} disagree")
+    dims = _lib.SceneReconstructDims(B, D, H, Wd, w, stride[0], stride[1], grid[0], grid[1], first, n, C, p0, p1, W.shape[0])
+    _lib.check(_lib.lib().msst_scene_reconstruct(ctypes.byref(dims), tokens.data_ptr(), mask.data_ptr(), W.data_ptr(), bias.data_ptr(),
+                                                 weight.data_ptr() if weight is not None else None, acc.data_ptr(), wsum.data_ptr(),
+                                                 torch.cuda.current_stream(acc.device).cuda_stream))
+
+
+def scene_mask(model, B, H, W, *, seed=0, device):
+    """A random scene mask [B, C, H, W] bool (C = spectral blocks) drawn with a SimMIM model's own settings, for held-out evaluation
+    with reconstruct_scene / reconstruction_metrics.  The scene is cut into mask_patch_size x mask_patch_size cells aligned to its
+    origin (partial cells at the bottom / right border count as cells), and exactly ceil(masking_ratio * cells) cells are hidden per
+    scene with tube_masking (every block alike), else per (scene, block) -- MaskGenerator's count, over the scene instead of a window.
+    (Per-window masks would disagree where windows overlap.)  Drawn from a CPU torch.Generator seeded with seed: rows in (scene, block)
+    order, one randperm each, so the mask is reproducible on any machine."""
+    if not isinstance(model, SimMIMSpatialSpectral):
+        raise ValueError(f"scene_mask: needs a SimMIMSpatialSpectral model, got {type(model).__name__}")
+    for name, v in (("B", B), ("H", H), ("W", W)):
+        if isinstance(v, bool) or not isinstance(v, int) or v < 1:
+            raise ValueError(f"scene_mask: {name}={v!r} must be a positive int")
+    if isinstance(seed, bool) or not isinstance(seed, int) or seed < 0:
+        raise ValueError(f"scene_mask: seed={seed!r} must be an int >= 0")
+    C, m = model.encoder.num_spectral_patches, model.mask_patch_size
+    ncy, ncx = -(-H // m), -(-W // m)
+    ncells = ncy * ncx
+    count = int(np.ceil(ncells * model.masking_ratio))
+    rows = B if model.tube_masking else B * C
+    g = torch.Generator().manual_seed(seed)
+    cells = torch.zeros(rows, ncells, dtype=torch.bool)
+    for r in range(rows):
+        cells[r, torch.randperm(ncells, generator=g)[:count]] = True
+    cells = cells.view(rows, ncy, ncx).repeat_interleave(m, 1).repeat_interleave(m, 2)[:, :H, :W]
+    out = cells[:, None].expand(B, C, H, W) if model.tube_masking else cells.view(B, C, H, W)
+    return out.contiguous().to(device)
+
+
+def reconstruction_metrics(recon, scene, mask):
+    """Reconstruction error of recon [B, C*p0, H, W] (reconstruct_scene) against the scene in the model's units, in float64 over the
+    hidden entries of mask [B, C, H, W] (pad bands of RawTiles left out):
+      count                                 hidden entries
+      l1   = mean |recon - target|,  rmse = sqrt(mean (recon - target)^2)
+      baseline_l1 = mean |target|           the error of predicting each band's mean of standardised data (0), so l1 / baseline_l1
+                                            is a scale-free figure
+      per_band_l1 / per_band_rmse / per_band_count   the same per band ([bands] float64 / int64 tensors on the CPU)
+    An empty mask gives count 0 and NaN errors.  For a one-window scene, l1 / num_masked is SimMIM's training loss on that mask.
+    -> dict."""
+    who = "reconstruction_metrics"
+    tiles = scene.tiles if isinstance(scene, RawTiles) else scene
+    if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
+        raise ValueError(f"{who}: scene must be a [B, C, H, W] tensor or RawTiles")
+    B, nb, H, W = tiles.shape
+    if not isinstance(recon, torch.Tensor) or recon.dim() != 4 or recon.shape[0] != B or tuple(recon.shape[2:]) != (H, W):
+        raise ValueError(f"{who}: recon must be a [{B}, bands, {H}, {W}] tensor, got "
+                         f"{tuple(recon.shape) if isinstance(recon, torch.Tensor) else type(recon).__name__}")
+    if not isinstance(mask, torch.Tensor) or mask.dim() != 4 or mask.shape[1] < 1 or recon.shape[1] % mask.shape[1]:
+        raise ValueError(f"{who}: mask must be [B, C, H, W] with C dividing the {recon.shape[1]} bands of recon")
+    C = mask.shape[1]
+    _check_scene_mask(who, mask, B, C, H, W, recon.device)
+    p0 = recon.shape[1] // C
+    if not isinstance(scene, RawTiles) and nb != recon.shape[1] or isinstance(scene, RawTiles) and nb + scene.pad_bands != recon.shape[1]:
+        raise ValueError(f"{who}: recon has {recon.shape[1]} bands, the scene {nb}"
+                         f"{f' + {scene.pad_bands} pad' if isinstance(scene, RawTiles) else ''}")
+    target = _model_units(scene, pad=False).to(device=recon.device, dtype=torch.float64)
+    hidden = mask.repeat_interleave(p0, 1)[:, :nb]
+    d = torch.where(hidden, recon[:, :nb].double() - target, 0.0)
+    t = torch.where(hidden, target, 0.0)
+    cnt = hidden.sum((0, 2, 3)).cpu()
+    s1, s2, st = d.abs().sum((0, 2, 3)).cpu(), (d * d).sum((0, 2, 3)).cpu(), t.abs().sum((0, 2, 3)).cpu()
+    n = cnt.sum().double()
+    return dict(count=int(n), l1=float(s1.sum() / n), rmse=float((s2.sum() / n).sqrt()), baseline_l1=float(st.sum() / n),
+                per_band_l1=s1 / cnt, per_band_rmse=(s2 / cnt).sqrt(), per_band_count=cnt)
 
 
 def confusion_matrix(pred, labels, num_classes, ignore_index=-1):

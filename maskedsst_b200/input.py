@@ -107,11 +107,16 @@ class RawTiles:
         band = torch.arange(self.tiles.shape[1], device=dev)
         win = self.tiles[t[:, None, None, None], band[None, :, None, None], (oy[:, None] + r)[:, None, :, None],
                          (ox[:, None] + r)[:, None, None, :]]   # [n, raw_bands, s, s]
-        win = win.to(torch.int32).to(torch.float64) if win.dtype != torch.float32 else win.to(torch.float64)
-        x = ((win - self.means[None, :, None, None]) / self.stds[None, :, None, None]).to(torch.float32)
+        return self.standardize(win, pad=True)
+
+    def standardize(self, raw, pad=True):
+        """Raw values [n, raw_bands, h, w] (the tiles' dtype) -> the fp32 model cube: (raw - mean) / std in float64 rounded once to
+        fp32, the clip, and (pad=True) the zero pad bands -- the arithmetic of the pixel reader (csrc/pixel_source.cuh)."""
+        raw = raw.to(torch.int32).to(torch.float64) if raw.dtype != torch.float32 else raw.to(torch.float64)
+        x = ((raw - self.means[None, :, None, None]) / self.stds[None, :, None, None]).to(torch.float32)
         if self.clip is not None:
             x = torch.clip(x, min=self.clip[0], max=self.clip[1])
-        if self.pad_bands:
+        if pad and self.pad_bands:
             x = torch.nn.functional.pad(x, (0, 0, 0, 0, 0, self.pad_bands), "constant", 0)
         return x.contiguous()
 
