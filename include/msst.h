@@ -433,6 +433,33 @@ MSST_API int msst_kmeans_update(const msst_kmeans_dims* d, const void* workspace
                                 int32_t* empty, msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Mean, covariance and projection of rows (the device half of PCA and of the global RX anomaly detector).  All arithmetic is FP64.
+ *   rows:        x [n, dim] fp32, centred as c = (double)x - mean (fp64 subtraction; the mean is never rounded to fp32).
+ *   slices       rows [16384 s, 16384 s + 16384): a fixed length, independent of the grid and the SM count.  S = ceil(n / 16384).
+ *   msst_moments_workspace  bytes of the workspace of msst_moments_mean / _cov: 8 * S * dim * (dim + 1) (46 MB at n = 1.43 M,
+ *                dim = 256); -1 (and the error message) on bad dims.  Layout: the mean partials [S][dim] fp64, then the covariance
+ *                partials [S][dim][dim] fp64 (only entries i <= j are written).
+ *   msst_moments_mean      mean [dim] fp64 = (sum_s P_s) / n, the slices added in ascending order, P_s = the slice's column sums
+ *                (fp64, rows added in ascending order).
+ *   msst_moments_cov       cov [dim, dim] fp64 = (sum_s Q_s) / (n - 1), the slices added in ascending order, Q_s[i][j] = the fp64 FMA
+ *                chain sum_r c_ri * c_rj over the slice's rows in ascending order (two passes: `mean` is an input, normally from
+ *                msst_moments_mean).  Entry (i, j), i <= j, is written to (i, j) and (j, i): the matrix is exactly symmetric.
+ *   msst_moments_project   W [k, dim] fp64 row-major, 1 <= k <= dim.  y [n, k] fp32: y_ij = fp32(sum_d c_id * W_jd), one fp64 FMA
+ *                chain in ascending d.  score [n] fp32: fp32(sum_j y_ij^2) over the unrounded fp64 y_ij, one fp64 FMA chain in
+ *                ascending j.  Either of y, score may be NULL, not both.  A row's y and score depend only on that row: bitwise
+ *                independent of how the rows are chunked.  PCA: W = the components; RX: W = the whitening matrix, score = the
+ *                squared Mahalanobis distance.
+ * Deterministic: no atomics, every sum runs in the order given.
+ * Limits (MSST_ERR_ARG before any launch, outputs untouched): 1 <= dim <= 256; 2 <= n < 2^31 for the workspace, mean and covariance,
+ * 1 <= n < 2^31 for the projection; 1 <= k <= dim; no NULL pointer other than one of y / score.
+ * ------------------------------------------------------------------------------------------- */
+MSST_API int64_t msst_moments_workspace(int64_t n, int dim);
+MSST_API int msst_moments_mean(int64_t n, int dim, const float* x, void* workspace, double* mean, msst_stream_t stream);
+MSST_API int msst_moments_cov(int64_t n, int dim, const float* x, const double* mean, void* workspace, double* cov, msst_stream_t stream);
+MSST_API int msst_moments_project(int64_t n, int dim, int k, const float* x, const double* mean, const double* W, float* y, float* score,
+                                  msst_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * SimMIM decoder + masked L1 loss (vit_simmim_original.py:314-338, BlockwiseToPixels :9-40):
  *   pred[b,n,:] = W[blk] enc[b, idx[b,n], :] + bias[blk],  blk = idx / S (0 when n_weight_blocks == 1)
  *   target      = raw pixels of patch idx gathered from img (or target_tokens [B,T,P] if not NULL)

@@ -134,6 +134,10 @@ SIGNATURES = {
     "msst_kmeans_seed": (C.c_int, [C.POINTER(KmeansDims), C.c_int, vp, vp, vp, vp, vp, vp, vp]),
     "msst_kmeans_assign": (C.c_int, [C.POINTER(KmeansDims), vp, vp, vp, vp, vp, vp]),
     "msst_kmeans_update": (C.c_int, [C.POINTER(KmeansDims), vp, vp, vp, vp, vp, vp]),
+    "msst_moments_workspace": (C.c_int64, [C.c_int64, C.c_int]),
+    "msst_moments_mean": (C.c_int, [C.c_int64, C.c_int, vp, vp, vp, vp]),
+    "msst_moments_cov": (C.c_int, [C.c_int64, C.c_int, vp, vp, vp, vp, vp]),
+    "msst_moments_project": (C.c_int, [C.c_int64, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp]),
     "msst_simmim_decode_l1_fwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 9 + [vp]),
     "msst_simmim_decode_l1_bwd": (C.c_int, [C.POINTER(DecodeDims)] + [vp] * 11 + [vp]),
     "msst_draw_masks": (C.c_int, [C.POINTER(MaskGenDims), vp, vp, vp]),

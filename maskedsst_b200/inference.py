@@ -32,6 +32,13 @@ patch touches a hidden entry, and csrc/scene.cu decodes the masked tokens with t
 predictions over the covering windows with the same ownership contract as the blends above.  The result is the inpainted scene in
 the model's units; `reconstruction_metrics` gives the held-out masked L1 / RMSE per band and overall, and |recon - scene| is a
 per-pixel reconstruction-error map.
+
+`pca_fit` / `PCA` / `pca_scene` give the principal components of features (or of any rows of up to 256 values): csrc/moments.cu computes
+the mean and the two-pass covariance in FP64 over fixed 16384-row slices, the host takes the float64 eigendecomposition, and the
+projection kernel projects every row in FP64.  `false_colour` turns the first three components into the usual RGB picture of an
+encoder's features.  `rx_scene` is the global RX anomaly detector, the squared Mahalanobis distance of each pixel from the scene's
+Gaussian, on the encoder's features or (model=None) on the raw spectra; `anomaly_metrics` scores any anomaly map, RX or a
+reconstruction-error map, against ground truth: ROC AUC, the ROC and the TPR at fixed false-positive rates.
 """
 import ctypes
 import math
@@ -1118,3 +1125,305 @@ def clustering_metrics(clusters, labels, *, num_clusters, num_classes, ignore_in
     mmap = cont.argmax(0).astype(np.int64)
     return dict(contingency=torch.from_numpy(cont.astype(np.int64)), nmi=nmi, ari=ari, oa_hungarian=matched / N,
                 hungarian_map=torch.from_numpy(hmap), oa_majority=float(cont.max(0).sum()) / N, majority_map=torch.from_numpy(mmap))
+
+
+MOMENTS_MAX_DIM = 256
+
+
+def _moment_rows(who, x, dim=None):
+    """x [n, dim] fp32 CUDA with 1 <= dim <= 256 (and == dim when given) -> contiguous x, else ValueError."""
+    if not isinstance(x, torch.Tensor) or x.dim() != 2 or x.dtype != torch.float32 or not x.is_cuda:
+        raise ValueError(f"{who}: x must be a 2-D fp32 CUDA tensor [rows, dim], got "
+                         f"{tuple(x.shape) if isinstance(x, torch.Tensor) else type(x).__name__}"
+                         f"{f' {x.dtype} on {x.device}' if isinstance(x, torch.Tensor) else ''}")
+    D = x.shape[1]
+    if not 1 <= D <= MOMENTS_MAX_DIM:
+        raise ValueError(f"{who}: feature width {D} outside [1, {MOMENTS_MAX_DIM}]")
+    if dim is not None and D != dim:
+        raise ValueError(f"{who}: x has {D} features, the fit {dim}")
+    if not x.shape[0] < 2 ** 31:
+        raise ValueError(f"{who}: {x.shape[0]} rows; need rows < 2^31")
+    return x.contiguous()
+
+
+def _ridge_arg(who, ridge):
+    if isinstance(ridge, bool) or not isinstance(ridge, (int, float)) or not 0 <= ridge < math.inf:
+        raise ValueError(f"{who}: ridge={ridge!r} must be a finite number >= 0")
+    return float(ridge)
+
+
+def _moments_mean(x, workspace, mean):
+    """msst_moments_mean: mean [dim] fp64 of x [n, dim] (the slice partials go to the workspace)."""
+    _lib.check(_lib.lib().msst_moments_mean(x.shape[0], x.shape[1], x.data_ptr(), workspace.data_ptr(), mean.data_ptr(), _stream(x)))
+
+
+def _moments_cov(x, mean, workspace, cov):
+    """msst_moments_cov: cov [dim, dim] fp64 of x [n, dim] centred on mean (two passes)."""
+    _lib.check(_lib.lib().msst_moments_cov(x.shape[0], x.shape[1], x.data_ptr(), mean.data_ptr(), workspace.data_ptr(), cov.data_ptr(),
+                                           _stream(x)))
+
+
+def _moments_project(x, mean, W, y=None, score=None):
+    """msst_moments_project: y [n, k] = (x - mean) W^T and / or score [n] = sum_j y_j^2, for W [k, dim] fp64."""
+    _lib.check(_lib.lib().msst_moments_project(x.shape[0], x.shape[1], W.shape[0], x.data_ptr(), mean.data_ptr(), W.data_ptr(),
+                                               y.data_ptr() if y is not None else None,
+                                               score.data_ptr() if score is not None else None, _stream(x)))
+
+
+def _sign_rule(vecs):
+    """Flips each row of vecs [k, dim] (numpy float64) so that its entry of largest |value| is positive, the lowest index on ties."""
+    idx = np.argmax(np.abs(vecs), axis=1)
+    flip = vecs[np.arange(vecs.shape[0]), idx] < 0
+    vecs[flip] *= -1.0
+    return vecs
+
+
+class PCA:
+    """Principal components of n rows of dim features, fitted by pca_fit.
+
+    n; mean [dim] and covariance [dim, dim] float64 on the rows' device (covariance with the 1 / (n - 1) normalisation);
+    eigenvalues [dim] float64, descending (as numpy.linalg.eigh returns them, so a zero-variance direction may show as -1e-17);
+    components [dim, dim] float64, one unit eigenvector per row, in the order of the eigenvalues, each signed so that its entry of
+    largest |value| is positive (the lowest index on ties), which keeps false-colour maps stable from run to run."""
+
+    def __init__(self, n, mean, covariance, eigenvalues, components):
+        self.n, self.mean, self.covariance, self.eigenvalues, self.components = n, mean, covariance, eigenvalues, components
+
+    @property
+    def dim(self):
+        return self.mean.shape[0]
+
+    @property
+    def explained_variance_ratio(self):
+        """[dim] float64: each eigenvalue (clipped at 0) over their sum."""
+        lam = self.eigenvalues.clamp_min(0)
+        return lam / lam.sum()
+
+    def _whitening(self, who, k, ridge):
+        """W [k, dim] float64 = components[:k] / sqrt(max(lambda, 0) + eps), eps = ridge * trace / dim."""
+        eps = ridge * float(torch.diagonal(self.covariance).sum()) / self.dim
+        den = self.eigenvalues[:k].clamp_min(0) + eps
+        if not bool((den > 0).all()):
+            raise ValueError(f"{who}: a zero-variance direction with ridge * trace / dim = {eps!r}; raise the ridge")
+        return (self.components[:k] / torch.sqrt(den)[:, None]).contiguous()
+
+    def _project(self, who, x, W, batch_queries, want_y):
+        x = _moment_rows(who, x, self.dim)
+        if x.device != self.mean.device:
+            raise ValueError(f"{who}: x on {x.device}, the fit on {self.mean.device}")
+        if isinstance(batch_queries, bool) or not isinstance(batch_queries, int) or batch_queries < 1:
+            raise ValueError(f"{who}: batch_queries={batch_queries!r} must be a positive int")
+        Q = x.shape[0]
+        out = (torch.empty(Q, W.shape[0], device=x.device, dtype=torch.float32) if want_y
+               else torch.empty(Q, device=x.device, dtype=torch.float32))
+        for first in range(0, Q, batch_queries):
+            last = min(first + batch_queries, Q)
+            if want_y:
+                _moments_project(x[first:last], self.mean, W, y=out[first:last])
+            else:
+                _moments_project(x[first:last], self.mean, W, score=out[first:last])
+        return out
+
+    @torch.no_grad()
+    def transform(self, x, n_components=None, *, whiten=False, ridge=1e-6, batch_queries=262144):
+        """x [Q, dim] fp32 CUDA -> y [Q, k] fp32, y_j = components[j] . (x - mean) in float64, rounded once (k = n_components, default
+        dim).  whiten: y_j / sqrt(max(lambda_j, 0) + eps), eps = ridge * trace(covariance) / dim.  Queries run in chunks of batch_queries;
+        the result is bitwise the same for any chunk size."""
+        who = "PCA.transform"
+        k = self.dim if n_components is None else n_components
+        if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= self.dim:
+            raise ValueError(f"{who}: n_components={n_components!r} must be an int in [1, dim={self.dim}]")
+        if not isinstance(whiten, bool):
+            raise ValueError(f"{who}: whiten={whiten!r} must be a bool")
+        ridge = _ridge_arg(who, ridge)
+        W = self._whitening(who, k, ridge) if whiten else self.components[:k].contiguous()
+        return self._project(who, x, W, batch_queries, True)
+
+    @torch.no_grad()
+    def mahalanobis(self, x, *, ridge=1e-6, batch_queries=262144):
+        """x [Q, dim] fp32 CUDA -> [Q] fp32: the squared Mahalanobis distance (x - mean)^T (covariance + eps I)^-1 (x - mean),
+        eps = ridge * trace(covariance) / dim, as the sum over all components of the whitened projections squared (eigenvalues clipped
+        at 0), added in float64 and rounded once: the global RX anomaly score.  Bitwise the same for any batch_queries."""
+        who = "PCA.mahalanobis"
+        ridge = _ridge_arg(who, ridge)
+        W = self._whitening(who, self.dim, ridge)
+        return self._project(who, x, W, batch_queries, False)
+
+
+@torch.no_grad()
+def pca_fit(x):
+    """Principal component analysis of rows on the device: csrc/moments.cu computes the fp64 mean and the two-pass fp64 covariance in a
+    fixed order (bitwise reproducible), then the host takes numpy's float64 eigh of the (at most 256 x 256) covariance.
+
+    x [n, dim] fp32 CUDA, 1 <= dim <= 256, 2 <= n < 2^31.  -> PCA."""
+    who = "pca_fit"
+    x = _moment_rows(who, x)
+    n, D = x.shape
+    if n < 2:
+        raise ValueError(f"{who}: {n} rows; need at least 2")
+    dev = x.device
+    workspace = torch.empty(_lib.lib().msst_moments_workspace(n, D), device=dev, dtype=torch.uint8)
+    mean = torch.empty(D, device=dev, dtype=torch.float64)
+    cov = torch.empty(D, D, device=dev, dtype=torch.float64)
+    _moments_mean(x, workspace, mean)
+    _moments_cov(x, mean, workspace, cov)
+    lam, vec = np.linalg.eigh(cov.cpu().numpy())
+    lam, vec = lam[::-1].copy(), _sign_rule(vec[:, ::-1].T.copy())
+    return PCA(n, mean, cov, torch.from_numpy(lam).to(dev), torch.from_numpy(vec).to(dev))
+
+
+def _valid_rows(who, valid, B, H, W, device):
+    """valid [B, H, W] bool on device (None: every pixel) -> flat [B*H*W] bool or None, else ValueError."""
+    if valid is None:
+        return None
+    if not isinstance(valid, torch.Tensor) or valid.dtype != torch.bool or valid.shape != (B, H, W) or valid.device != device:
+        raise ValueError(f"{who}: valid must be a bool tensor [{B}, {H}, {W}] on {device}")
+    return valid.reshape(-1)
+
+
+def _feature_width(who, model):
+    """The feature width of embed_scene(model, ...), else ValueError."""
+    enc = model.encoder if isinstance(model, SimMIMSpatialSpectral) else model
+    if not isinstance(enc, ViTSpatialSpectral):
+        raise ValueError(f"{who}: needs a ViTSpatialSpectral encoder, got {type(enc).__name__}")
+    return enc.dim
+
+
+def _scene_rows(who, model, scene, valid, stride, weight, batch_windows):
+    """Checks a scene and its valid mask, then -> (feats [B, D, H, W] fp32, the pixel rows [B*H*W, D], the rows to fit on): the
+    embed_scene features of model, or with model=None the scene's own spectra in model units (RawTiles: standardised and clipped,
+    no pad bands)."""
+    tiles = scene.tiles if isinstance(scene, RawTiles) else scene
+    if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
+        raise ValueError(f"{who}: scene must be a [B, C, H, W] tensor or RawTiles")
+    if not tiles.is_cuda:
+        raise ValueError(f"{who}: the scene must be on a CUDA device")
+    B, _, H, W = tiles.shape
+    D = tiles.shape[1] if model is None else _feature_width(who, model)
+    if not 1 <= D <= MOMENTS_MAX_DIM:
+        raise ValueError(f"{who}: feature width {D} outside [1, {MOMENTS_MAX_DIM}]")
+    keep = _valid_rows(who, valid, B, H, W, tiles.device)
+    fit_n = B * H * W if keep is None else int(keep.sum())
+    if not 2 <= fit_n < 2 ** 31:
+        raise ValueError(f"{who}: {fit_n} pixels to fit on; need 2 <= pixels < 2^31")
+    if model is None:
+        feats = _model_units(scene, pad=False)
+    else:
+        feats = embed_scene(model, scene, stride=stride, weight=weight, batch_windows=batch_windows)
+    flat = _pixel_rows(feats).contiguous()
+    return feats, flat, (flat if keep is None else flat[keep])
+
+
+@torch.no_grad()
+def pca_scene(model, scene, *, n_components=3, valid=None, stride=None, weight=None, batch_windows=4096, batch_queries=262144):
+    """PCA of an encoder's features on whole scenes: embed_scene, a fit on the pixels where valid [B, H, W] (bool, default every pixel)
+    is set, every pixel projected on the first n_components components.  With n_components=3, false_colour(maps) is the usual picture
+    of a self-supervised encoder's features.
+
+    model, scene, stride, weight, batch_windows: as in embed_scene (a SimMIMSpatialSpectral checkpoint works directly);
+    batch_queries: as in PCA.transform.  -> (maps [B, n_components, H, W] fp32, the PCA)."""
+    who = "pca_scene"
+    D = _feature_width(who, model)
+    if isinstance(n_components, bool) or not isinstance(n_components, int) or not 1 <= n_components <= D:
+        raise ValueError(f"{who}: n_components={n_components!r} must be an int in [1, dim={D}]")
+    feats, flat, fit = _scene_rows(who, model, scene, valid, stride, weight, batch_windows)
+    pca = pca_fit(fit)
+    return _pixel_map(pca.transform(flat, n_components, batch_queries=batch_queries), feats), pca
+
+
+@torch.no_grad()
+def rx_scene(model, scene, *, ridge=1e-6, valid=None, stride=None, weight=None, batch_windows=4096, batch_queries=262144):
+    """Global RX (Reed-Xiaoli) anomaly detection on whole scenes: every pixel scored by its squared Mahalanobis distance from the
+    Gaussian (mean, covariance + eps I, eps = ridge * trace / dim) fitted on the pixels where valid [B, H, W] is set (default all).
+
+    model: RX on its embed_scene features (model, scene, stride, weight, batch_windows as in embed_scene); None: RX on the scene's own
+    spectra in model units, the classical baseline (a RawTiles scene standardised and clipped as the model sees it, without the pad
+    bands, whose zero variance would make the covariance singular; stride / weight / batch_windows are not used).
+    Score the map against ground truth with anomaly_metrics.  -> (scores [B, H, W] fp32, the PCA of the fit)."""
+    who = "rx_scene"
+    ridge = _ridge_arg(who, ridge)
+    feats, flat, fit = _scene_rows(who, model, scene, valid, stride, weight, batch_windows)
+    pca = pca_fit(fit)
+    B, _, H, W = feats.shape
+    return pca.mahalanobis(flat, ridge=ridge, batch_queries=batch_queries).reshape(B, H, W), pca
+
+
+def _quantile_sorted(s, q):
+    """Linear-interpolation quantile q of the sorted float64 vector s (numpy's default method)."""
+    pos = q * (s.numel() - 1)
+    i = min(int(math.floor(pos)), s.numel() - 1)
+    j = min(i + 1, s.numel() - 1)
+    t = pos - i
+    a, b = float(s[i]), float(s[j])
+    return a + t * (b - a) if t < 0.5 else b - (b - a) * (1 - t)
+
+
+@torch.no_grad()
+def false_colour(maps, *, lo=0.01, hi=0.99):
+    """maps [B, 3, H, W] (e.g. pca_scene's first three components) -> an RGB image [B, 3, H, W] fp32 in [0, 1]: each channel clipped at
+    its lo / hi quantiles over all pixels of all scenes (linear interpolation, numpy's default) and rescaled to [0, 1]; a channel whose
+    two quantiles are equal maps to 0.  The quantiles come from one sort per channel (torch.quantile refuses more than 2^24 values)."""
+    who = "false_colour"
+    if not isinstance(maps, torch.Tensor) or maps.dim() != 4 or maps.shape[1] != 3 or not maps.dtype.is_floating_point:
+        raise ValueError(f"{who}: maps must be a floating-point tensor [B, 3, H, W], got "
+                         f"{tuple(maps.shape) if isinstance(maps, torch.Tensor) else type(maps).__name__}")
+    if maps.numel() == 0:
+        raise ValueError(f"{who}: maps is empty")
+    for name, v in (("lo", lo), ("hi", hi)):
+        if isinstance(v, bool) or not isinstance(v, (int, float)) or not 0 <= v <= 1:
+            raise ValueError(f"{who}: {name}={v!r} must be a number in [0, 1]")
+    if not lo < hi:
+        raise ValueError(f"{who}: lo={lo!r} must be below hi={hi!r}")
+    out = torch.empty(maps.shape, device=maps.device, dtype=torch.float32)
+    for c in range(3):
+        v = maps[:, c].double()
+        s = torch.sort(v.reshape(-1)).values
+        a, b = _quantile_sorted(s, lo), _quantile_sorted(s, hi)
+        out[:, c] = ((v.clamp(a, b) - a) / (b - a)).float() if b > a else 0.0
+    return out
+
+
+ANOMALY_FPRS = (1e-3, 1e-2, 1e-1)
+
+
+def anomaly_metrics(score, anomalies, valid=None):
+    """Scores an anomaly map against ground truth on the host, in float64: any per-pixel score (rx_scene, |recon - scene| reduced over
+    bands, ...) where larger means more anomalous.  score: a real tensor / array; anomalies: bool of the same shape; valid: optional
+    bool of the same shape, the pixels that count (default all).  NaN scores among them are refused.
+      auc                     the Mann-Whitney statistic: the share of (anomaly, background) pairs whose anomaly scores higher, tied
+                              pairs counting 1/2 (= the area under the ROC below)
+      n_anomalies, n_background
+      thresholds, fpr, tpr    the ROC over the distinct scores t in descending order, a pixel counted anomalous when score >= t
+                              (float64 CPU tensors)
+      tpr_at_fpr              {f: the best TPR among the thresholds with FPR <= f} for f in 1e-3, 1e-2, 1e-1 (0.0 when none, the
+                              threshold above every score)
+    ValueError when either class is empty."""
+    who = "anomaly_metrics"
+    s = torch.as_tensor(score)
+    a = torch.as_tensor(anomalies)
+    if s.dtype == torch.bool or s.dtype.is_complex:
+        raise ValueError(f"{who}: score must be a real tensor, got {s.dtype}")
+    if a.dtype != torch.bool or a.shape != s.shape:
+        raise ValueError(f"{who}: anomalies must be a bool tensor of the score's shape {tuple(s.shape)}, got {a.dtype} {tuple(a.shape)}")
+    s = s.detach().reshape(-1).to("cpu", torch.float64).numpy()
+    a = a.reshape(-1).cpu().numpy()
+    if valid is not None:
+        v = torch.as_tensor(valid)
+        if v.dtype != torch.bool or v.numel() != s.size:
+            raise ValueError(f"{who}: valid must be a bool tensor of the score's shape")
+        v = v.reshape(-1).cpu().numpy()
+        s, a = s[v], a[v]
+    if np.isnan(s).any():
+        raise ValueError(f"{who}: NaN scores")
+    na, nb = int(a.sum()), int((~a).sum())
+    if na == 0 or nb == 0:
+        raise ValueError(f"{who}: {na} anomalous and {nb} background pixels; need both")
+    u, inv = np.unique(s, return_inverse=True)
+    tp_g = np.bincount(inv, weights=a.astype(np.float64), minlength=u.size)[::-1]   # per distinct score, descending
+    fp_g = np.bincount(inv, weights=(~a).astype(np.float64), minlength=u.size)[::-1]
+    tp, fp = np.cumsum(tp_g), np.cumsum(fp_g)
+    auc = float(np.sum(fp_g * (tp - 0.5 * tp_g))) / (float(na) * float(nb))
+    tpr, fpr = tp / na, fp / nb
+    at = {f: float(tpr[fpr <= f].max()) if bool((fpr <= f).any()) else 0.0 for f in ANOMALY_FPRS}
+    return dict(auc=auc, n_anomalies=na, n_background=nb, thresholds=torch.from_numpy(u[::-1].copy()),
+                fpr=torch.from_numpy(fpr), tpr=torch.from_numpy(tpr), tpr_at_fpr=at)
