@@ -102,6 +102,17 @@ MSST_API int msst_patch_embed_bwd(const msst_embed_dims* d, const float* img, co
                          const uint8_t* mask, const float* d_tokens, const float* d_patches_ln /*or NULL*/,
                          float* d_pre_w, float* d_pre_b, float* d_W, float* d_bias, float* d_post_w,
                          float* d_post_b, float* d_pos, float* d_mask_token, msst_stream_t stream);
+/* Data gradient of the same map: d_img [B, C*p0, G*p1, G*p1] fp32 = d(tokens, patches_ln) / d(img) applied to d_tokens [B,T,D] and
+ * d_patches_ln [B,T,P] (or NULL), for the fp32 cube `img`.  Per token: g_o = d_tokens * emb-dropout factor (0 when the token is
+ * masked: mask-token select), g_z = LN_D'(g_o * post_w), g_h = W_blk^T g_z + d_patches_ln (which still flows for masked tokens),
+ * g_x = LN_P'(g_h * pre_w), written to the patch's pixels.  Patches tile the image: every element of d_img is written exactly once
+ * (plain stores, bitwise deterministic; the caller need not zero it).  No parameter gradient is formed (msst_patch_embed_bwd).
+ * D in {32, 64, 96, 128}, P <= 64, n_weight_blocks in {1, C}, drop_p in [0, 1], d->raw == NULL (raw tiles have no gradient),
+ * img / d_tokens / d_img non-NULL; MSST_ERR_ARG before any launch otherwise, d_img untouched. */
+MSST_API int msst_patch_embed_bwd_data(const msst_embed_dims* d, const float* img, const float* pre_w, const float* pre_b,
+                                       const float* W, const float* bias, const float* post_w, const float* post_b,
+                                       const uint8_t* mask, const float* d_tokens, const float* d_patches_ln /*or NULL*/,
+                                       float* d_img, msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * (4) LayerNorm (nn.LayerNorm, biased variance, eps inside sqrt; PreNorm vit_spatial_spectral.py:22-29)
@@ -314,6 +325,20 @@ typedef struct {
 } msst_scene_reconstruct_dims;
 MSST_API int msst_scene_reconstruct(const msst_scene_reconstruct_dims* d, const float* tokens, const uint8_t* mask, const float* W,
                                     const float* bias, const float* weight, float* acc, float* wsum, msst_stream_t stream);
+/* Whole-scene integrated-gradients attribution: the same windows, chunks, weight and ownership contract as msst_scene_blend, but each
+ * covering window contributes its input gradients at the pixel, summed over the integration steps.  One call adds the chunk
+ * [win_first, win_first + n):
+ *   grads [n, steps, bands, win, win]  d objective / d input of every interpolated window (window-major, step-minor), read in place
+ *   weight [win, win] or NULL          per-window-pixel weight (NULL: 1)
+ *   acc  [B, bands, H, W] +=  weight(py, px) * sum_{k ascending} grads[g - win_first, k, band, py, px]   over covering windows g, ascending
+ *   wsum [B, H, W]        +=  weight(py, px)
+ * Bitwise independent of the chunking (chunks in ascending order); only the scene rows the chunk touches are visited.
+ * 1 <= stride <= win <= H, W;  win_y <= ceil((H - win) / stride_y) + 1 (ditto x);  bands, steps >= 1.  MSST_ERR_ARG before any launch
+ * otherwise, outputs untouched.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct { int B, bands, H, W, win, stride_y, stride_x, win_y, win_x, win_first, n, steps; } msst_scene_attribute_dims;
+MSST_API int msst_scene_attribute(const msst_scene_attribute_dims* d, const float* grads, const float* weight, float* acc, float* wsum,
+                                  msst_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * k-nearest-neighbour probing of embeddings (e.g. msst_scene_embed maps): cosine similarity, k best references per query, class vote.

@@ -65,6 +65,10 @@ class SceneReconstructDims(C.Structure):   # msst_scene_reconstruct_dims
                                        "p1", "n_wb")]
 
 
+class SceneAttributeDims(C.Structure):   # msst_scene_attribute_dims
+    _fields_ = [(n, C.c_int) for n in ("B", "bands", "H", "W", "win", "stride_y", "stride_x", "win_y", "win_x", "win_first", "n", "steps")]
+
+
 class KnnDims(C.Structure):   # msst_knn_dims
     _fields_ = [("n_ref", C.c_int64), ("n_query", C.c_int64), ("dim", C.c_int), ("k", C.c_int)]
 
@@ -101,6 +105,7 @@ SIGNATURES = {
     "msst_launch_count": (C.c_longlong, []),
     "msst_patch_embed_fwd": (C.c_int, [C.POINTER(EmbedDims)] + [vp] * 12 + [vp]),
     "msst_patch_embed_bwd": (C.c_int, [C.POINTER(EmbedDims)] + [vp] * 18 + [vp]),
+    "msst_patch_embed_bwd_data": (C.c_int, [C.POINTER(EmbedDims)] + [vp] * 11 + [vp]),
     "msst_layernorm_fwd": (C.c_int, [vp, vp, vp, vp, C.c_int, vp, C.c_int64, C.c_int, C.c_float, vp]),
     "msst_layernorm_bwd": (C.c_int, [vp] * 8 + [C.c_int64, C.c_int, vp]),
     "msst_linear_fwd": (C.c_int, [C.POINTER(LinearDims)] + [vp] * 6 + [vp]),
@@ -123,6 +128,7 @@ SIGNATURES = {
     "msst_scene_blend": (C.c_int, [C.POINTER(SceneDims), vp, vp, vp, vp, vp]),
     "msst_scene_embed": (C.c_int, [C.POINTER(SceneEmbedDims), vp, vp, vp, vp, vp]),
     "msst_scene_reconstruct": (C.c_int, [C.POINTER(SceneReconstructDims)] + [vp] * 7 + [vp]),
+    "msst_scene_attribute": (C.c_int, [C.POINTER(SceneAttributeDims)] + [vp] * 4 + [vp]),
     "msst_knn_prepare": (C.c_int, [vp, C.c_int64, C.c_int, vp, vp]),
     "msst_knn_topk": (C.c_int, [C.POINTER(KnnDims), vp, vp, vp, vp, vp]),
     "msst_knn_vote": (C.c_int, [C.c_int64, C.c_int, C.c_int64, vp, vp, vp, C.c_int, C.c_float, vp, vp, vp]),

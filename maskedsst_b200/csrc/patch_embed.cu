@@ -27,7 +27,9 @@ __device__ __forceinline__ float load_pixel(const EmbedGeom& g, int b, int c, in
     return g.src.load(b, c * g.p0 + p0i, h * g.p1 + p1i, w * g.p1 + p2i);
 }
 
-// loads the chunk's raw patches into xs[tok][P+1] and pre-normalises: xs <- xhat, hs <- xhat*w+b
+// loads the chunk's raw patches into xs[tok][P+1] and pre-normalises: xs <- xhat, hs <- xhat*w+b.  kShift: the statistics are taken
+// of x - x[0] (exact for a patch within a factor 2 of its first value), so a row far from 0 keeps its deviations to full precision
+template <bool kShift = false>
 __device__ __forceinline__ void load_and_prenorm(const EmbedGeom& g, int b, int c, int s0,
                                                  const float* __restrict__ pre_w, const float* __restrict__ pre_b,
                                                  float* xs, float* hs, float* rstd_s) {
@@ -40,15 +42,16 @@ __device__ __forceinline__ void load_and_prenorm(const EmbedGeom& g, int b, int 
     __syncthreads();
     if (threadIdx.x < kTok) {
         const int tok = threadIdx.x;
+        const float x0 = kShift ? xs[tok * ld] : 0.f;
         float mean = 0.f;
-        for (int p = 0; p < P; ++p) mean += xs[tok * ld + p];
+        for (int p = 0; p < P; ++p) mean += xs[tok * ld + p] - x0;
         mean /= P;
         float var = 0.f;
-        for (int p = 0; p < P; ++p) { const float dlt = xs[tok * ld + p] - mean; var += dlt * dlt; }
+        for (int p = 0; p < P; ++p) { const float dlt = (xs[tok * ld + p] - x0) - mean; var += dlt * dlt; }
         const float rstd = rsqrtf(var / P + 1e-5f);
         rstd_s[tok] = rstd;
         for (int p = 0; p < P; ++p) {
-            const float xh = (xs[tok * ld + p] - mean) * rstd;
+            const float xh = ((xs[tok * ld + p] - x0) - mean) * rstd;
             xs[tok * ld + p] = xh;
             hs[tok * ld + p] = xh * pre_w[p] + pre_b[p];
         }
@@ -313,6 +316,108 @@ patch_embed_bwd_kernel(EmbedGeom g, int n_wb, const float* __restrict__ img, con
     if (d_patches_ln && lane < P) { atomicAdd(d_pre_w + lane, a_plw); atomicAdd(d_pre_b + lane, a_plb); }
 }
 
+// Offset in the [B, C*p0, G*p1, G*p1] cube of element p of patch (b, c, s): the (p0i, p1i, p2i) order of load_pixel.
+__device__ __forceinline__ int64_t pixel_offset(const EmbedGeom& g, int b, int c, int s, int p) {
+    const int pp = g.p1 * g.p1;
+    const int p0i = p / pp, r = p % pp, p1i = r / g.p1, p2i = r % g.p1;
+    const int h = s / g.G, w = s % g.G;
+    return ((int64_t)b * g.C * g.p0 + c * g.p0 + p0i) * g.HW + (int64_t)(h * g.p1 + p1i) * g.Wimg + w * g.p1 + p2i;
+}
+
+// Data gradient (msst_patch_embed_bwd_data): the forward's decomposition, one CTA per (b, c, 64-token chunk), one warp per token with
+// lanes over D.  Per token: g_o = d_tokens * drop factor (0 when masked), g_z = LN_D'(g_o * post_w), g_h = W^T g_z (+ d_patches_ln),
+// g_x = LN_P'(g_h * pre_w).  g_z goes through shared memory so that W^T g_z is a per-lane dot product over D (lane p, p + 32), with no
+// reduction across lanes; g_x is staged in xs and stored with the load's (coalesced) order.  Patches tile the image, so every element of
+// d_img is written exactly once, by plain stores.
+template <int NJ>
+__global__ void __launch_bounds__(kThreads)
+patch_embed_bwd_data_kernel(EmbedGeom g, int n_wb, const float* __restrict__ img, const float* __restrict__ pre_w,
+                            const float* __restrict__ pre_b, const float* __restrict__ W, const float* __restrict__ bias,
+                            const float* __restrict__ post_w, const float* __restrict__ post_b, const uint8_t* __restrict__ mask,
+                            const float* __restrict__ d_tokens, const float* __restrict__ d_patches_ln, float* __restrict__ d_img,
+                            Drop drop) {
+    extern __shared__ float smem[];
+    const int P = g.P, ld = P + 1;
+    constexpr int D = NJ * 32;
+    float* xs = smem;                    // [64][P+1]  xhat, then g_x
+    float* hs = xs + kTok * ld;          // [64][P+1]
+    float* Ws = hs + kTok * ld;          // [D][P+1]
+    float* rstd_s = Ws + D * ld;         // [64]
+    float* gz_s = rstd_s + kTok;         // [8 warps][D]
+    const int chunks = (g.S + kTok - 1) / kTok;
+    const int chunk = blockIdx.x % chunks, c = (blockIdx.x / chunks) % g.C, b = blockIdx.x / (chunks * g.C);
+    const int s0 = chunk * kTok;
+    const int wb = n_wb == 1 ? 0 : c;
+    for (int i = threadIdx.x; i < D * P; i += kThreads) Ws[(i / P) * ld + (i % P)] = __ldg(W + (int64_t)wb * D * P + i);
+    load_and_prenorm<true>(g, b, c, s0, pre_w, pre_b, xs, hs, rstd_s);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    float* gz = gz_s + warp * D;
+    float bj[NJ], pw[NJ];
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) { bj[j] = bias[wb * D + lane + 32 * j]; pw[j] = post_w[lane + 32 * j]; }
+    const float pre0 = lane < P ? pre_w[lane] : 0.f, pre1 = lane + 32 < P ? pre_w[lane + 32] : 0.f;
+    for (int k = 0; k < kTok / 8; ++k) {
+        const int tok = warp * (kTok / 8) + k, s = s0 + tok;
+        if (s >= g.S) break;
+        const int64_t row = (int64_t)b * g.T + c * g.S + s;
+        const bool masked = mask && mask[row];
+        float gh0 = 0.f, gh1 = 0.f;      // g_h at p = lane, lane + 32
+        if (!masked) {
+            float y[NJ], sum = 0.f;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) {
+                const int f = lane + 32 * j;
+                float acc = bj[j];
+                for (int p = 0; p < P; ++p) acc = fmaf(Ws[f * ld + p], hs[tok * ld + p], acc);
+                y[j] = acc; sum += acc;
+            }
+            const float mean = warp_sum(sum) / D;
+            float sq = 0.f;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) { y[j] -= mean; sq += y[j] * y[j]; }
+            const float rstd = rsqrtf(warp_sum(sq) / D + 1e-5f);
+            float c1 = 0.f, c2 = 0.f, dyh[NJ];
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) {
+                const int f = lane + 32 * j;
+                float go = d_tokens[row * D + f];
+                if (drop.on()) go *= drop_factor(drop, (uint64_t)row * D + f);
+                y[j] *= rstd;
+                dyh[j] = go * pw[j];
+                c1 += dyh[j]; c2 += dyh[j] * y[j];
+            }
+            c1 = warp_sum(c1) / D; c2 = warp_sum(c2) / D;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) gz[lane + 32 * j] = rstd * (dyh[j] - c1 - y[j] * c2);
+            __syncwarp();
+            const int q0 = lane < P ? lane : 0, q1 = lane + 32 < P ? lane + 32 : 0;   // lanes past P compute an unused column
+            for (int f = 0; f < D; ++f) {
+                const float gf = gz[f];
+                gh0 = fmaf(Ws[f * ld + q0], gf, gh0);
+                if (P > 32) gh1 = fmaf(Ws[f * ld + q1], gf, gh1);
+            }
+            __syncwarp();
+        }
+        if (d_patches_ln) {
+            if (lane < P) gh0 += d_patches_ln[row * P + lane];
+            if (lane + 32 < P) gh1 += d_patches_ln[row * P + lane + 32];
+        }
+        const float xh0 = lane < P ? xs[tok * ld + lane] : 0.f, xh1 = lane + 32 < P ? xs[tok * ld + lane + 32] : 0.f;
+        const float gx0 = lane < P ? gh0 * pre0 : 0.f, gx1 = lane + 32 < P ? gh1 * pre1 : 0.f;
+        const float m1 = warp_sum(gx0 + gx1) / P, m2 = warp_sum(gx0 * xh0 + gx1 * xh1) / P;
+        const float r = rstd_s[tok];
+        __syncwarp();
+        if (lane < P) xs[tok * ld + lane] = r * (gx0 - m1 - xh0 * m2);
+        if (lane + 32 < P) xs[tok * ld + lane + 32] = r * (gx1 - m1 - xh1 * m2);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < kTok * P; i += kThreads) {
+        const int tok = i % kTok, p = i / kTok, s = s0 + tok;
+        if (s < g.S) d_img[pixel_offset(g, b, c, s, p)] = xs[tok * ld + p];
+    }
+}
+
 static int make_geom(const msst_embed_dims* d, const float* img, EmbedGeom& g) {
     MSST_REQUIRE(d && d->B > 0 && d->C > 0 && d->G > 0 && d->p0 > 0 && d->p1 > 0, "patch_embed: bad dims");
     MSST_REQUIRE(d->D % 32 == 0 && d->D >= 32 && d->D <= 256, "patch_embed: D=%d must be a multiple of 32 in [32,256]", d->D);
@@ -404,4 +509,31 @@ extern "C" int msst_patch_embed_bwd(const msst_embed_dims* d, const float* img, 
 #undef MSST_BWD
     set_error("patch_embed_bwd: (D=%d, P=%d) unsupported", g.D, g.P);
     return MSST_ERR_ARG;
+}
+
+extern "C" int msst_patch_embed_bwd_data(const msst_embed_dims* d, const float* img, const float* pre_w, const float* pre_b,
+                                         const float* W, const float* bias, const float* post_w, const float* post_b,
+                                         const uint8_t* mask, const float* d_tokens, const float* d_patches_ln, float* d_img,
+                                         msst_stream_t stream) {
+    MSST_REQUIRE(d, "patch_embed_bwd_data: bad dims");
+    MSST_REQUIRE(!d->raw, "patch_embed_bwd_data: raw tiles have no gradient (dims.raw must be NULL)");
+    MSST_REQUIRE(img && d_img && d_tokens, "patch_embed_bwd_data: img / d_tokens / d_img must be set");
+    EmbedGeom g;
+    if (int rc = make_geom(d, img, g)) return rc;
+    MSST_REQUIRE(g.D <= 128, "patch_embed_bwd_data: D=%d unsupported (32,64,96,128)", g.D);
+    const size_t smem = sizeof(float) * ((size_t)2 * kTok * (g.P + 1) + (size_t)g.D * (g.P + 1) + kTok + (size_t)8 * g.D);
+    const Drop drop = make_drop(d->drop_p, d->seed, kSiteEmb, d->seed_dev);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int chunks = (g.S + kTok - 1) / kTok;
+#define MSST_BD(NJ)                                                                                                                 \
+    case NJ:                                                                                                                        \
+        MSST_CUDA(cudaFuncSetAttribute(patch_embed_bwd_data_kernel<NJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
+        patch_embed_bwd_data_kernel<NJ><<<g.B * g.C * chunks, kThreads, smem, st>>>(g, d->n_weight_blocks, img, pre_w, pre_b, W, bias, \
+                                                                                   post_w, post_b, mask, d_tokens, d_patches_ln,    \
+                                                                                   d_img, drop);                                    \
+        break;
+    switch (g.D / 32) { MSST_BD(1) MSST_BD(2) MSST_BD(3) MSST_BD(4) }
+#undef MSST_BD
+    MSST_LAUNCH_CHECK();
+    return MSST_OK;
 }

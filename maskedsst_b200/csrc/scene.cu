@@ -5,7 +5,8 @@
 // One thread owns one scene pixel and adds its covering windows in ascending global window index, one at a time (acc = acc + c): no
 // atomics, so the sums are bitwise independent of how the windows were cut into chunks.  Which windows cover the pixel follows from
 // the origin rule of the pixel reader (window_origin, pixel_source.cuh); the windows are never enumerated.  msst_scene_embed blends
-// per-pixel encoder features and msst_scene_reconstruct the SimMIM decoder's predictions of masked values the same way (below).
+// per-pixel encoder features, msst_scene_reconstruct the SimMIM decoder's predictions of masked values and msst_scene_attribute the
+// integrated-gradients sums of input gradients the same way (below).
 #include "common.cuh"
 #include "pixel_source.cuh"
 
@@ -221,6 +222,46 @@ __global__ void __launch_bounds__(kEmbedThreads) scene_reconstruct_kernel(SceneG
     }
 }
 
+// Integrated-gradients attribution (msst_scene_attribute): the same ownership and window order as the blend, but each covering window
+// contributes its input gradients at the pixel summed over the integration steps, sum_k grads[window, k, band, py, px] with k ascending,
+// so the [n, steps, bands, win, win] gradients are read once.  One thread owns one scene pixel; bands are the outer loop, so each band's
+// running sum stays in a register (the covering windows are recomputed per band: integer work only).  Consecutive threads own
+// consecutive columns: acc is read and stored coalesced, and the gradients are read in runs along window rows.
+constexpr int kAttrThreads = 128;
+
+__global__ void __launch_bounds__(kAttrThreads) scene_attribute_kernel(SceneGeom g, int steps, const float* __restrict__ grads,
+                                                                       const float* __restrict__ weight, float* __restrict__ acc,
+                                                                       float* __restrict__ wsum) {
+    const int64_t q = (int64_t)blockIdx.x * kAttrThreads + threadIdx.x;
+    if (q >= g.npix) return;
+    const int64_t p = g.pix0 + q;
+    const int64_t HW = (int64_t)g.H * g.W;
+    const int b = (int)(p / HW), y = (int)((p / g.W) % g.H), x = (int)(p % g.W);
+    const int nb = g.nc, ww = g.win * g.win;
+    float ws = 0.f;
+    bool any = false;
+    for_each_covering_window(g, b, y, x, [&](int64_t, int py, int px) {
+        if (!any) { any = true; ws = wsum[p]; }
+        ws = __fadd_rn(ws, weight ? __ldg(weight + py * g.win + px) : 1.f);
+    });
+    if (!any) return;
+    wsum[p] = ws;
+    float* ap = acc + (int64_t)b * nb * HW + (int64_t)y * g.W + x;
+    const int64_t kstride = (int64_t)nb * ww;
+    for (int band = 0; band < nb; ++band) {
+        float a = ap[band * HW];
+        for_each_covering_window(g, b, y, x, [&](int64_t gw, int py, int px) {
+            const float wt = weight ? __ldg(weight + py * g.win + px) : 1.f;
+            const float* gp = grads + ((gw - g.g0) * steps * nb + band) * ww + py * g.win + px;
+            float s = 0.f;
+#pragma unroll 4
+            for (int k = 0; k < steps; ++k) s = __fadd_rn(s, __ldg(gp + k * kstride));
+            a = __fadd_rn(a, __fmul_rn(wt, s));
+        });
+        ap[band * HW] = a;
+    }
+}
+
 static int64_t windows_along(int extent, int win, int step) { return (extent - win + step - 1) / step + 1; }
 
 // Checks the window geometry both entry points share (msst_scene_dims and msst_scene_embed_dims name it alike) and fills g: the
@@ -308,6 +349,19 @@ extern "C" int msst_scene_reconstruct(const msst_scene_reconstruct_dims* d, cons
         break;
     switch (d->D / 32) { MSST_R(1) MSST_R(2) MSST_R(3) MSST_R(4) MSST_R(5) MSST_R(6) MSST_R(7) MSST_R(8) }
 #undef MSST_R
+    MSST_LAUNCH_CHECK();
+    return MSST_OK;
+}
+
+extern "C" int msst_scene_attribute(const msst_scene_attribute_dims* d, const float* grads, const float* weight, float* acc, float* wsum,
+                                    msst_stream_t stream) {
+    MSST_REQUIRE(d && d->B > 0 && d->bands > 0 && d->win > 0 && d->steps > 0, "scene_attribute: bad dims");
+    SceneGeom g;
+    const int rc = scene_geom("scene_attribute", d, d->bands, g);
+    if (rc != MSST_OK) return rc;
+    MSST_REQUIRE(grads && acc && wsum, "scene_attribute: grads / acc / wsum must be set");
+    scene_attribute_kernel<<<(unsigned)ceil_div(g.npix, kAttrThreads), kAttrThreads, 0, (cudaStream_t)stream>>>(g, d->steps, grads, weight,
+                                                                                                              acc, wsum);
     MSST_LAUNCH_CHECK();
     return MSST_OK;
 }

@@ -39,6 +39,11 @@ projection kernel projects every row in FP64.  `false_colour` turns the first th
 encoder's features.  `rx_scene` is the global RX anomaly detector, the squared Mahalanobis distance of each pixel from the scene's
 Gaussian, on the encoder's features or (model=None) on the raw spectra; `anomaly_metrics` scores any anomaly map, RX or a
 reconstruction-error map, against ground truth: ROC AUC, the ROC and the TPR at fixed false-positive rates.
+
+`attribute_windows` / `attribute_scene` answer which bands at which pixels drove a classifier's decision: integrated gradients of each
+pixel's target-class logit with respect to the input cube, through the model's own kernels (the patch embedding's data gradient is
+csrc/patch_embed.cu, msst_patch_embed_bwd_data), with the step sums blended over overlapping windows by csrc/scene.cu under the same
+ownership contract as the blends above.  `band_importance` reduces an attribution map to per-class band profiles.
 """
 import ctypes
 import math
@@ -49,7 +54,7 @@ import torch
 from . import _lib
 from .input import RawTiles
 from .vit_simmim_original import SimMIMSpatialSpectral
-from .vit_spatial_spectral import ViTSpatialSpectral
+from .vit_spatial_spectral import ViTSpatialSpectral, ViTSpatialSpectral_V1
 
 
 @torch.no_grad()
@@ -1427,3 +1432,252 @@ def anomaly_metrics(score, anomalies, valid=None):
     at = {f: float(tpr[fpr <= f].max()) if bool((fpr <= f).any()) else 0.0 for f in ANOMALY_FPRS}
     return dict(auc=auc, n_anomalies=na, n_background=nb, thresholds=torch.from_numpy(u[::-1].copy()),
                 fpr=torch.from_numpy(fpr), tpr=torch.from_numpy(tpr), tpr_at_fpr=at)
+
+
+def ig_alphas(steps):
+    """The integration points of attribute_windows / attribute_scene: alpha_k = (k + 1/2) / steps, k = 0 .. steps - 1 (the midpoint rule,
+    ascending), as float64."""
+    return (torch.arange(steps, dtype=torch.float64) + 0.5) / steps
+
+
+def _attr_model(who, model):
+    """-> (bands, window side, classes) of a classifier whose head gives [n, nc, w, w], else ValueError."""
+    if isinstance(model, SimMIMSpatialSpectral):
+        raise ValueError(f"{who}: needs a classifier (ViTSpatialSpectral or ViTSpatialSpectral_V1), got a SimMIM model; attribute its "
+                         f"encoder after fine-tuning instead")
+    if not isinstance(model, (ViTSpatialSpectral, ViTSpatialSpectral_V1)):
+        raise ValueError(f"{who}: needs a ViTSpatialSpectral or ViTSpatialSpectral_V1, got {type(model).__name__}")
+    if getattr(model, "pixelwise", False):
+        raise ValueError(f"{who}: the pixelwise head gives one class vector per window; attribution needs a head that classifies every "
+                         f"pixel ([n, nc, w, w])")
+    return model.num_spectral_patches * model.patch_depth, model.image_size, model.num_classes
+
+
+def _steps_arg(who, steps):
+    if isinstance(steps, bool) or not isinstance(steps, int) or steps < 1:
+        raise ValueError(f"{who}: steps={steps!r} must be an int >= 1")
+    return steps
+
+
+def _baseline_arg(who, baseline, bands, device):
+    """-> [bands] fp32 on device: the baseline spectrum x' (None: 0 in model units, the band mean of a standardised scene)."""
+    if baseline is None:
+        return torch.zeros(bands, dtype=torch.float32, device=device)
+    b = torch.as_tensor(baseline)
+    if b.dtype == torch.bool or b.dtype.is_complex or tuple(b.shape) != (bands,):
+        raise ValueError(f"{who}: baseline must be a real [{bands}] spectrum, got {b.dtype} {tuple(b.shape)}")
+    b = b.to(device=device, dtype=torch.float32).contiguous()
+    if not bool(torch.isfinite(b).all()):
+        raise ValueError(f"{who}: baseline has non-finite values")
+    return b
+
+
+def _target_arg(who, target, shape, device):
+    if (not isinstance(target, torch.Tensor) or tuple(target.shape) != shape or target.dtype.is_floating_point
+            or target.dtype.is_complex or target.dtype == torch.bool or target.device != device):
+        got = f"{target.dtype} {tuple(target.shape)} on {target.device}" if isinstance(target, torch.Tensor) else type(target).__name__
+        raise ValueError(f"{who}: target must be an integer tensor {list(shape)} on {device}, got {got}")
+    return target.to(torch.int64)
+
+
+def _objective_weights(target, nc):
+    """[n, w, w] int64 -> [n, nc, w, w] fp32: dF/dlogits of F = sum over counted pixels p of logits[target(p), p].  A pixel counts when
+    its target is in [0, nc) (so != -1): the rule of confusion_matrix."""
+    valid = (target >= 0) & (target < nc)
+    oh = torch.nn.functional.one_hot(torch.where(valid, target, 0), nc).permute(0, 3, 1, 2)
+    return (oh * valid[:, None]).to(torch.float32).contiguous()
+
+
+def _interpolate(windows, base, steps):
+    """[n, bands, w, w] windows -> [n * steps, bands, w, w] fp32 (window-major, step-minor): x' + alpha_k (x - x'), x' = base [bands]."""
+    a = ig_alphas(steps).to(device=windows.device, dtype=torch.float32)
+    b = base[None, None, :, None, None]
+    return (b + a[None, :, None, None, None] * (windows[:, None] - b)).reshape(-1, *windows.shape[1:]).contiguous()
+
+
+def _gather_windows(x, window, stride, grid, first, n):
+    """Windows [first, first + n) of scenes x [B, H, W] or [B, C, H, W], laid out as in blend_windows with the origin rule of
+    window_origin (csrc/pixel_source.cuh): -> [n, window, window] or [n, C, window, window]."""
+    H, W = x.shape[-2:]
+    (sy, sx), (ny, nx) = stride, grid
+    g = torch.arange(first, first + n, device=x.device)
+    b, k = g // (ny * nx), g % (ny * nx)
+    oy = torch.clamp_max((k // nx) * sy, H - window)
+    ox = torch.clamp_max((k % nx) * sx, W - window)
+    r = torch.arange(window, device=x.device)
+    rows, cols = (oy[:, None] + r)[:, :, None], (ox[:, None] + r)[:, None, :]
+    bi = b[:, None, None]
+    if x.dim() == 3:
+        return x[bi, rows, cols]
+    return x[bi, :, rows, cols].permute(0, 3, 1, 2).contiguous()        # advanced indices first: [n, w, w, C] -> [n, C, w, w]
+
+
+def _input_grads(model, xi, dF):
+    """d F / d xi for a batch of interpolated windows xi [m, bands, w, w] through the model's kernels (patch-embedding data gradient
+    included), with dF = dF/dlogits [m, nc, w, w]."""
+    xi = xi.detach().requires_grad_(True)
+    with torch.enable_grad():
+        y = model(xi)
+        if tuple(y.shape) != tuple(dF.shape):
+            raise ValueError(f"attribution: the model must classify every pixel of a window ({list(dF.shape)}), got {tuple(y.shape)}")
+        (g,) = torch.autograd.grad(y, xi, grad_outputs=dF.to(y.dtype))
+    return g.contiguous()
+
+
+def attribute_sum(grads, acc, wsum, *, steps, stride, grid, first, weight=None):
+    """One chunk of msst_scene_attribute: acc [B, bands, H, W] += weight * sum_k grads[window, k] and wsum [B, H, W] += weight over the
+    pixels of global windows [first, first + n), grads [n * steps, bands, w, w] fp32 (window-major, step-minor; windows laid out as in
+    blend_windows).  Chunks must be added in ascending order; the sums are then bitwise independent of the chunking."""
+    who = "attribute_sum"
+    for t, name in ((grads, "grads"), (acc, "acc"), (wsum, "wsum"), (weight, "weight")):
+        if (t is not None or name != "weight") and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32
+                                                         and t.is_contiguous() and t.device == acc.device):
+            raise ValueError(f"{who}: {name} must be a contiguous fp32 CUDA tensor on the device of acc")
+    if grads.dim() != 4 or acc.dim() != 4 or steps < 1 or grads.shape[0] % steps:
+        raise ValueError(f"{who}: grads must be [n * steps, bands, w, w] and acc [B, bands, H, W], got {tuple(grads.shape)}, "
+                         f"{tuple(acc.shape)} (steps={steps})")
+    n, w = grads.shape[0] // steps, grads.shape[-1]
+    B, nb, H, W = acc.shape
+    if (grads.shape[1] != nb or grads.shape[2] != w or tuple(wsum.shape) != (B, H, W)
+            or (weight is not None and tuple(weight.shape) != (w, w))):
+        raise ValueError(f"{who}: shapes grads {tuple(grads.shape)}, acc {tuple(acc.shape)}, wsum {tuple(wsum.shape)} disagree")
+    dims = _lib.SceneAttributeDims(B, nb, H, W, w, stride[0], stride[1], grid[0], grid[1], first, n, steps)
+    _lib.check(_lib.lib().msst_scene_attribute(ctypes.byref(dims), grads.data_ptr(), weight.data_ptr() if weight is not None else None,
+                                               acc.data_ptr(), wsum.data_ptr(), torch.cuda.current_stream(acc.device).cuda_stream))
+
+
+class _AttributionMode:
+    """Eval mode and requires_grad off on every parameter for the duration of an attribution call; both restored on exit.  With the
+    parameters frozen no parameter-gradient kernel of the patch embedding runs, and no backward hands a parameter gradient to a
+    FusedAdam gradient arena (ops._grad_buffers) that a training step may be about to read."""
+
+    def __init__(self, model):
+        self.model = model
+
+    def __enter__(self):
+        self.training = self.model.training
+        self.params = [p for p in self.model.parameters()]
+        self.flags = [p.requires_grad for p in self.params]
+        self.model.eval()
+        for p in self.params:
+            p.requires_grad_(False)
+
+    def __exit__(self, *exc):
+        for p, f in zip(self.params, self.flags):
+            p.requires_grad_(f)
+        self.model.train(self.training)
+        return False
+
+
+def attribute_windows(model, windows, target, *, steps=32, baseline=None):
+    """Integrated gradients (IG) of a classifier's per-pixel logits with respect to its input windows.
+
+    model: ViTSpatialSpectral (any head that classifies every pixel, spectral_only / PatchEmbed / spectral positions too) or
+    ViTSpatialSpectral_V1, fp32 or bf16 precision.  windows [n, bands, w, w] fp32 CUDA in the model's units (standardised).
+    target [n, w, w] integer: the class whose logit each pixel explains; a pixel counts when its target is in [0, nc) (so -1 is left
+    out), the rule of confusion_matrix.  The objective is F(x) = sum over counted pixels p of logits(x)[target(p), p].
+    baseline: None (0 in model units: the band mean of a standardised scene) or a [bands] spectrum x'.
+      attr  = (x - x') * (1 / steps) * sum_k dF/dx at x' + alpha_k (x - x'),  alpha_k = (k + 1/2) / steps (ig_alphas), k ascending
+      delta = sum attr - (F(x) - F(x'))   per window, float64: IG's completeness gap, -> 0 as steps grows
+    All n * steps interpolated windows run through the model's kernels in one forward and one backward (eval mode, parameters frozen
+    for the call); the step sums use msst_scene_attribute, so attribute_scene with stride = window stitches these windows bit for bit.
+    -> (attr [n, bands, w, w] fp32, delta [n] float64)."""
+    who = "attribute_windows"
+    bands, w, nc = _attr_model(who, model)
+    steps = _steps_arg(who, steps)
+    if (not isinstance(windows, torch.Tensor) or windows.dim() != 4 or tuple(windows.shape[1:]) != (bands, w, w)
+            or windows.dtype != torch.float32 or not windows.is_cuda or windows.shape[0] < 1):
+        got = f"{windows.dtype} {tuple(windows.shape)} on {windows.device}" if isinstance(windows, torch.Tensor) else type(windows).__name__
+        raise ValueError(f"{who}: windows must be a fp32 CUDA tensor [n >= 1, {bands}, {w}, {w}], got {got}")
+    n = windows.shape[0]
+    target = _target_arg(who, target, (n, w, w), windows.device)
+    base = _baseline_arg(who, baseline, bands, windows.device)
+    x = windows.contiguous()
+    dF = _objective_weights(target, nc)
+    acc = torch.zeros(n, bands, w, w, device=x.device, dtype=torch.float32)
+    wsum = torch.zeros(n, w, w, device=x.device, dtype=torch.float32)
+    with _AttributionMode(model):
+        g = _input_grads(model, _interpolate(x, base, steps), dF.repeat_interleave(steps, 0))
+        attribute_sum(g, acc, wsum, steps=steps, stride=(w, w), grid=(1, 1), first=0)
+        with torch.no_grad():
+            ends = model(torch.cat([x, base[None, :, None, None].expand(n, -1, w, w)]))
+        F = (ends.double() * dF.double().repeat(2, 1, 1, 1)).sum((1, 2, 3))
+    attr = (x - base[:, None, None]) * (acc / (steps * wsum[:, None]))
+    delta = attr.double().sum((1, 2, 3)) - (F[:n] - F[n:])
+    return attr, delta
+
+
+def attribute_scene(model, scene, target, *, steps=32, baseline=None, stride=None, weight=None, batch_samples=4096):
+    """Integrated-gradients attribution of whole scenes from overlapping windows: which bands, at which pixels, drove the classifier's
+    logit of each pixel's target class.
+
+    model, steps, baseline: as in attribute_windows.  scene: fp32 CUDA cube [B, bands, H, W] in the model's units, or RawTiles over
+    whole scenes (crop (0, 0)), standardised with its pad bands as the model sees them.  target [B, H, W] integer: labels, or
+    predict_scene's pred; the counting rule of attribute_windows.  stride, weight: as in predict_scene (weight weighs a window's
+    gradients).  Every window is attributed for its own pixels' objective, as in attribute_windows; chunks of max(1, batch_samples //
+    steps) windows run their n * steps interpolated windows through one forward and one backward, and msst_scene_attribute adds each
+    pixel's step sums over the covering windows on the device, deterministically and independently of the chunking.
+    -> attr [B, bands, H, W] fp32 = (x - x') * sum_windows weight * sum_k dF/dx / (steps * sum_windows weight), in the model's units
+    (pad bands included; at baseline 0 they are exactly 0)."""
+    who = "attribute_scene"
+    bands, w, nc = _attr_model(who, model)
+    steps = _steps_arg(who, steps)
+    tiles = scene.tiles if isinstance(scene, RawTiles) else scene
+    if not isinstance(tiles, torch.Tensor) or tiles.dim() != 4:
+        raise ValueError(f"{who}: scene must be a [B, bands, H, W] tensor or RawTiles")
+    if not tiles.is_cuda:
+        raise ValueError(f"{who}: the scene must be on a CUDA device")
+    if isinstance(scene, RawTiles):
+        if scene.crop != (0, 0):
+            raise ValueError(f"{who}: RawTiles must cover whole scenes (crop (0, 0)), got crop {scene.crop}")
+    elif tiles.dtype != torch.float32:
+        raise ValueError(f"{who}: a scene cube must be fp32 in the model's units, got {tiles.dtype}")
+    B, nb, H, W = tiles.shape
+    nb += scene.pad_bands if isinstance(scene, RawTiles) else 0
+    if nb != bands:
+        raise ValueError(f"{who}: the scene has {nb} bands, the model {bands}")
+    stride = stride if stride is not None else w
+    ny, nx = scene_windows(H, W, w, stride)
+    sy, sx = (stride, stride) if isinstance(stride, int) else stride
+    target = _target_arg(who, target, (B, H, W), tiles.device)
+    base = _baseline_arg(who, baseline, bands, tiles.device)
+    if weight is not None:
+        weight = torch.as_tensor(weight, dtype=torch.float32, device=tiles.device).contiguous()
+        if weight.shape != (w, w):
+            raise ValueError(f"{who}: weight must be [{w}, {w}], got {tuple(weight.shape)}")
+    if isinstance(batch_samples, bool) or not isinstance(batch_samples, int) or batch_samples < 1:
+        raise ValueError(f"{who}: batch_samples={batch_samples!r} must be an int >= 1")
+    x = _model_units(scene, pad=True).contiguous()
+    acc = torch.zeros(B, bands, H, W, device=x.device, dtype=torch.float32)
+    wsum = torch.zeros(B, H, W, device=x.device, dtype=torch.float32)
+    total, step = B * ny * nx, max(1, batch_samples // steps)
+    with _AttributionMode(model):
+        for first in range(0, total, step):
+            n = min(step, total - first)
+            xw = _gather_windows(x, w, (sy, sx), (ny, nx), first, n)
+            dF = _objective_weights(_gather_windows(target, w, (sy, sx), (ny, nx), first, n), nc)
+            g = _input_grads(model, _interpolate(xw, base, steps), dF.repeat_interleave(steps, 0))
+            attribute_sum(g, acc, wsum, steps=steps, stride=(sy, sx), grid=(ny, nx), first=first, weight=weight)
+    return (x - base[:, None, None]) * (acc / (steps * wsum[:, None]))
+
+
+def band_importance(attr, labels, *, num_classes, ignore_index=-1):
+    """Per-class band profile of an attribution map: the mean |attr| over the pixels of each class, in float64.
+    attr [B, bands, H, W] (attribute_scene), labels [B, H, W] integer; a pixel counts when its label is != ignore_index and in
+    [0, num_classes) (the rule of confusion_matrix).  Sums run as one float64 one-hot matrix product, with no float atomics, so the
+    profile is deterministic.  Runs wherever the tensors are.
+    -> [num_classes, bands] float64; a class without pixels gives a row of NaN."""
+    who = "band_importance"
+    if not isinstance(attr, torch.Tensor) or attr.dim() != 4 or not attr.dtype.is_floating_point:
+        raise ValueError(f"{who}: attr must be a real floating [B, bands, H, W] tensor")
+    B, nb, H, W = attr.shape
+    if (not isinstance(labels, torch.Tensor) or tuple(labels.shape) != (B, H, W) or labels.dtype.is_floating_point
+            or labels.dtype.is_complex or labels.dtype == torch.bool or labels.device != attr.device):
+        raise ValueError(f"{who}: labels must be an integer tensor [{B}, {H}, {W}] on {attr.device}")
+    if isinstance(num_classes, bool) or not isinstance(num_classes, int) or num_classes < 1:
+        raise ValueError(f"{who}: num_classes={num_classes!r} must be an int >= 1")
+    lab = labels.reshape(-1).to(torch.int64)
+    valid = (lab != ignore_index) & (lab >= 0) & (lab < num_classes)
+    oh = torch.nn.functional.one_hot(torch.where(valid, lab, 0), num_classes).to(torch.float64) * valid[:, None]
+    rows = attr.detach().abs().to(torch.float64).permute(0, 2, 3, 1).reshape(-1, nb)
+    return (oh.T @ rows) / oh.sum(0)[:, None]

@@ -141,15 +141,22 @@ class PatchEmbedFn(torch.autograd.Function):
         img, pre_w, pre_b, W, bias, post_w, post_b, mask_u8 = ctx.saved_tensors
         dims = ctx.dims
         T, D = ctx.pos_shape
-        g = _grad_buffers([pre_w, pre_b, W, bias, post_w, post_b])
-        g += list(torch.split(torch.zeros(T * D + D, device=pre_w.device, dtype=torch.float32), [T * D, D]))   # pos rows, mask token
         d_tokens = _c(d_tokens)
         d_pln = _c(d_pln) if d_pln is not None else None
+        d_img = None
+        if ctx.needs_input_grad[0] and img is not None:     # raw tiles (img None) have no gradient
+            d_img = torch.empty_like(img)
+            check(_lib.lib().msst_patch_embed_bwd_data(C.byref(dims), _p(img), _p(pre_w), _p(pre_b), _p(W), _p(bias), _p(post_w),
+                                                       _p(post_b), _p(mask_u8), _p(d_tokens), _p(d_pln), _p(d_img), _stream()))
+        if not any(ctx.needs_input_grad[1:9]):
+            return (d_img,) + (None,) * 13
+        g = _grad_buffers([pre_w, pre_b, W, bias, post_w, post_b])
+        g += list(torch.split(torch.zeros(T * D + D, device=pre_w.device, dtype=torch.float32), [T * D, D]))   # pos rows, mask token
         check(_lib.lib().msst_patch_embed_bwd(C.byref(dims), _p(img), _p(pre_w), _p(pre_b), _p(W), _p(bias), _p(post_w),
                                               _p(post_b), _p(mask_u8), _p(d_tokens), _p(d_pln), _p(g[0]), _p(g[1]), _p(g[2]),
                                               _p(g[3]), _p(g[4]), _p(g[5]), _p(g[6]), _p(g[7]) if ctx.has_mt else None,
                                               _stream()))
-        return (None, g[0], g[1], g[2], g[3], g[4], g[5], g[6].view(T, D),
+        return (d_img, g[0], g[1], g[2], g[3], g[4], g[5], g[6].view(T, D),
                 g[7] if ctx.has_mt else None, None, None, None, None, None)
 
 
@@ -340,12 +347,17 @@ class DecodeL1Fn(torch.autograd.Function):
         d_loss = _c(d_loss.to(torch.float32))
         d_enc = torch.zeros_like(enc)
         g = _grad_buffers([W, bias])
-        d_tgt = None
+        d_tgt = d_img = None
         if target_tokens is not None and ctx.needs_input_grad[3]:
             d_tgt = torch.zeros_like(target_tokens)
+        elif img is not None and ctx.needs_input_grad[2]:   # the cube is the target: the kernel writes -dloss/dpred per patch element
+            d_tgt = torch.zeros(dims.B, dims.C * dims.G * dims.G, dims.p0 * dims.p1 * dims.p1, device=enc.device, dtype=torch.float32)
         check(_lib.lib().msst_simmim_decode_l1_bwd(C.byref(dims), _p(enc), _p(idx), _p(img), _p(target_tokens), _p(W), _p(bias),
                                                    _p(d_loss), _p(d_enc), _p(g[0]), _p(g[1]), _p(d_tgt), _stream()))
-        return d_enc, None, None, d_tgt, g[0], g[1], None
+        if target_tokens is None and d_tgt is not None:
+            from .vit_spatial_spectral import _patches_to_img   # (import cycle: that module imports this one)
+            d_img, d_tgt = _patches_to_img(d_tgt, dims.C, dims.G, dims.p0, dims.p1), None
+        return d_enc, None, d_img, d_tgt, g[0], g[1], None
 
 
 def simmim_decode_l1(enc, idx, img, target_tokens, W, bias, *, geom):
